@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — image-pairs/s of the bi-temporal change-detection hot path on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the hot path over one batch of synthetic image pairs on every rank:
@@ -16,6 +16,10 @@ the int64[4] all-reduce of the matrix (the path's only collective).  Prints ONE 
 * ``cpu_baseline``  the oracle's fp32 CPU forward (torch.nn.functional restatement of the
                 reference, oracle/nets.py) on this box's host cores, bounded sample, rank 0, N=1.
 ``--impl reference`` times that CPU path alone with all host threads and prints the same line.
+``--dump-outputs DIR`` writes the last timed step's logits, change map and confusion matrix as .npy files; inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
+The default workloads SNUNet 256^2 and SegCD 1024^2 also time the other one, in an ``also`` object of the same line:
+``--steps`` timed steps after a fixed 3 warm-up steps, whatever ``--warmup`` says.
 """
 from __future__ import annotations
 
@@ -139,6 +143,27 @@ def measured_peaks():
         return dict(hbm=d["hbm_gbs"], tf_burst=d["bf16_tflops"], tf_sust=d.get("bf16_tflops_sustained", d["bf16_tflops"]),
                     src="measured")
     return dict(hbm=6650.0, tf_burst=1590.0, tf_sust=1400.0, src="fallback")
+
+
+DUMP_BYTES = 60 << 20           # what --dump-outputs writes in all: under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor of ``arrays`` as ``out_dir/<name>.npy``: int64 counts as float64, everything else as float32.
+    Arrays under 1 MiB are written whole.  When the larger ones together exceed what is left of DUMP_BYTES, each keeps
+    the same share of its elements, drawn with a fixed seed and written flattened in index order, so the files of two
+    builds run with the same arguments compare element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: (t.double() if t.dtype == torch.int64 else t.float()).cpu().numpy() for k, t in arrays.items()}
+    small = sum(a.nbytes for a in host.values() if a.nbytes < 1 << 20)
+    large = sum(a.nbytes for a in host.values() if a.nbytes >= 1 << 20)
+    keep = max(0.0, min(1.0, (DUMP_BYTES - small) / max(large, 1)))
+    for name, a in host.items():
+        if keep < 1.0 and a.nbytes >= 1 << 20:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, int(a.size * keep), replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 class ClockSampler:
@@ -348,14 +373,14 @@ def run_ours(args, wl, rank, world, local_rank):
         dist.init_process_group("nccl", device_id=dev)
     out = measure(args, args.workload, wl, rank, world, local_rank, dev, full=True)
     # BASELINE.json's metric names both sizes ("at 256^2 and 1024^2"): the other headline configuration rides
-    # along as a compact object (fewer steps, no CPU leg) so one default run reports both
+    # along as a compact object (same --steps, no CPU leg) so one default run reports both
     other = {"snunet_256_b64": "segcd_r34_1024_b16", "segcd_r34_1024_b16": "snunet_256_b64"}.get(args.workload)
     if other and not args.no_also:
         import copy
         a2 = copy.copy(args)
         wl2 = WORKLOADS[other]
         a2.workload, a2.chunk, a2.input_sets = other, wl2.get("chunk", 32), wl2.get("input_sets", 4)
-        a2.steps, a2.warmup, a2.no_cpu_baseline = min(args.steps, 5), 3, True
+        a2.warmup, a2.no_cpu_baseline = 3, True
         torch.cuda.empty_cache()
         o2 = measure(a2, other, wl2, rank, world, local_rank, dev, full=False)
         if out is not None and o2 is not None:
@@ -488,6 +513,15 @@ def measure(args, wl_name, wl, rank, world, local_rank, dev, full=True):
         return float(ms.item())
 
     ms_total = timed(step, args.steps, args.warmup, sampler)
+    if full and rank == 0 and args.dump_outputs:
+        # the last timed step's logits and change map (the e2e passes below overwrite these buffers) and that step's own
+        # confusion matrix: the evaluator kernel run again on its logits and labels into a fresh accumulator, since
+        # `metric` holds the sum over the warm-up and timed steps
+        last = SegmentationMetric(2, dev)
+        last.addLogits(logits[-1], dlab[(args.warmup + args.steps - 1) % n_sets], kind=wl["kind"])
+        outs = {("logits" if len(logits) == 1 else f"logits{i}"): t for i, t in enumerate(logits)}
+        outs.update(change_map=pred, confusion_matrix=last.confusion_counts())
+        dump_outputs(args.dump_outputs, outs)
     metric.reset()
     ms_e2e = timed(step_e2e, args.steps, max(1, args.warmup // 2))
     metric.reset()
@@ -585,7 +619,11 @@ def main():
     ap.add_argument("--input-sets", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the compact run of the other headline configuration")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's outputs to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     wl = WORKLOADS[args.workload]
