@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define STCD_ABI_VERSION 18
+#define STCD_ABI_VERSION 19
 
 enum stcd_status {
   STCD_OK = 0,
@@ -312,6 +312,22 @@ int stcd_plan_add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int
 int stcd_plan_add_sr_attention(stcd_plan* plan, int q_tensor, int kv_tensor, int dst_tensor, int c, int heads, float scale);
 int stcd_plan_add_dwconv3x3(stcd_plan* plan, int src_tensor, int dst_tensor, int c, const float* weight, const float* bias,
                             int gelu);
+
+/* Split-precision variants (see stcd_conv_desc.split), same arguments as the functions above.  Every tensor holds a value as
+ * hi + lo bf16 planes: a tensor of c logical channels stores 2c (a multiple of 16), the hi plane in channels [0, c) and the lo
+ * plane in [c, 2c), hi = bf16(v), lo = bf16(v - hi).  The kernels read hi + lo, compute in fp32 and write both planes.
+ * layernorm_split: src and dst store 2c channels; the space-to-depth copy stores 8c: hi of parity class k, channel ch at
+ *   k*c + ch, lo at 4c + k*c + ch.
+ * sr_attention_split: q and dst store 2c, kv 4c (k hi [0, c), v hi [c, 2c), k lo [2c, 3c), v lo [3c, 4c)); exactly 64 keys.
+ *   S = Qhi Khi^T + Qlo Khi^T + Qhi Klo^T, fp32 softmax, P split into hi + lo, O = Phi Vhi + Plo Vhi + Phi Vlo, normalised by
+ *   the fp32 row sum.
+ * dwconv3x3_split, bilinear_up_split: src and dst store 2c channels. */
+int stcd_plan_add_layernorm_split(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d_or_neg, int c, const float* gamma,
+                                  const float* beta, float eps);
+int stcd_plan_add_sr_attention_split(stcd_plan* plan, int q_tensor, int kv_tensor, int dst_tensor, int c, int heads, float scale);
+int stcd_plan_add_dwconv3x3_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, const float* weight, const float* bias,
+                                  int gelu);
+int stcd_plan_add_bilinear_up_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int scale);
 
 /* SNUNet's ECAM tail (models/SNUNet.py:144-149: two ChannelAttention blocks :46-59 + conv_final)
  * over four activation tensors of `c` channels each, as one fused op writing external output

@@ -100,6 +100,7 @@ class _EncoderTransformerV3(nn.Module):
 class ChangeFormerV6(PlannedModule):
     """models/ChangeFormer.py:1669-1701."""
     default_chunk_pairs = 32
+    supports_precision_path = True
 
     def __init__(self, input_nc: int = 3, output_nc: int = 2, decoder_softmax: bool = False, embed_dim: int = 256):
         super().__init__()
@@ -123,7 +124,7 @@ class ChangeFormerV6(PlannedModule):
                 m.bias.data.zero_()
 
     def lower(self, h: int, w: int) -> L.Program:
-        return lower_changeformer(self.state_dict(), self.input_nc, self.embedding_dim, self.output_nc, h, w)
+        return lower_changeformer(self.state_dict(), self.input_nc, self.embedding_dim, self.output_nc, h, w, precision=self.plan_precision)
 
     @torch.no_grad()
     def forward(self, x1: torch.Tensor, x2: torch.Tensor):
@@ -134,15 +135,16 @@ class ChangeFormerV6(PlannedModule):
 
 
 # ------------------------------------------------------------------------------------------
-def lower_changeformer(sd: Dict[str, torch.Tensor], in_ch: int, e: int, n_class: int, h: int, w: int) -> L.Program:
-    """state_dict of the reference ChangeFormerV6 -> fused-op Program (eval mode)."""
+def lower_changeformer(sd: Dict[str, torch.Tensor], in_ch: int, e: int, n_class: int, h: int, w: int, precision: str = "bf16") -> L.Program:
+    """state_dict of the reference ChangeFormerV6 -> fused-op Program (eval mode).  precision "split": every op carries (hi, lo)
+    bf16 planes (lowering.Program.precision); the split K-programs that outgrow the conv kernel's tables are cut along K."""
     if h % 256 or w % 256:
         # stage 1 reduces its keys by sr = 8 at 1/4 scale, ..., and every stage must leave an integer, even token grid
         raise ValueError(f"ChangeFormerV6 lowering needs H and W divisible by 256 (got {h}x{w}); the reference is built for 256")
     if (h // 32) * (w // 32) > 64:
         raise ValueError("the attention kernel keeps at most 64 reduced tokens per image (256x256 inputs, the reference's img_size)")
     sd = {k: v.detach().to("cpu", torch.float32) for k, v in sd.items()}
-    p = L.Program(model="ChangeFormerV6", in_channels=in_ch, h=h, w=w)
+    p = L.Program(model="ChangeFormerV6", in_channels=in_ch, h=h, w=w, precision=precision)
     feats = lower_mit_encoder(p, sd, "Tenc_x2", in_ch, _DEPTHS, h, w)
     lower_diff_decoder(p, sd, feats, e, n_class, "TDec_x2", "TDec_x2.linear_c{k}")
     return p
@@ -160,10 +162,10 @@ def lower_mit_encoder(p: L.Program, sd: Dict[str, torch.Tensor], enc: str, in_ch
                    pair=True, macs_per_pair=2 * hh * ww * cin * cout, **kw)
 
     def layernorm(name: str, pre: str, src: str, dst: str, c: int, eps: float, dst_s2d=None) -> None:
-        p.ops.append(L.LayerNormSpec(name, src, dst, c, npf(sd[f"{pre}.weight"]), npf(sd[f"{pre}.bias"]), eps, dst_s2d))
+        p.ops.append(L.LayerNormSpec(name, src, dst, c, npf(sd[f"{pre}.weight"]), npf(sd[f"{pre}.bias"]), eps, dst_s2d, split=p.split))
 
     p.tensor("in", 2, h, w, 8)
-    p.ops.append(L.InputPackSpec("pack", "in", in_ch))
+    p.ops.append(L.InputPackSpec("pack", "in", in_ch, split=p.split))
     feats = []
     x_s2d = None
     hh, ww = h, w
@@ -206,7 +208,7 @@ def lower_mit_encoder(p: L.Program, sd: Dict[str, torch.Tensor], enc: str, in_ch
             ao = p.tensor(f"{a}.o", 2, hh, ww, c)
             d = c // heads
             p.ops.append(L.AttentionSpec(f"{a}.softmax", q, kv, ao, c, heads, float(d ** -0.5),
-                                         macs_per_pair=2 * 2 * hh * ww * hk * wk * c))
+                                         macs_per_pair=2 * 2 * hh * ww * hk * wk * c, split=p.split))
             x1 = p.tensor(f"{blk}.x1", 2, hh, ww, c)
             linear(f"{a}.proj", f"{a}.proj", ao, c, c, hh, ww, res=x, out0=x1)
             n2 = p.tensor(f"{blk}.n2", 2, hh, ww, c)
@@ -216,7 +218,8 @@ def lower_mit_encoder(p: L.Program, sd: Dict[str, torch.Tensor], enc: str, in_ch
             linear(f"{m}.fc1", f"{m}.fc1", n2, c, 4 * c, hh, ww, out0=h1)
             h2 = p.tensor(f"{m}.h2", 2, hh, ww, 4 * c)
             p.ops.append(L.DWConvSpec(f"{m}.dwconv", h1, h2, 4 * c, npf(sd[f"{m}.dwconv.dwconv.weight"].reshape(4 * c, 9)),
-                                      npf(sd[f"{m}.dwconv.dwconv.bias"]), gelu=True, macs_per_pair=2 * hh * ww * 9 * 4 * c))
+                                      npf(sd[f"{m}.dwconv.dwconv.bias"]), gelu=True, macs_per_pair=2 * hh * ww * 9 * 4 * c,
+                                      split=p.split))
             x = p.tensor(f"{blk}.out", 2, hh, ww, c)
             linear(f"{m}.fc2", f"{m}.fc2", h2, 4 * c, c, hh, ww, res=x1, out0=x)
         f = p.tensor(f"{enc}.f{s + 1}", 2, hh, ww, c)

@@ -368,7 +368,7 @@ def lower_diff_decoder(p: L.Program, sd: Dict[str, torch.Tensor], feats, e: int,
         res = None
         if c_prev is not None:
             res = p.tensor(f"{dk}.up_prev", 1, fh, fw, e)
-            p.ops.append(L.BilinearUpSpec(f"{dk}.up_prev", c_prev, res, e, 2))
+            p.ops.append(L.BilinearUpSpec(f"{dk}.up_prev", c_prev, res, e, 2, split=p.split))
         ck = p.tensor(f"{dk}.out", 1, fh, fw, e)
         s2, b2 = L.fold_bn(None, L.bn_params(sd, f"{dk}.6"), e)
         L.add_conv(p, f"{dk}.4", [L.Segment(ta, e)], L.conv_taps(sd[f"{dk}.4.weight"], pad=1), e, fh, fw, 1, ones(e),
@@ -393,7 +393,7 @@ def lower_diff_decoder(p: L.Program, sd: Dict[str, torch.Tensor], feats, e: int,
             ups.append(ck)
         else:
             up = p.tensor(f"{dk}.up_full", 1, full_h, full_w, e)
-            p.ops.append(L.BilinearUpSpec(f"{dk}.up_full", ck, up, e, full_h // fh))
+            p.ops.append(L.BilinearUpSpec(f"{dk}.up_full", ck, up, e, full_h // fh, split=p.split))
             ups.append(up)
         c_prev = ck
     fused = p.tensor(f"{d}.fused", 1, full_h, full_w, e)

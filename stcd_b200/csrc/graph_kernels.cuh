@@ -15,6 +15,7 @@
 #include <stdint.h>
 
 #include "ptx.cuh"
+#include "transformer_kernels.cuh"     // unpack8 / split8 (split-precision bilinear up-sampling)
 
 namespace stcd {
 
@@ -584,6 +585,9 @@ __global__ void __launch_bounds__(256) max_relative_nc8_kernel(const float* __re
 
 // Bilinear up-sampling by an integer factor, align_corners=False (PyTorch's area_pixel_compute_source_index:
 // src = (dst + 0.5) / scale - 0.5 clamped at 0), bf16 [B][c8][h][w][8] -> bf16 [B][c8][s*h][s*w][8], fp32 arithmetic.
+// SPLIT (lowering.Program.precision): src and dst hold hi and lo planes (channel groups [0, c8/2) and [c8/2, c8)); the four taps
+// read hi + lo and the result is written as hi = bf16(v), lo = bf16(v - hi).
+template <bool SPLIT>
 __global__ void __launch_bounds__(256) bilinear_up_kernel(const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ dst,
                                                           int B, int g8, int src_c8, int dst_c8, int h, int w, int scale) {
   const int ho = h * scale, wo = w * scale;
@@ -609,6 +613,35 @@ __global__ void __launch_bounds__(256) bilinear_up_kernel(const __nv_bfloat16* _
     const uint4 q11 = __ldg(reinterpret_cast<const uint4*>(base + (static_cast<size_t>(y1) * w + x1) * 8));
     const uint32_t a[4] = {q00.x, q00.y, q00.z, q00.w}, bq[4] = {q01.x, q01.y, q01.z, q01.w};
     const uint32_t c[4] = {q10.x, q10.y, q10.z, q10.w}, dq[4] = {q11.x, q11.y, q11.z, q11.w};
+    if constexpr (SPLIT) {
+      const size_t s_lo = static_cast<size_t>(src_c8 >> 1) * h * w * 8;
+      const uint4 l00 = __ldg(reinterpret_cast<const uint4*>(base + s_lo + (static_cast<size_t>(y0) * w + x0) * 8));
+      const uint4 l01 = __ldg(reinterpret_cast<const uint4*>(base + s_lo + (static_cast<size_t>(y0) * w + x1) * 8));
+      const uint4 l10 = __ldg(reinterpret_cast<const uint4*>(base + s_lo + (static_cast<size_t>(y1) * w + x0) * 8));
+      const uint4 l11 = __ldg(reinterpret_cast<const uint4*>(base + s_lo + (static_cast<size_t>(y1) * w + x1) * 8));
+      float v00[8], v01[8], v10[8], v11[8], t8[8], r[8];
+      unpack8(q00, v00), unpack8(q01, v01), unpack8(q10, v10), unpack8(q11, v11);
+      unpack8(l00, t8);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) v00[j] += t8[j];
+      unpack8(l01, t8);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) v01[j] += t8[j];
+      unpack8(l10, t8);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) v10[j] += t8[j];
+      unpack8(l11, t8);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) v11[j] += t8[j];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) r[j] = hy * (hx * v00[j] + lx * v01[j]) + ly * (hx * v10[j] + lx * v11[j]);
+      uint4 oh, ol;
+      split8(r, oh, ol);
+      __nv_bfloat16* op = dst + ((b * dst_c8 + g) * static_cast<size_t>(ho) * wo + static_cast<size_t>(oy) * wo + ox) * 8;
+      *reinterpret_cast<uint4*>(op) = oh;
+      *reinterpret_cast<uint4*>(op + static_cast<size_t>(dst_c8 >> 1) * ho * wo * 8) = ol;
+      continue;
+    }
     uint32_t o[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {

@@ -117,8 +117,10 @@ struct GraphOp {
   float* ysq = nullptr;        // r > 1
 };
 
+// split: split precision (lowering.Program.precision), every tensor of the op holds a hi and a lo plane
 struct BilinearOp {
   int src, dst, c, scale;
+  int split = 0;
 };
 
 struct LayerNormOp {
@@ -126,17 +128,20 @@ struct LayerNormOp {
   float eps;
   std::vector<float> gb;   // gamma | beta
   float* gb_dev = nullptr;
+  int split = 0;
 };
 
 struct AttentionOp {
   int q, kv, dst, c, heads;
   float scale;
+  int split = 0;
 };
 
 struct DWConvOp {
   int src, dst, c, gelu;
   std::vector<float> wb;   // weight [c][9] | bias [c]
   float* wb_dev = nullptr;
+  int split = 0;
 };
 
 struct AbsDiffOp {
@@ -583,9 +588,10 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const size_t total = (size_t)B * ts.h * ts.w;
       __nv_bfloat16* d2 = k.dst2 >= 0 ? (__nv_bfloat16*)plan->tensors[k.dst2].ptr : nullptr;
       // 4 threads per pixel (a warp = 8 pixels x 4 channel slices)
-      stcd::layernorm_kernel<<<(unsigned)std::max<size_t>(1, std::min<size_t>((total * 4 + 255) / 256, 148 * 16)), 256, 0, st>>>(
-          (const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, d2, k.gb_dev, k.gb_dev + k.c, B, k.c, ts.c / 8, td.c / 8,
-          k.dst2 >= 0 ? plan->tensors[k.dst2].c / 8 : 0, ts.h, ts.w, k.eps);
+      const unsigned blocks = (unsigned)std::max<size_t>(1, std::min<size_t>((total * 4 + 255) / 256, 148 * 16));
+      auto kern = k.split ? stcd::layernorm_kernel<true> : stcd::layernorm_kernel<false>;
+      kern<<<blocks, 256, 0, st>>>((const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, d2, k.gb_dev, k.gb_dev + k.c, B, k.c, ts.c / 8,
+                                   td.c / 8, k.dst2 >= 0 ? plan->tensors[k.dst2].c / 8 : 0, ts.h, ts.w, k.eps);
       CUDA_TRY(cudaGetLastError());
     } else if (o.kind == 8) {
       const AttentionOp& k = plan->attns[o.idx];
@@ -595,11 +601,14 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const int B = tq.mult * plan->chunk, N = tq.h * tq.w, NK = tk.h * tk.w, D = k.c / k.heads;
       const dim3 grid((N + 255) / 256, k.heads, B);                       // two queries per thread
       const bool use_mma = NK == 64 && env_int("STCD_ATTN_MMA", 1);        // every stage of the 256 x 256 configurations
-      if (use_mma && D == 64)
-        stcd::sr_attention_mma_kernel<64><<<dim3((N + 63) / 64, k.heads, B), 128, 0, st>>>(
+      if (k.split)                                                          // split precision: tensor-core kernel only (NK == 64)
+        (D == 64 ? stcd::sr_attention_mma_kernel<64, true> : stcd::sr_attention_mma_kernel<80, true>)<<<dim3((N + 63) / 64, k.heads, B), 128, 0, st>>>(
+            (const __nv_bfloat16*)tq.ptr, (const __nv_bfloat16*)tk.ptr, (__nv_bfloat16*)td.ptr, k.c, tq.c / 8, tk.c / 8, td.c / 8, N, k.scale);
+      else if (use_mma && D == 64)
+        stcd::sr_attention_mma_kernel<64, false><<<dim3((N + 63) / 64, k.heads, B), 128, 0, st>>>(
             (const __nv_bfloat16*)tq.ptr, (const __nv_bfloat16*)tk.ptr, (__nv_bfloat16*)td.ptr, k.c, tq.c / 8, tk.c / 8, td.c / 8, N, k.scale);
       else if (use_mma && D == 80)
-        stcd::sr_attention_mma_kernel<80><<<dim3((N + 63) / 64, k.heads, B), 128, 0, st>>>(
+        stcd::sr_attention_mma_kernel<80, false><<<dim3((N + 63) / 64, k.heads, B), 128, 0, st>>>(
             (const __nv_bfloat16*)tq.ptr, (const __nv_bfloat16*)tk.ptr, (__nv_bfloat16*)td.ptr, k.c, tq.c / 8, tk.c / 8, td.c / 8, N, k.scale);
       else if (D == 64)
         stcd::sr_attention_kernel<64><<<grid, 128, 0, st>>>((const __nv_bfloat16*)tq.ptr, (const __nv_bfloat16*)tk.ptr, (__nv_bfloat16*)td.ptr,
@@ -617,8 +626,9 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const int items = ((ts.w + 3) / 4) * ts.h;                        // one thread per 4 horizontally adjacent pixels
       const dim3 grid((unsigned)std::max(1, (items + 127) / 128), (unsigned)(k.c / 8), (unsigned)B);
       (void)hwp;
-      stcd::dwconv3x3_kernel<<<grid, 128, 0, st>>>((const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, k.wb_dev, k.wb_dev + (size_t)k.c * 9, B,
-                                                   k.c / 8, ts.c / 8, td.c / 8, ts.h, ts.w, k.gelu);
+      auto kern = k.split ? stcd::dwconv3x3_kernel<true> : stcd::dwconv3x3_kernel<false>;
+      kern<<<grid, 128, 0, st>>>((const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, k.wb_dev, k.wb_dev + (size_t)k.c * 9, B, k.c / 8,
+                                 ts.c / 8, td.c / 8, ts.h, ts.w, k.gelu);
       CUDA_TRY(cudaGetLastError());
     } else if (o.kind == 6) {
       const BilinearOp& k = plan->bilinears[o.idx];
@@ -626,7 +636,8 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const Tensor& td = plan->tensors[k.dst];
       const int B = ts.mult * plan->chunk;
       const size_t total = (size_t)B * (k.c / 8) * td.h * td.w;
-      stcd::bilinear_up_kernel<<<(unsigned)std::max<size_t>(1, std::min<size_t>((total + 255) / 256, 148 * 16)), 256, 0, st>>>(
+      auto kern = k.split ? stcd::bilinear_up_kernel<true> : stcd::bilinear_up_kernel<false>;
+      kern<<<(unsigned)std::max<size_t>(1, std::min<size_t>((total + 255) / 256, 148 * 16)), 256, 0, st>>>(
           (const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, B, k.c / 8, ts.c / 8, td.c / 8, ts.h, ts.w, k.scale);
       CUDA_TRY(cudaGetLastError());
     } else if (o.kind == 4) {
@@ -971,8 +982,8 @@ int stcd_plan_add_graph_conv(stcd_plan* plan, int src_tensor, int dst_tensor, in
   return (int)plan->ops.size() - 1;
 }
 
-int stcd_plan_add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d, int c, const float* gamma, const float* beta,
-                            float eps) {
+static int add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d, int c, const float* gamma, const float* beta,
+                         float eps, int split) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor) || (dst_s2d >= 0 && !valid_tensor(plan, dst_s2d)) || !gamma || !beta)
@@ -984,8 +995,9 @@ int stcd_plan_add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int
                  ts.h, ts.w, ts.c, td.mult, td.h, td.w, td.c, c);
   if (dst_s2d >= 0) {
     const Tensor& t2 = plan->tensors[dst_s2d];
-    if ((ts.h % 2) || (ts.w % 2) || t2.h != ts.h / 2 || t2.w != ts.w / 2 || t2.c != 4 * c || t2.mult != ts.mult)
-      return -fail(STCD_ERR_INVALID, "layer norm: space-to-depth copy must be [%d*chunk,%d,%d,%d]", ts.mult, ts.h / 2, ts.w / 2, 4 * c);
+    if ((ts.h % 2) || (ts.w % 2) || t2.h != ts.h / 2 || t2.w != ts.w / 2 || t2.c != (split ? 8 : 4) * c || t2.mult != ts.mult)
+      return -fail(STCD_ERR_INVALID, "layer norm: space-to-depth copy must be [%d*chunk,%d,%d,%d]", ts.mult, ts.h / 2, ts.w / 2,
+                   (split ? 8 : 4) * c);
   }
   LayerNormOp k;
   k.src = src_tensor;
@@ -995,9 +1007,15 @@ int stcd_plan_add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int
   k.eps = eps;
   k.gb.assign(gamma, gamma + c);
   k.gb.insert(k.gb.end(), beta, beta + c);
+  k.split = split;
   plan->lns.push_back(std::move(k));
   plan->ops.push_back({7, (int)plan->lns.size() - 1});
   return (int)plan->ops.size() - 1;
+}
+
+int stcd_plan_add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d, int c, const float* gamma, const float* beta,
+                            float eps) {
+  return add_layernorm(plan, src_tensor, dst_tensor, dst_s2d, c, gamma, beta, eps, 0);
 }
 
 int stcd_plan_add_sr_attention(stcd_plan* plan, int q_tensor, int kv_tensor, int dst_tensor, int c, int heads, float scale) {
@@ -1050,6 +1068,61 @@ int stcd_plan_add_bilinear_up(stcd_plan* plan, int src_tensor, int dst_tensor, i
   plan->bilinears.push_back({src_tensor, dst_tensor, c, scale});
   plan->ops.push_back({6, (int)plan->bilinears.size() - 1});
   return (int)plan->ops.size() - 1;
+}
+
+// ---- split precision (lowering.Program.precision "split"): the same ops on tensors that hold a hi and a lo plane.  Every
+// tensor must store its logical channels twice over (hi plane first, lo plane at half the stored channels), in multiples of 16.
+static bool split_planes(const Tensor& t, int c) { return t.c % 16 == 0 && t.c / 2 >= c; }
+
+int stcd_plan_add_layernorm_split(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d, int c, const float* gamma,
+                                  const float* beta, float eps) {
+  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (valid_tensor(plan, src_tensor) && valid_tensor(plan, dst_tensor) &&
+      (!split_planes(plan->tensors[src_tensor], c) || !split_planes(plan->tensors[dst_tensor], c)))
+    return -fail(STCD_ERR_INVALID, "split layer norm: src / dst must store 2 x %d channels in multiples of 16 (got %d, %d)", c,
+                 plan->tensors[src_tensor].c, plan->tensors[dst_tensor].c);
+  return add_layernorm(plan, src_tensor, dst_tensor, dst_s2d, c, gamma, beta, eps, 1);     // space-to-depth copy: 8c (4 classes x 2 planes)
+}
+
+int stcd_plan_add_sr_attention_split(stcd_plan* plan, int q_tensor, int kv_tensor, int dst_tensor, int c, int heads, float scale) {
+  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
+  if (!valid_tensor(plan, q_tensor) || !valid_tensor(plan, kv_tensor) || !valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad tensor id");
+  const Tensor& tq = plan->tensors[q_tensor];
+  const Tensor& tk = plan->tensors[kv_tensor];
+  const Tensor& td = plan->tensors[dst_tensor];
+  if (heads < 1 || c < 8 || (c % heads) || ((c / heads) != 64 && (c / heads) != 80))
+    return -fail(STCD_ERR_INVALID, "split attention: c=%d heads=%d: head dim must be 64 or 80", c, heads);
+  if (tq.c != 2 * c || td.c != 2 * c || tk.c != 4 * c || tq.h != td.h || tq.w != td.w || tq.mult != td.mult || tq.mult != tk.mult)
+    return -fail(STCD_ERR_INVALID, "split attention: q/dst must be [m*chunk,h,w,2 x %d] and kv [m*chunk,hk,wk,2 x %d] (hi and lo planes)", c, 2 * c);
+  if (tk.h * tk.w != 64) return -fail(STCD_ERR_INVALID, "split attention: %d keys (the tensor-core kernel takes exactly 64)", tk.h * tk.w);
+  AttentionOp k{q_tensor, kv_tensor, dst_tensor, c, heads, scale};
+  k.split = 1;
+  plan->attns.push_back(k);
+  plan->ops.push_back({8, (int)plan->attns.size() - 1});
+  return (int)plan->ops.size() - 1;
+}
+
+int stcd_plan_add_dwconv3x3_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, const float* weight, const float* bias, int gelu) {
+  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (valid_tensor(plan, src_tensor) && valid_tensor(plan, dst_tensor) &&
+      (!split_planes(plan->tensors[src_tensor], c) || !split_planes(plan->tensors[dst_tensor], c)))
+    return -fail(STCD_ERR_INVALID, "split dw conv: src / dst must store 2 x %d channels in multiples of 16 (got %d, %d)", c,
+                 plan->tensors[src_tensor].c, plan->tensors[dst_tensor].c);
+  const int r = stcd_plan_add_dwconv3x3(plan, src_tensor, dst_tensor, c, weight, bias, gelu);
+  if (r >= 0) plan->dws.back().split = 1;
+  return r;
+}
+
+int stcd_plan_add_bilinear_up_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int scale) {
+  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (valid_tensor(plan, src_tensor) && valid_tensor(plan, dst_tensor) &&
+      (!split_planes(plan->tensors[src_tensor], c) || !split_planes(plan->tensors[dst_tensor], c)))
+    return -fail(STCD_ERR_INVALID, "split bilinear up: src / dst must store 2 x %d channels in multiples of 16 (got %d, %d)", c,
+                 plan->tensors[src_tensor].c, plan->tensors[dst_tensor].c);
+  const int r = stcd_plan_add_bilinear_up(plan, src_tensor, dst_tensor, c, scale);
+  if (r >= 0) plan->bilinears.back().split = 1;
+  return r;
 }
 
 int stcd_plan_add_absdiff(stcd_plan* plan, int src_tensor, int dst_tensor) {
@@ -1327,8 +1400,8 @@ int stcd_plan_add_conv(stcd_plan* plan, const stcd_conv_desc* d) {
   if (2 * mt * d->n_tile > 512)
     return -fail(STCD_ERR_INVALID, "double-buffered accumulators need %d TMEM columns (> 512)", 2 * mt * d->n_tile);
   if (d->pair && (plan->chunk < 1)) return -fail(STCD_ERR_INVALID, "pair op on an empty chunk");
-  if (d->split && (d->out0_s2d || d->fold_cs || d->xf_cs || d->relu > 1 || d->act_pre))
-    return -fail(STCD_ERR_INVALID, "split precision: plain / ReLU epilogues only (no space-to-depth, folded or horizontally folded stores)");
+  if (d->split && (d->out0_s2d || d->fold_cs || d->xf_cs))
+    return -fail(STCD_ERR_INVALID, "split precision: no space-to-depth, folded or horizontally folded stores");
   if (d->xf_cs) {
     bool ok = d->xf_cs >= 16 && d->xf_cs % 16 == 0 && d->n_tile == 3 * d->xf_cs && d->cout_pad == d->n_tile && d->cout <= d->xf_cs &&
               d->n_phase == 1 && d->osy == 1 && d->osx == 1 && !d->out0_s2d && !d->fold_cs;

@@ -27,6 +27,24 @@ __device__ __forceinline__ uint4 pack8(const float* v) {
   return make_uint4(w[0], w[1], w[2], w[3]);
 }
 
+// Split precision (lowering.Program.precision "split"): a value is hi + lo, hi in channel groups [0, c8/2) of the tensor, lo in
+// [c8/2, c8).  load8_split reads both planes as fp32 sums; split8 writes hi = bf16(v), lo = bf16(v - hi).
+__device__ __forceinline__ void load8_split(const __nv_bfloat16* p, size_t lo_off, float* v) {
+  float l[8];
+  unpack8(__ldg(reinterpret_cast<const uint4*>(p)), v);
+  unpack8(__ldg(reinterpret_cast<const uint4*>(p + lo_off)), l);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) v[j] += l[j];
+}
+__device__ __forceinline__ void split8(const float* v, uint4& hi, uint4& lo) {
+  float h[8], r[8];
+  hi = pack8(v);
+  unpack8(hi, h);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) r[j] = v[j] - h[j];
+  lo = pack8(r);
+}
+
 // nn.LayerNorm(C, eps) per pixel: y = (x - mean) / sqrt(var + eps) * gamma + beta, biased variance, fp32 statistics
 // (two passes over the pixel's C channels: mean, then centred sum of squares; the second and third reads hit L1/L2).
 // A warp covers 8 consecutive pixels x 4 channel slices (lane = slice * 8 + pixel): every load is a 128-byte row of one channel
@@ -34,6 +52,9 @@ __device__ __forceinline__ uint4 pack8(const float* v) {
 // walked 64 groups three times at the coarse MiT stages (33 us for 8 MB); this is 4x shorter and has 4x the threads.
 // Optionally also writes the space-to-depth copy dst2 ([h/2][w/2] pixels, channel block (y%2)*2 + x%2).
 // HBM-bound: 2 B read + 2 (or 4) B written per element.
+// SPLIT: src, dst and dst2 hold hi and lo planes (lowering.Program.precision); the statistics run over hi + lo and both planes are
+// written (dst2's lo plane of class k, channel ch sits at channel 4C + k*C + ch).
+template <bool SPLIT>
 __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ dst,
                                                         __nv_bfloat16* __restrict__ dst2, const float* __restrict__ gamma,
                                                         const float* __restrict__ beta, int B, int C, int src_c8, int dst_c8,
@@ -49,10 +70,12 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
     const size_t b = i / hw;
     const int pix = static_cast<int>(i - b * hw);
     const __nv_bfloat16* s = src + (b * src_c8 * hw + pix) * 8;
+    const size_t s_lo = static_cast<size_t>(src_c8 >> 1) * hw * 8;        // split: offset of the lo plane
     float sum = 0.f;
     for (int g = slice; g < g8; g += 4) {
       float v[8];
-      unpack8(__ldg(reinterpret_cast<const uint4*>(s + static_cast<size_t>(g) * hw * 8)), v);
+      if constexpr (SPLIT) load8_split(s + static_cast<size_t>(g) * hw * 8, s_lo, v);
+      else unpack8(__ldg(reinterpret_cast<const uint4*>(s + static_cast<size_t>(g) * hw * 8)), v);
 #pragma unroll
       for (int j = 0; j < 8; ++j) sum += v[j];
     }
@@ -62,7 +85,8 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
     float sq = 0.f;
     for (int g = slice; g < g8; g += 4) {
       float v[8];
-      unpack8(__ldg(reinterpret_cast<const uint4*>(s + static_cast<size_t>(g) * hw * 8)), v);
+      if constexpr (SPLIT) load8_split(s + static_cast<size_t>(g) * hw * 8, s_lo, v);
+      else unpack8(__ldg(reinterpret_cast<const uint4*>(s + static_cast<size_t>(g) * hw * 8)), v);
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         const float d = v[j] - mean;
@@ -83,16 +107,28 @@ __global__ void __launch_bounds__(256) layernorm_kernel(const __nv_bfloat16* __r
     if (!live) continue;
     for (int g = slice; g < g8; g += 4) {
       float v[8];
-      unpack8(__ldg(reinterpret_cast<const uint4*>(s + static_cast<size_t>(g) * hw * 8)), v);
+      if constexpr (SPLIT) load8_split(s + static_cast<size_t>(g) * hw * 8, s_lo, v);
+      else unpack8(__ldg(reinterpret_cast<const uint4*>(s + static_cast<size_t>(g) * hw * 8)), v);
       const float4 g0 = __ldg(reinterpret_cast<const float4*>(gamma + g * 8)), g1 = __ldg(reinterpret_cast<const float4*>(gamma + g * 8 + 4));
       const float4 b0 = __ldg(reinterpret_cast<const float4*>(beta + g * 8)), b1 = __ldg(reinterpret_cast<const float4*>(beta + g * 8 + 4));
       const float gm[8] = {g0.x, g0.y, g0.z, g0.w, g1.x, g1.y, g1.z, g1.w};
       const float bt[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = fmaf((v[j] - mean) * rstd, gm[j], bt[j]);
-      const uint4 q = pack8(v);
-      *reinterpret_cast<uint4*>(o + static_cast<size_t>(g) * hw * 8) = q;
-      if (o2 != nullptr) *reinterpret_cast<uint4*>(o2 + static_cast<size_t>(g) * hw2 * 8) = q;
+      if constexpr (SPLIT) {
+        uint4 qh, ql;
+        split8(v, qh, ql);
+        *reinterpret_cast<uint4*>(o + static_cast<size_t>(g) * hw * 8) = qh;
+        *reinterpret_cast<uint4*>(o + (static_cast<size_t>(g) + (dst_c8 >> 1)) * hw * 8) = ql;
+        if (o2 != nullptr) {
+          *reinterpret_cast<uint4*>(o2 + static_cast<size_t>(g) * hw2 * 8) = qh;
+          *reinterpret_cast<uint4*>(o2 + (static_cast<size_t>(g) + (dst2_c8 >> 1)) * hw2 * 8) = ql;
+        }
+      } else {
+        const uint4 q = pack8(v);
+        *reinterpret_cast<uint4*>(o + static_cast<size_t>(g) * hw * 8) = q;
+        if (o2 != nullptr) *reinterpret_cast<uint4*>(o2 + static_cast<size_t>(g) * hw2 * 8) = q;
+      }
     }
   }
 }
@@ -199,6 +235,8 @@ __global__ void __launch_bounds__(128) sr_attention_kernel(const __nv_bfloat16* 
 // produces 4 horizontally adjacent pixels from a 3 x 6 window, so every loaded and unpacked neighbour feeds up to three taps, the MACs
 // run as packed FFMA2 over channel pairs and the GELU on packed pairs.  The first version (one pixel per thread, scalar math) measured
 // at the SM's issue limit (330 instructions per 8 outputs, 171 us against a 41 us HBM floor at stage 1); this one issues ~180.
+// SPLIT: src and dst hold hi and lo planes; the taps read hi + lo, the output is written as both planes.
+template <bool SPLIT>
 __global__ void __launch_bounds__(128) dwconv3x3_kernel(const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ dst,
                                                         const float* __restrict__ wgt, const float* __restrict__ bias, int B, int g8,
                                                         int src_c8, int dst_c8, int h, int w, int gelu) {
@@ -212,6 +250,7 @@ __global__ void __launch_bounds__(128) dwconv3x3_kernel(const __nv_bfloat16* __r
   __syncthreads();
   const __nv_bfloat16* base = src + (b * src_c8 + g) * static_cast<size_t>(hw) * 8;
   __nv_bfloat16* obase = dst + (b * dst_c8 + g) * static_cast<size_t>(hw) * 8;
+  const size_t s_lo = static_cast<size_t>(src_c8 >> 1) * hw * 8, d_lo = static_cast<size_t>(dst_c8 >> 1) * hw * 8;   // split planes
   const int xg = (w + 3) >> 2;                                   // groups of 4 pixels per row
   for (int item = blockIdx.x * blockDim.x + threadIdx.x; item < xg * h; item += gridDim.x * blockDim.x) {
     const int y = item / xg, x0 = (item - y * xg) * 4;
@@ -228,12 +267,15 @@ __global__ void __launch_bounds__(128) dwconv3x3_kernel(const __nv_bfloat16* __r
     for (int ky = 0; ky < 3; ++ky) {
       const int yy = y + ky - 1;
       const bool row_ok = yy >= 0 && yy < h;
-      uint4 q[6];
+      uint4 q[6], ql[6];
 #pragma unroll
       for (int c = 0; c < 6; ++c) {                              // the row's six loads first: independent, in flight together
         const int xx = x0 + c - 1;
         q[c] = (row_ok && xx >= 0 && xx < w) ? __ldg(reinterpret_cast<const uint4*>(base + (static_cast<size_t>(yy) * w + xx) * 8))
                                              : make_uint4(0u, 0u, 0u, 0u);
+        if constexpr (SPLIT)
+          ql[c] = (row_ok && xx >= 0 && xx < w) ? __ldg(reinterpret_cast<const uint4*>(base + s_lo + (static_cast<size_t>(yy) * w + xx) * 8))
+                                                : make_uint4(0u, 0u, 0u, 0u);
       }
       float2 wk[3][4];
 #pragma unroll
@@ -246,6 +288,12 @@ __global__ void __launch_bounds__(128) dwconv3x3_kernel(const __nv_bfloat16* __r
       for (int c = 0; c < 6; ++c) {
         float v[8];
         unpack8(q[c], v);
+        if constexpr (SPLIT) {
+          float l[8];
+          unpack8(ql[c], l);
+#pragma unroll
+          for (int j = 0; j < 8; ++j) v[j] += l[j];
+        }
         const float2 vp[4] = {make_float2(v[0], v[1]), make_float2(v[2], v[3]), make_float2(v[4], v[5]), make_float2(v[6], v[7])};
 #pragma unroll
         for (int kx = 0; kx < 3; ++kx) {
@@ -266,7 +314,14 @@ __global__ void __launch_bounds__(128) dwconv3x3_kernel(const __nv_bfloat16* __r
           const float2 r = gelu ? gelu_fast2(acc[p][e]) : acc[p][e];
           o[2 * e] = r.x, o[2 * e + 1] = r.y;
         }
-        *reinterpret_cast<uint4*>(obase + (static_cast<size_t>(y) * w + x0 + p) * 8) = pack8(o);
+        if constexpr (SPLIT) {
+          uint4 oh, olo;
+          split8(o, oh, olo);
+          *reinterpret_cast<uint4*>(obase + (static_cast<size_t>(y) * w + x0 + p) * 8) = oh;
+          *reinterpret_cast<uint4*>(obase + d_lo + (static_cast<size_t>(y) * w + x0 + p) * 8) = olo;
+        } else {
+          *reinterpret_cast<uint4*>(obase + (static_cast<size_t>(y) * w + x0 + p) * 8) = pack8(o);
+        }
       }
     }
   }
@@ -280,13 +335,24 @@ __global__ void __launch_bounds__(128) dwconv3x3_kernel(const __nv_bfloat16* __r
 // registers.  K ([key][d]) and V^T ([d][key]) of the (image, head) sit in shared memory as bf16 with padded rows (no bank conflicts
 // on the B-fragment loads).  Q, K, V are bf16 tensors already; P is rounded to bf16 for the second product (one more bf16 rounding
 // on a path that is bf16 end to end).  grid (N / 64, heads, images), 128 threads.
-template <int D>   // head dim: 64 or 80 (multiples of 16)
+// SPLIT (lowering.Program.precision): q, kv and out hold hi and lo planes.  K and V^T are staged as both planes (45 KB at D = 80),
+// S = Qh Kh + Ql Kh + Qh Kl and O = Ph Vh + Pl Vh + Ph Vl (three mma.sync per tile; the lo x lo term is below 2^-16 relative) with
+// P = exp(s - max) split into hi = bf16(P), lo = bf16(P - hi) after the fp32 softmax; the output is normalised by the fp32 row sum
+// and written as both planes.
+__device__ __forceinline__ void split_bf16x2(float a, float b, uint32_t& hi, uint32_t& lo) {
+  hi = pack_bf16x2(a, b);
+  const __nv_bfloat162 h = *reinterpret_cast<const __nv_bfloat162*>(&hi);
+  lo = pack_bf16x2(a - __low2float(h), b - __high2float(h));
+}
+
+template <int D, bool SPLIT>   // head dim: 64 or 80 (multiples of 16)
 __global__ void __launch_bounds__(128) sr_attention_mma_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ kv,
                                                                __nv_bfloat16* __restrict__ out, int C, int q_c8, int kv_c8, int out_c8,
                                                                int N, float scale) {
   constexpr int NK = 64, KS = D + 8, VS = NK + 8;              // padded row strides (bf16 elements)
-  __shared__ __align__(16) __nv_bfloat16 sk[NK * KS];          // K [key][d]
-  __shared__ __align__(16) __nv_bfloat16 svt[D * VS];          // V^T [d][key]
+  constexpr int NP = SPLIT ? 2 : 1;                            // planes: hi [, lo]
+  __shared__ __align__(16) __nv_bfloat16 sk[NP * NK * KS];     // K [plane][key][d]
+  __shared__ __align__(16) __nv_bfloat16 svt[NP * D * VS];     // V^T [plane][d][key]
   const int b = blockIdx.z, hd = blockIdx.y;
   const int g0 = hd * (D / 8);
   for (int i = threadIdx.x; i < NK * (D / 8); i += blockDim.x) {
@@ -297,6 +363,18 @@ __global__ void __launch_bounds__(128) sr_attention_mma_kernel(const __nv_bfloat
     const __nv_bfloat16* ve = reinterpret_cast<const __nv_bfloat16*>(&vq);
 #pragma unroll
     for (int e = 0; e < 8; ++e) svt[(g * 8 + e) * VS + j] = ve[e];
+  }
+  if constexpr (SPLIT) {
+    const int lo = kv_c8 >> 1;                                 // first channel group of the lo plane
+    for (int i = threadIdx.x; i < NK * (D / 8); i += blockDim.x) {
+      const int j = i % NK, g = i / NK;
+      const uint4 kq = __ldg(reinterpret_cast<const uint4*>(kv + ((static_cast<size_t>(b) * kv_c8 + lo + g0 + g) * NK + j) * 8));
+      *reinterpret_cast<uint4*>(&sk[NK * KS + j * KS + g * 8]) = kq;
+      const uint4 vq = __ldg(reinterpret_cast<const uint4*>(kv + ((static_cast<size_t>(b) * kv_c8 + lo + (C >> 3) + g0 + g) * NK + j) * 8));
+      const __nv_bfloat16* ve = reinterpret_cast<const __nv_bfloat16*>(&vq);
+#pragma unroll
+      for (int e = 0; e < 8; ++e) svt[D * VS + (g * 8 + e) * VS + j] = ve[e];
+    }
   }
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -318,10 +396,23 @@ __global__ void __launch_bounds__(128) sr_attention_mma_kernel(const __nv_bfloat
     a[1] = __ldg(reinterpret_cast<const uint32_t*>(q0 + static_cast<size_t>(nb) * 8 + cq));
     a[2] = __ldg(reinterpret_cast<const uint32_t*>(q1 + static_cast<size_t>(na) * 8 + cq));
     a[3] = __ldg(reinterpret_cast<const uint32_t*>(q1 + static_cast<size_t>(nb) * 8 + cq));
+    uint32_t al[4];
+    if constexpr (SPLIT) {
+      const size_t lo = static_cast<size_t>(q_c8 >> 1) * N * 8;
+      al[0] = __ldg(reinterpret_cast<const uint32_t*>(q0 + lo + static_cast<size_t>(na) * 8 + cq));
+      al[1] = __ldg(reinterpret_cast<const uint32_t*>(q0 + lo + static_cast<size_t>(nb) * 8 + cq));
+      al[2] = __ldg(reinterpret_cast<const uint32_t*>(q1 + lo + static_cast<size_t>(na) * 8 + cq));
+      al[3] = __ldg(reinterpret_cast<const uint32_t*>(q1 + lo + static_cast<size_t>(nb) * 8 + cq));
+    }
 #pragma unroll
     for (int t = 0; t < 8; ++t) {
       const __nv_bfloat16* kr = &sk[(t * 8 + r) * KS + ks * 16 + cq];
       mma_bf16_16816(sacc[t], a, *reinterpret_cast<const uint32_t*>(kr), *reinterpret_cast<const uint32_t*>(kr + 8));
+      if constexpr (SPLIT) {
+        const __nv_bfloat16* kl = kr + NK * KS;
+        mma_bf16_16816(sacc[t], al, *reinterpret_cast<const uint32_t*>(kr), *reinterpret_cast<const uint32_t*>(kr + 8));
+        mma_bf16_16816(sacc[t], a, *reinterpret_cast<const uint32_t*>(kl), *reinterpret_cast<const uint32_t*>(kl + 8));
+      }
     }
   }
   // ---- softmax over the 64 keys of rows r (values [t][0..1]) and r + 8 (values [t][2..3]); a row lives in the 4 lanes of a quad
@@ -337,14 +428,20 @@ __global__ void __launch_bounds__(128) sr_attention_mma_kernel(const __nv_bfloat
   mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
   float sum0 = 0.f, sum1 = 0.f;
   uint32_t pa[4][4];                                           // P as A fragments: k-step = 16 keys = two key tiles
+  uint32_t pl[4][4];                                           // split: the lo plane of P
 #pragma unroll
   for (int t = 0; t < 8; ++t) {
     const float p0 = __expf((sacc[t][0] - mx0) * scale), p1 = __expf((sacc[t][1] - mx0) * scale);
     const float p2 = __expf((sacc[t][2] - mx1) * scale), p3 = __expf((sacc[t][3] - mx1) * scale);
     sum0 += p0 + p1;
     sum1 += p2 + p3;
-    pa[t >> 1][(t & 1) * 2] = pack_bf16x2(p0, p1);
-    pa[t >> 1][(t & 1) * 2 + 1] = pack_bf16x2(p2, p3);
+    if constexpr (SPLIT) {
+      split_bf16x2(p0, p1, pa[t >> 1][(t & 1) * 2], pl[t >> 1][(t & 1) * 2]);
+      split_bf16x2(p2, p3, pa[t >> 1][(t & 1) * 2 + 1], pl[t >> 1][(t & 1) * 2 + 1]);
+    } else {
+      pa[t >> 1][(t & 1) * 2] = pack_bf16x2(p0, p1);
+      pa[t >> 1][(t & 1) * 2 + 1] = pack_bf16x2(p2, p3);
+    }
   }
   sum0 += __shfl_xor_sync(0xffffffffu, sum0, 1);
   sum0 += __shfl_xor_sync(0xffffffffu, sum0, 2);
@@ -360,9 +457,29 @@ __global__ void __launch_bounds__(128) sr_attention_mma_kernel(const __nv_bfloat
     for (int ks = 0; ks < 4; ++ks) {
       const __nv_bfloat16* vr = &svt[(t * 8 + r) * VS + ks * 16 + cq];
       mma_bf16_16816(o, pa[ks], *reinterpret_cast<const uint32_t*>(vr), *reinterpret_cast<const uint32_t*>(vr + 8));
+      if constexpr (SPLIT) {
+        const __nv_bfloat16* vl = vr + D * VS;
+        mma_bf16_16816(o, pl[ks], *reinterpret_cast<const uint32_t*>(vr), *reinterpret_cast<const uint32_t*>(vr + 8));
+        mma_bf16_16816(o, pa[ks], *reinterpret_cast<const uint32_t*>(vl), *reinterpret_cast<const uint32_t*>(vl + 8));
+      }
     }
-    if (n0 + r < N) *reinterpret_cast<uint32_t*>(ob + (static_cast<size_t>(t) * N + n0 + r) * 8 + cq) = pack_bf16x2(o[0] * inv0, o[1] * inv0);
-    if (n0 + r + 8 < N) *reinterpret_cast<uint32_t*>(ob + (static_cast<size_t>(t) * N + n0 + r + 8) * 8 + cq) = pack_bf16x2(o[2] * inv1, o[3] * inv1);
+    if constexpr (SPLIT) {
+      const size_t lo = static_cast<size_t>(out_c8 >> 1) * N * 8;
+      uint32_t h, l;
+      if (n0 + r < N) {
+        split_bf16x2(o[0] * inv0, o[1] * inv0, h, l);
+        *reinterpret_cast<uint32_t*>(ob + (static_cast<size_t>(t) * N + n0 + r) * 8 + cq) = h;
+        *reinterpret_cast<uint32_t*>(ob + lo + (static_cast<size_t>(t) * N + n0 + r) * 8 + cq) = l;
+      }
+      if (n0 + r + 8 < N) {
+        split_bf16x2(o[2] * inv1, o[3] * inv1, h, l);
+        *reinterpret_cast<uint32_t*>(ob + (static_cast<size_t>(t) * N + n0 + r + 8) * 8 + cq) = h;
+        *reinterpret_cast<uint32_t*>(ob + lo + (static_cast<size_t>(t) * N + n0 + r + 8) * 8 + cq) = l;
+      }
+    } else {
+      if (n0 + r < N) *reinterpret_cast<uint32_t*>(ob + (static_cast<size_t>(t) * N + n0 + r) * 8 + cq) = pack_bf16x2(o[0] * inv0, o[1] * inv0);
+      if (n0 + r + 8 < N) *reinterpret_cast<uint32_t*>(ob + (static_cast<size_t>(t) * N + n0 + r + 8) * 8 + cq) = pack_bf16x2(o[2] * inv1, o[3] * inv1);
+    }
   }
 }
 

@@ -184,6 +184,7 @@ class LayerNormSpec:
     beta: np.ndarray
     eps: float
     dst_s2d: Optional[str] = None
+    split: bool = False          # split precision: reads hi + lo, writes both planes of dst (and of dst_s2d: lo of class k at 4c + k*c)
 
 
 @dataclass
@@ -199,6 +200,7 @@ class AttentionSpec:
     heads: int
     scale: float
     macs_per_pair: int = 0
+    split: bool = False          # split precision: S = QhKh + QlKh + QhKl, O = PhVh + PlVh + PhVl (P split after the fp32 softmax)
 
 
 @dataclass
@@ -212,6 +214,7 @@ class DWConvSpec:
     bias: np.ndarray             # float32 [c]
     gelu: bool = True
     macs_per_pair: int = 0
+    split: bool = False          # split precision: reads hi + lo, writes both planes
 
 
 @dataclass
@@ -223,6 +226,7 @@ class BilinearUpSpec:
     dst: str
     c: int
     scale: int
+    split: bool = False          # split precision: reads hi + lo, writes both planes
 
 
 @dataclass
@@ -942,10 +946,20 @@ def add_conv(
         raise ValueError(f"{name}: act_pre needs the second affine")
     split = prog.split
     if split:
-        if out0_s2d or act_kind not in (0, 1) or act_pre:
-            raise NotImplementedError(f"{name}: split precision covers the ReLU conv families (FC-Siam, SNUNet)")
+        if out0_s2d:
+            raise NotImplementedError(f"{name}: split precision has no space-to-depth store")
         fold = False                # folded / horizontally folded forms keep their specialised bf16 epilogues
         segs, phase_taps = _split_operands(prog, name, segs, phase_taps)
+        parts = _k_partition(prog, name, segs, phase_taps, cout, pair, max_kc)
+        if len(parts) > 1:
+            plain = (res is None and out_raw is None and out_pool is None and out_diff is None and out_ext < 0 and scale2 is None
+                     and out0 is not None and len(phase_taps) == 1 and osy == 1 and osx == 1)
+            if not plain:
+                raise NotImplementedError(f"{name}: the split K-program is too long and only single-phase affine + activation + out0 "
+                                          "ops are partitioned along K")
+            return _add_k_partitioned(prog, name, segs, phase_taps, parts, cout, hg, wg, img_mult, scale, shift, pair=pair,
+                                      out0=out0, out0_coff=out0_coff, macs_per_pair=macs_per_pair, act_kind=act_kind,
+                                      act_alpha=act_alpha, max_kc=max_kc)
     fold_cs = fold_cout = 0
     plain_out = (res is None and out_raw is None and out_pool is None and out_diff is None and out_ext < 0
                  and scale2 is None and not out0_s2d and out0 is not None)
@@ -1003,6 +1017,94 @@ def add_conv(
         fold_cs=fold_cs, fold_cout=fold_cout, act_kind=act_kind, act_alpha=float(act_alpha), act_pre=act_pre,
         xf_cs=xf_cs, split=split,
     )
+    prog.ops.append(spec)
+    return spec
+
+
+def _k_program_len(prog: Program, name: str, segs: Sequence[Segment], taps, cout: int, pair: bool, max_kc: int,
+                   res: bool) -> Tuple[int, int]:
+    """(chunks, weight blocks) of ONE phase's K-program as ``_taps_to_gemm`` would build it (``taps``: that phase's SegTaps),
+    with the chunk width ``add_conv`` picks for an op with (``res``) or without a residual."""
+    if res and pair and cout <= 64:
+        max_kc = min(max_kc, 32)
+    stored_c = [(prog.tensors[s.tensor].c - s.c_off) if s.c_store < 0 else s.c_store for s in segs]
+    per_seg = _split_taps(name, segs, taps)
+    kc = choose_kc(stored_c, max(1, max((len(t) for t in per_seg), default=1)), cap=max_kc if max_kc < 64 else 112)
+    n_chunks = n_blocks = 0
+    for s, sc, t in zip(segs, stored_c, per_seg):
+        if not t:
+            continue
+        k_blocks = sum(1 for c0 in range(0, sc, kc) if c0 < s.c_real)
+        n_chunks += k_blocks * (1 if s.sy == 1 and s.sx == 1 else len(t))
+        n_blocks += k_blocks * len(t)
+    return n_chunks, n_blocks
+
+
+def _k_partition(prog: Program, name: str, segs: Sequence[Segment], phase_taps, cout: int, pair: bool, max_kc: int) -> List[range]:
+    """Split programs only: the segment ranges of the fewest launches whose K-programs fit the kernel's per-phase tables
+    (MAX_CHUNKS / MAX_TAPS).  The split form triples every K-program, so a few ops that fit in bf16 (the 7x7 stride-4 patch
+    embedding, 8x8 stride-8 spatial reduction) outgrow them.  Cuts fall on segment boundaries; the last launch reads the partial
+    sum as its residual, so it is sized with the residual's chunk width.  One range = no partitioning."""
+    whole = range(len(segs))
+    if len(phase_taps) != 1:
+        return [whole]
+    taps = _split_taps(name, segs, phase_taps[0][2])
+
+    def fits(lo: int, hi: int, res: bool) -> bool:
+        n_c, n_b = _k_program_len(prog, name, segs[lo:hi], SegTaps(taps[lo:hi]), cout, pair, max_kc, res)
+        return n_c <= MAX_CHUNKS and n_b <= MAX_TAPS
+
+    if fits(0, len(segs), False):
+        return [whole]
+    parts: List[range] = []
+    hi, res = len(segs), True          # packed from the back: the last launch is the one with the residual
+    while hi > 0:
+        lo = hi - 1
+        if not fits(lo, hi, res):
+            raise ValueError(f"{name}: one K segment alone exceeds the K-program tables")
+        while lo > 0 and fits(lo - 1, hi, res):
+            lo -= 1
+        parts.insert(0, range(lo, hi))
+        hi, res = lo, False
+    return parts
+
+
+def _add_k_partitioned(prog: Program, name: str, segs: Sequence[Segment], phase_taps, parts: List[range], cout: int, hg: int, wg: int,
+                       img_mult: int, scale: np.ndarray, shift: np.ndarray, *, pair: bool, out0: str, out0_coff: int,
+                       macs_per_pair: int, act_kind: int, act_alpha: float, max_kc: int) -> ConvSpec:
+    """One split conv as len(parts) launches along K: launch i < last writes acc_i*scale (+ launch i-1's partial) to the split
+    intermediate ``{name}.part{i}``; the last computes acc*scale + shift + partial, then the activation, into out0.  Each
+    intermediate rounds to hi + lo (16 mantissa bits), like every other split activation."""
+    oy, ox, taps = phase_taps[0]
+    taps = _split_taps(name, segs, taps)
+    t0 = prog.tensors[out0]
+    mult = 2 if pair else img_mult
+    zero = np.zeros_like(np.asarray(shift, np.float32))
+    prev = None
+    for i, r in enumerate(parts[:-1]):
+        part = prog.tensor(f"{name}.part{i}", mult, t0.h, t0.w, cout)
+        _emit_conv(prog, f"{name}.part{i}", [segs[j] for j in r], [(oy, ox, SegTaps(taps[j] for j in r))], cout, hg, wg, img_mult,
+                   scale, zero, pair=pair, res=prev, out0=part, split=True, max_kc=max_kc)
+        prev = part
+    r = parts[-1]
+    return _emit_conv(prog, name, [segs[j] for j in r], [(oy, ox, SegTaps(taps[j] for j in r))], cout, hg, wg, img_mult, scale, shift,
+                      pair=pair, res=prev, out0=out0, out0_coff=out0_coff, macs_per_pair=macs_per_pair, act_kind=act_kind,
+                      act_alpha=act_alpha, split=True, max_kc=max_kc)
+
+
+def _emit_conv(prog: Program, name: str, segs, phase_taps, cout: int, hg: int, wg: int, img_mult: int, scale: np.ndarray,
+               shift: np.ndarray, *, pair: bool, res: Optional[str], out0: str, split: bool, max_kc: int, out0_coff: int = 0,
+               macs_per_pair: int = 0, act_kind: int = 0, act_alpha: float = 0.0) -> ConvSpec:
+    """One launch of a K-partitioned split conv (single phase, out0 store, no folding)."""
+    if res is not None and pair and cout <= 64:
+        max_kc = min(max_kc, 32)
+    wbits, kc, n_tile, cout_pad, phases, chunks, taps, srcs, sy, sx, ey, ex = _taps_to_gemm(prog, name, segs, phase_taps, cout, pair, max_kc)
+    spec = ConvSpec(
+        name=name, srcs=srcs, src_sy=sy, src_sx=sx, src_ey=ey, src_ex=ex, hg=hg, wg=wg, img_mult=img_mult, pair=pair,
+        weights=wbits, kc=kc, n_tile=n_tile, cout=cout, cout_pad=cout_pad, phases=phases, chunks=chunks, taps=taps,
+        osy=1, osx=1, scale=_pad_vec(scale, cout_pad, 1.0), shift=_pad_vec(shift, cout_pad, 0.0),
+        relu=act_kind != 0, res=res, out0=out0, out0_coff=out0_coff, macs_per_pair=macs_per_pair, act_kind=act_kind,
+        act_alpha=float(act_alpha), split=split)
     prog.ops.append(spec)
     return spec
 
@@ -1084,16 +1186,16 @@ def op_bytes_per_pair(prog: Program, op) -> int:
         return t.mult * (2 * op.c * t.h * t.w * 2 + (0 if op.relpos is None else op.relpos.size * 4))
     if isinstance(op, LayerNormSpec):
         t = T[op.src]
-        return t.mult * op.c * t.h * t.w * 2 * (2 if op.dst_s2d is None else 3)
+        return t.mult * op.c * t.h * t.w * 2 * (2 if op.dst_s2d is None else 3) * (2 if op.split else 1)
     if isinstance(op, DWConvSpec):
         t = T[op.src]
-        return t.mult * op.c * t.h * t.w * 2 * 2
+        return t.mult * op.c * t.h * t.w * 2 * 2 * (2 if op.split else 1)
     if isinstance(op, AttentionSpec):
         tq, tk = T[op.q], T[op.kv]
-        return tq.mult * (2 * op.c * tq.h * tq.w * 2 + 2 * op.c * tk.h * tk.w * 2)
+        return tq.mult * (2 * op.c * tq.h * tq.w * 2 + 2 * op.c * tk.h * tk.w * 2) * (2 if op.split else 1)
     if isinstance(op, BilinearUpSpec):
         t = T[op.dst]
-        return t.mult * (op.c * t.h * t.w * 2 + op.c * t.h * t.w * 2 // (op.scale * op.scale))
+        return t.mult * (op.c * t.h * t.w * 2 + op.c * t.h * t.w * 2 // (op.scale * op.scale)) * (2 if op.split else 1)
     if isinstance(op, ConvSpec):
         imgs = 2 if op.pair else op.img_mult
         seen, byt = set(), 0

@@ -116,17 +116,19 @@ class Plan:
                 _lib.check_id(lib.stcd_plan_add_sum(h, arr, len(op.srcs), ids[op.dst]), f"sum {op.name}")
             elif isinstance(op, LayerNormSpec):
                 g, b = np.ascontiguousarray(op.gamma, np.float32), np.ascontiguousarray(op.beta, np.float32)
-                _lib.check_id(lib.stcd_plan_add_layernorm(h, ids[op.src], ids[op.dst], -1 if op.dst_s2d is None else ids[op.dst_s2d],
-                                                          op.c, _fptr(g), _fptr(b), float(op.eps)), f"layer norm {op.name}")
+                add = lib.stcd_plan_add_layernorm_split if op.split else lib.stcd_plan_add_layernorm
+                _lib.check_id(add(h, ids[op.src], ids[op.dst], -1 if op.dst_s2d is None else ids[op.dst_s2d], op.c, _fptr(g), _fptr(b),
+                                  float(op.eps)), f"layer norm {op.name}")
             elif isinstance(op, AttentionSpec):
-                _lib.check_id(lib.stcd_plan_add_sr_attention(h, ids[op.q], ids[op.kv], ids[op.dst], op.c, op.heads, float(op.scale)),
-                              f"attention {op.name}")
+                add = lib.stcd_plan_add_sr_attention_split if op.split else lib.stcd_plan_add_sr_attention
+                _lib.check_id(add(h, ids[op.q], ids[op.kv], ids[op.dst], op.c, op.heads, float(op.scale)), f"attention {op.name}")
             elif isinstance(op, DWConvSpec):
                 wt, b = np.ascontiguousarray(op.weight, np.float32), np.ascontiguousarray(op.bias, np.float32)
-                _lib.check_id(lib.stcd_plan_add_dwconv3x3(h, ids[op.src], ids[op.dst], op.c, _fptr(wt), _fptr(b), 1 if op.gelu else 0),
-                              f"dw conv {op.name}")
+                add = lib.stcd_plan_add_dwconv3x3_split if op.split else lib.stcd_plan_add_dwconv3x3
+                _lib.check_id(add(h, ids[op.src], ids[op.dst], op.c, _fptr(wt), _fptr(b), 1 if op.gelu else 0), f"dw conv {op.name}")
             elif isinstance(op, BilinearUpSpec):
-                _lib.check_id(lib.stcd_plan_add_bilinear_up(h, ids[op.src], ids[op.dst], op.c, op.scale), f"bilinear {op.name}")
+                add = lib.stcd_plan_add_bilinear_up_split if op.split else lib.stcd_plan_add_bilinear_up
+                _lib.check_id(add(h, ids[op.src], ids[op.dst], op.c, op.scale), f"bilinear {op.name}")
             elif isinstance(op, MaxPoolS2DSpec):
                 _lib.check_id(lib.stcd_plan_add_maxpool_s2d(h, ids[op.src], ids[op.dst], op.c), f"maxpool {op.name}")
             elif isinstance(op, SegHeadSpec):
