@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define STCD_ABI_VERSION 19
+#define STCD_ABI_VERSION 20
 
 enum stcd_status {
   STCD_OK = 0,
@@ -171,8 +171,8 @@ typedef struct stcd_conv_desc {
    * itself computes in fp32, models/SNUNet.py:116-152).  split = 1: every bf16 tensor this op touches stores 2x its logical
    * channels -- a hi plane bf16(v) in channel groups [0, c8/2) and a lo plane bf16(v - hi) in [c8/2, c8) -- the K-program
    * (built by the host) reads each logical source as the three segments (hi, lo, hi) against the weights (Whi, Whi, Wlo), the
-   * epilogue writes both planes of out0 / out_raw / out_pool / out_diff and reads the residual as hi + lo.  Not combined
-   * with out0_s2d, fold_cs or xf_cs. */
+   * epilogue writes both planes of out0 / out_raw / out_pool / out_diff and reads the residual as hi + lo.  A space-to-depth
+   * out0 stores 8*cout channels: hi of parity class k at k*cout, lo at 4*cout + k*cout.  Not combined with fold_cs or xf_cs. */
   int32_t split;
 } stcd_conv_desc;
 
@@ -328,6 +328,23 @@ int stcd_plan_add_sr_attention_split(stcd_plan* plan, int q_tensor, int kv_tenso
 int stcd_plan_add_dwconv3x3_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, const float* weight, const float* bias,
                                   int gelu);
 int stcd_plan_add_bilinear_up_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int scale);
+
+/* Split-precision variants of the ResNet-family ops (BIT, DTCDSCN), same arguments as the functions above and the same hi + lo
+ * layout; each reads hi + lo, computes in fp32 in the order of its bf16 form and writes hi = bf16(v), lo = bf16(v - hi).
+ * input_pack_s2d_split: dst stores 32 channels, the hi plane in [0, 16) (channel (py*2 + px)*cin + c), the lo plane in [16, 32).
+ * maxpool_s2d_split: src stores 8c channels (hi of parity class k at k*c, lo at 4c + k*c), dst 2c; the max over hi + lo selects
+ *   the winning (hi, lo) pair (first maximum in the kernel's window order).
+ * absdiff_split, subdiff_split, sum_split: every tensor stores hi and lo planes (channels a multiple of 16).
+ * channel_gate_split: src, res, dst store 2c channels; the space-to-depth copy 8c (as layernorm_split's).
+ * bit_transformer_split: src and dst store 64 channels (2 x 32); the token path itself is fp32 in both forms. */
+int stcd_plan_add_input_pack_s2d_split(stcd_plan* plan, int dst_tensor, int cin);
+int stcd_plan_add_maxpool_s2d_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c);
+int stcd_plan_add_absdiff_split(stcd_plan* plan, int src_tensor, int dst_tensor);
+int stcd_plan_add_subdiff_split(stcd_plan* plan, int src_tensor, int add_or_neg, int dst_tensor);
+int stcd_plan_add_sum_split(stcd_plan* plan, const int* src_tensors, int n, int dst_tensor);
+int stcd_plan_add_channel_gate_split(stcd_plan* plan, int src_tensor, int res_or_neg, int dst_tensor, int dst_s2d_or_neg, int c,
+                                     int hid, const float* w1, const float* w2, const float* ws_or_null, int mode);
+int stcd_plan_add_bit_transformer_split(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* desc);
 
 /* SNUNet's ECAM tail (models/SNUNet.py:144-149: two ChannelAttention blocks :46-59 + conv_final)
  * over four activation tensors of `c` channels each, as one fused op writing external output

@@ -174,7 +174,7 @@ class EcamDesc(C.Structure):
     ]
 
 
-ABI_VERSION = 19
+ABI_VERSION = 20
 
 # every symbol include/stcd_b200.h declares: (name, restype, argtypes)
 SYMBOLS = [
@@ -215,6 +215,14 @@ SYMBOLS = [
     ("stcd_plan_add_sr_attention_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float]),
     ("stcd_plan_add_dwconv3x3_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int]),
     ("stcd_plan_add_bilinear_up_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]),
+    ("stcd_plan_add_input_pack_s2d_split", C.c_int, [C.c_void_p, C.c_int, C.c_int]),
+    ("stcd_plan_add_maxpool_s2d_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
+    ("stcd_plan_add_absdiff_split", C.c_int, [C.c_void_p, C.c_int, C.c_int]),
+    ("stcd_plan_add_subdiff_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
+    ("stcd_plan_add_sum_split", C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_int, C.c_int]),
+    ("stcd_plan_add_channel_gate_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float),
+                                                   C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int]),
+    ("stcd_plan_add_bit_transformer_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     ("stcd_plan_add_ecam_head", C.c_int, [C.c_void_p, C.c_void_p]),
     ("stcd_plan_finalize", C.c_int, [C.c_void_p]),
     ("stcd_plan_tensor_copy", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_int]),

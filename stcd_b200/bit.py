@@ -118,6 +118,7 @@ class _Transformer(nn.Module):
 class ResNet(PlannedModule):
     """models/networks.py:223-305."""
     default_chunk_pairs = 32
+    supports_precision_path = True
 
     def __init__(self, input_nc: int, output_nc: int, resnet_stages_num: int = 5, backbone: str = "resnet18",
                  output_sigmoid: bool = False, if_upsample_2x: bool = True):
@@ -139,7 +140,7 @@ class ResNet(PlannedModule):
         self.output_sigmoid = output_sigmoid
 
     def lower(self, h: int, w: int) -> L.Program:
-        return lower_bit(self.state_dict(), self.input_nc, self.output_nc, self.resnet_stages_num, None, h, w)
+        return lower_bit(self.state_dict(), self.input_nc, self.output_nc, self.resnet_stages_num, None, h, w, precision=self.plan_precision)
 
     @torch.no_grad()
     def forward(self, x1: torch.Tensor, x2: torch.Tensor):
@@ -175,7 +176,7 @@ class BASE_Transformer(ResNet):
     def lower(self, h: int, w: int) -> L.Program:
         cfg = dict(token_len=self.token_len, heads=8, inner_enc=8 * self.dim_head, inner_dec=8 * self.decoder_dim_head, mlp=64,
                    n_enc=self.enc_depth, n_dec=self.dec_depth, softmax=self.decoder_softmax)
-        return lower_bit(self.state_dict(), self.input_nc, self.output_nc, self.resnet_stages_num, cfg, h, w)
+        return lower_bit(self.state_dict(), self.input_nc, self.output_nc, self.resnet_stages_num, cfg, h, w, precision=self.plan_precision)
 
     @torch.no_grad()
     def forward(self, x1: torch.Tensor, x2: torch.Tensor):
@@ -186,12 +187,14 @@ class BASE_Transformer(ResNet):
 
 
 # ------------------------------------------------------------------------------------------
-def lower_bit(sd: Dict[str, torch.Tensor], in_channels: int, n_class: int, stages: int, cfg: Optional[dict], h: int, w: int) -> L.Program:
-    """state_dict of the reference ResNet / BASE_Transformer -> fused-op Program (eval mode)."""
+def lower_bit(sd: Dict[str, torch.Tensor], in_channels: int, n_class: int, stages: int, cfg: Optional[dict], h: int, w: int,
+              precision: str = "bf16") -> L.Program:
+    """state_dict of the reference ResNet / BASE_Transformer -> fused-op Program (eval mode).  precision "split": every op carries
+    (hi, lo) bf16 planes (lowering.Program.precision)."""
     if h % 16 or w % 16:
         raise ValueError(f"BIT lowering needs H and W divisible by 16 (got {h}x{w})")
     sd = {k: v.detach().to("cpu", torch.float32) for k, v in sd.items()}
-    p = L.Program(model="BIT" if cfg else "BIT-ResNet18", in_channels=in_channels, h=h, w=w)
+    p = L.Program(model="BIT" if cfg else "BIT-ResNet18", in_channels=in_channels, h=h, w=w, precision=precision)
 
     def bn(prefix: str, c: int):
         return L.fold_bn(None, L.bn_params(sd, prefix), c)
@@ -202,14 +205,14 @@ def lower_bit(sd: Dict[str, torch.Tensor], in_channels: int, n_class: int, stage
     # ---------------- stem + max-pool (forward_single, :279-282)
     hh, ww = h // 2, w // 2
     p.tensor("in", 2, hh, ww, 16)
-    p.ops.append(L.InputPackSpec("pack", "in", in_channels, s2d=True))
+    p.ops.append(L.InputPackSpec("pack", "in", in_channels, s2d=True, split=p.split))
     f1s = p.tensor("f1s", 2, hh // 2, ww // 2, 4 * 64)
     sc, sh = bn("resnet.bn1", 64)
     L.add_conv(p, "resnet.conv1", [L.Segment("in", 4 * in_channels)], stem_s2d_taps(sd["resnet.conv1.weight"]), 64, hh, ww, 1, sc, sh,
                pair=True, relu=True, out0=f1s, out0_s2d=True, macs_per_pair=2 * hh * ww * 64 * in_channels * 49)
     hh, ww = hh // 2, ww // 2
     x = p.tensor("p1", 2, hh, ww, 64)
-    p.ops.append(L.MaxPoolS2DSpec("resnet.maxpool", f1s, x, 64))
+    p.ops.append(L.MaxPoolS2DSpec("resnet.maxpool", f1s, x, 64, split=p.split))
     cin, x_s2d = 64, False
 
     # ---------------- layer1 .. layer{stages-1} (:284-294): only layer2 strides
@@ -281,14 +284,15 @@ def lower_bit(sd: Dict[str, torch.Tensor], in_channels: int, n_class: int, stage
         # explicit q / dots / attn.v / to_out is 72 * inner + 4096)
         p.ops.append(L.BitTransformerSpec("bit", f, g, c, cfg["token_len"], cfg["heads"], ie, idd, mlp, f32(sd["conv_a.weight"].reshape(-1, c)),
                                           f32(sd["pos_embedding"].reshape(-1, c)), np.stack(enc_rows), np.stack(dec_rows),
-                                          softmax=cfg["softmax"], macs_per_pair=2 * hh * ww * (cfg["n_dec"] * 6144 + cfg["token_len"] * 2 * c)))
+                                          softmax=cfg["softmax"], macs_per_pair=2 * hh * ww * (cfg["n_dec"] * 6144 + cfg["token_len"] * 2 * c),
+                                          split=p.split))
         f = g
 
     # ---------------- |x1 - x2|, bilinear x4, classifier (:430-436)
     d = p.tensor("diff", 1, hh, ww, 32)
-    p.ops.append(L.AbsDiffSpec("diff", f, d, 32))
+    p.ops.append(L.AbsDiffSpec("diff", f, d, 32, split=p.split))
     u = p.tensor("diff.up4", 1, 4 * hh, 4 * ww, 32)
-    p.ops.append(L.BilinearUpSpec("upsamplex4", d, u, 32, 4))
+    p.ops.append(L.BilinearUpSpec("upsamplex4", d, u, 32, 4, split=p.split))
     hh, ww = 4 * hh, 4 * ww
     c1 = p.tensor("classifier.t", 1, hh, ww, 32)
     sc, sh = bn("classifier.1", 32)

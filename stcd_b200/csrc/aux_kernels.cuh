@@ -430,7 +430,9 @@ __device__ __forceinline__ void unpack8_bf16_f(uint4 q, float* v) {
 // -> dst bf16 [2*chunk][2][h][w][8], channel (py*2 + px)*cin + c = x[c][2y + py][2x + px] (4*cin <= 16).
 // One thread per half-resolution pixel: each (c, py) row is read as one float2, so a warp reads 256
 // contiguous bytes per row and writes 2 x 512 contiguous bytes.  HBM-bound: 16*cin B read + 32 B written.
-template <int CIN>
+// SPLIT: dst is [2*chunk][4][h][w][8], the hi plane bf16(x) in channels [0, 16) (same order) and the lo plane bf16(x - hi) in
+// [16, 32).
+template <int CIN, bool SPLIT>
 __global__ void __launch_bounds__(256) input_pack_s2d_kernel(const float* __restrict__ x1, const float* __restrict__ x2,
                                                              __nv_bfloat16* __restrict__ dst, int chunk, int n_valid,
                                                              int h, int w) {
@@ -467,9 +469,19 @@ __global__ void __launch_bounds__(256) input_pack_s2d_kernel(const float* __rest
       __nv_bfloat162 hv = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
       wd[j] = *reinterpret_cast<uint32_t*>(&hv);
     }
-    __nv_bfloat16* o = dst + (static_cast<size_t>(n) * 2 * hw + pix) * 8;
+    __nv_bfloat16* o = dst + (static_cast<size_t>(n) * (SPLIT ? 4 : 2) * hw + pix) * 8;
     *reinterpret_cast<uint4*>(o) = make_uint4(wd[0], wd[1], wd[2], wd[3]);
     *reinterpret_cast<uint4*>(o + static_cast<size_t>(hw) * 8) = make_uint4(wd[4], wd[5], wd[6], wd[7]);
+    if constexpr (SPLIT) {
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const __nv_bfloat162 hv = *reinterpret_cast<const __nv_bfloat162*>(&wd[j]);
+        const __nv_bfloat162 lv = __floats2bfloat162_rn(v[2 * j] - __low2float(hv), v[2 * j + 1] - __high2float(hv));
+        wd[j] = *reinterpret_cast<const uint32_t*>(&lv);
+      }
+      *reinterpret_cast<uint4*>(o + static_cast<size_t>(2) * hw * 8) = make_uint4(wd[0], wd[1], wd[2], wd[3]);
+      *reinterpret_cast<uint4*>(o + static_cast<size_t>(3) * hw * 8) = make_uint4(wd[4], wd[5], wd[6], wd[7]);
+    }
   }
 }
 
@@ -492,6 +504,10 @@ __device__ __forceinline__ uint4 max8_bf16(uint4 a, uint4 b) {
   return r;
 }
 
+// SPLIT: src stores 8c channels (hi of class k at k*c, lo at 4c + k*c), dst 2c (hi, then lo at dst_c8/2 groups).  The max runs
+// over the fp32 values hi + lo (first maximum wins, in the order below) and the winner's (hi, lo) pair is copied: a selection,
+// so nothing is rounded.
+template <bool SPLIT>
 __global__ void __launch_bounds__(256) maxpool3x3s2_s2d_kernel(const __nv_bfloat16* __restrict__ src,
                                                                __nv_bfloat16* __restrict__ dst, int n_img, int c8, int dst_c8,
                                                                int h, int w) {
@@ -504,9 +520,49 @@ __global__ void __launch_bounds__(256) maxpool3x3s2_s2d_kernel(const __nv_bfloat
     const int g = static_cast<int>(r % c8);
     const int n = static_cast<int>(r / c8);
     const int y = pix / w, x = pix - y * w;
-    const __nv_bfloat16* base = src + (static_cast<size_t>(n) * 4 * c8 + g) * hw * 8;
+    const __nv_bfloat16* base = src + (static_cast<size_t>(n) * (SPLIT ? 8 : 4) * c8 + g) * hw * 8;
     const size_t cls = static_cast<size_t>(c8) * hw * 8;     // stride between parity classes
     auto ld = [&](int k, int yy, int xx) { return __ldg(reinterpret_cast<const uint4*>(base + k * cls + (static_cast<size_t>(yy) * w + xx) * 8)); };
+    if constexpr (SPLIT) {
+      float bh[8], bl[8], bv[8];
+      auto take = [&](int k, int yy, int xx, bool first) {
+        float hv[8], lv[8];
+        unpack8_bf16_f(ld(k, yy, xx), hv);
+        unpack8_bf16_f(ld(4 + k, yy, xx), lv);          // lo plane of class k
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const float v = hv[j] + lv[j];
+          if (first || v > bv[j]) {
+            bv[j] = v;
+            bh[j] = hv[j];
+            bl[j] = lv[j];
+          }
+        }
+      };
+      take(0, y, x, true);
+      take(1, y, x, false);
+      take(2, y, x, false);
+      take(3, y, x, false);
+      if (x > 0) {
+        take(1, y, x - 1, false);
+        take(3, y, x - 1, false);
+      }
+      if (y > 0) {
+        take(2, y - 1, x, false);
+        take(3, y - 1, x, false);
+        if (x > 0) take(3, y - 1, x - 1, false);
+      }
+      uint32_t wh[4], wl[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        wh[j] = pack_bf16x2(bh[2 * j], bh[2 * j + 1]);       // exact: bf16 values
+        wl[j] = pack_bf16x2(bl[2 * j], bl[2 * j + 1]);
+      }
+      __nv_bfloat16* o = dst + ((static_cast<size_t>(n) * dst_c8 + g) * hw + pix) * 8;
+      *reinterpret_cast<uint4*>(o) = make_uint4(wh[0], wh[1], wh[2], wh[3]);
+      *reinterpret_cast<uint4*>(o + static_cast<size_t>(dst_c8 >> 1) * hw * 8) = make_uint4(wl[0], wl[1], wl[2], wl[3]);
+      continue;
+    }
     uint4 m = ld(0, y, x);                       // (2y, 2x)
     m = max8_bf16(m, ld(1, y, x));               // (2y, 2x+1)
     m = max8_bf16(m, ld(2, y, x));               // (2y+1, 2x)
@@ -535,10 +591,51 @@ constexpr int kHeadTW = 32, kHeadTH = 16;
 // dst[b] = |src[b] - src[chunk + b]| on packed bf16 (fp32 subtract, one rounding): torch.abs(f1 - f2) of FFCTLCD
 // (decoders/unet/model.py:412).  Elementwise over 16-byte vectors: layout-agnostic.  HBM-bound: 4 B read + 2 B written.
 // signed_diff: dst = (add ? add : 0) + src[T1] - src[T2]  (DTCDSCN's skip terms "decoder(...) + e_x - e_y", models/DTCDSCN.py:296-300)
+// SPLIT: every tensor holds hi + lo planes; vec_per_stream counts the hi vectors of a stream and plane_vecs the vectors of one
+// plane of one image (hi vector i of image b sits at b * 2 * plane_vecs + i % plane_vecs, its lo vector plane_vecs further).
+// The operands are read as hi + lo and the fp32 result is written as hi = bf16(v), lo = bf16(v - hi).
+template <bool SPLIT>
 __global__ void __launch_bounds__(256) absdiff_kernel(const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ dst,
-                                                      size_t vec_per_stream, int signed_diff, const __nv_bfloat16* __restrict__ add) {
+                                                      size_t vec_per_stream, int signed_diff, const __nv_bfloat16* __restrict__ add,
+                                                      int plane_vecs) {
   for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < vec_per_stream;
        i += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    if constexpr (SPLIT) {
+      const size_t b = i / plane_vecs, hv = i + b * plane_vecs;        // hi vector of image b; the lo vector is plane_vecs further
+      const size_t sv = 2 * vec_per_stream;                            // vectors per stream, both planes
+      const uint4* s4 = reinterpret_cast<const uint4*>(src);
+      float a[8], b_[8], al[8], bl[8];
+      unpack8_bf16_f(__ldg(s4 + hv), a);
+      unpack8_bf16_f(__ldg(s4 + hv + plane_vecs), al);
+      unpack8_bf16_f(__ldg(s4 + sv + hv), b_);
+      unpack8_bf16_f(__ldg(s4 + sv + hv + plane_vecs), bl);
+      float d[8];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        a[j] += al[j];
+        b_[j] += bl[j];
+      }
+      if (add != nullptr) {
+        float c[8], cl[8];
+        unpack8_bf16_f(__ldg(reinterpret_cast<const uint4*>(add) + hv), c);
+        unpack8_bf16_f(__ldg(reinterpret_cast<const uint4*>(add) + hv + plane_vecs), cl);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) a[j] = (c[j] + cl[j]) + a[j];      // reference order: (d + e_x) - e_y
+      }
+#pragma unroll
+      for (int j = 0; j < 8; ++j) d[j] = signed_diff ? a[j] - b_[j] : fabsf(a[j] - b_[j]);
+      uint32_t wh[4], wl[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const __nv_bfloat162 h2 = __floats2bfloat162_rn(d[2 * j], d[2 * j + 1]);
+        const __nv_bfloat162 l2 = __floats2bfloat162_rn(d[2 * j] - __low2float(h2), d[2 * j + 1] - __high2float(h2));
+        wh[j] = *reinterpret_cast<const uint32_t*>(&h2);
+        wl[j] = *reinterpret_cast<const uint32_t*>(&l2);
+      }
+      reinterpret_cast<uint4*>(dst)[hv] = make_uint4(wh[0], wh[1], wh[2], wh[3]);
+      reinterpret_cast<uint4*>(dst)[hv + plane_vecs] = make_uint4(wl[0], wl[1], wl[2], wl[3]);
+      continue;
+    }
     float a[8], b[8];
     unpack8_bf16_f(__ldg(reinterpret_cast<const uint4*>(src) + i), a);
     unpack8_bf16_f(__ldg(reinterpret_cast<const uint4*>(src) + vec_per_stream + i), b);

@@ -38,6 +38,8 @@ __device__ __forceinline__ float bit_gelu(float x) { return gelu_fast(x); }
 
 // ------------------------------------------------------------------------------------------ tokenizer
 // grid = images, 256 threads.  State per thread and token: running max m, sum s, weighted channel sums acc[32].
+// SPLIT: src holds hi + lo planes (lo at src_c8/2 groups), read as hi + lo; the token path is fp32 either way.
+template <bool SPLIT>
 __global__ void __launch_bounds__(256) bit_tokenizer_kernel(const __nv_bfloat16* __restrict__ src, const float* __restrict__ conv_a,
                                                             float* __restrict__ tokens, int src_c8, int hw) {
   __shared__ float s_wa[kBitL * kBitC];
@@ -57,7 +59,10 @@ __global__ void __launch_bounds__(256) bit_tokenizer_kernel(const __nv_bfloat16*
   for (int n = threadIdx.x; n < hw; n += blockDim.x) {
     float x[kBitC];
 #pragma unroll
-    for (int g = 0; g < 4; ++g) unpack8(__ldg(reinterpret_cast<const uint4*>(base + (static_cast<size_t>(g) * hw + n) * 8)), x + 8 * g);
+    for (int g = 0; g < 4; ++g) {
+      if constexpr (SPLIT) load8_split(base + (static_cast<size_t>(g) * hw + n) * 8, static_cast<size_t>(src_c8 >> 1) * hw * 8, x + 8 * g);
+      else unpack8(__ldg(reinterpret_cast<const uint4*>(base + (static_cast<size_t>(g) * hw + n) * 8)), x + 8 * g);
+    }
 #pragma unroll
     for (int l = 0; l < kBitL; ++l) {
       float a = 0.f;
@@ -347,6 +352,9 @@ __device__ __forceinline__ void bit_softmax_groups(BitPx& d) {       // 8 heads 
 constexpr int kBitDecThreads = 128;
 
 // grid (pixel blocks of 2 * kBitDecThreads, images)
+// SPLIT: src and dst hold hi + lo planes (lo at half the stored channel groups): the map is read as hi + lo and written as
+// hi = bf16(x), lo = bf16(x - hi).
+template <bool SPLIT>
 __global__ void __launch_bounds__(kBitDecThreads) bit_decoder_kernel(const __nv_bfloat16* __restrict__ src, __nv_bfloat16* __restrict__ dst,
                                                                      const float* __restrict__ dec, const float* __restrict__ coef,
                                                                      int src_c8, int dst_c8, int hw, int n_dec, int inner_d, int softmax) {
@@ -361,15 +369,19 @@ __global__ void __launch_bounds__(kBitDecThreads) bit_decoder_kernel(const __nv_
 #pragma unroll
     for (int g = 0; g < 4; ++g) {
       float t[8];
-      if (pix0 < hw) unpack8(__ldg(reinterpret_cast<const uint4*>(b + (static_cast<size_t>(g) * hw + pix0) * 8)), t);
-      else {
+      if (pix0 < hw) {
+        if constexpr (SPLIT) load8_split(b + (static_cast<size_t>(g) * hw + pix0) * 8, static_cast<size_t>(src_c8 >> 1) * hw * 8, t);
+        else unpack8(__ldg(reinterpret_cast<const uint4*>(b + (static_cast<size_t>(g) * hw + pix0) * 8)), t);
+      } else {
 #pragma unroll
         for (int j = 0; j < 8; ++j) t[j] = 0.f;
       }
 #pragma unroll
       for (int j = 0; j < 4; ++j) x0.v[4 * g + j] = make_float2(t[2 * j], t[2 * j + 1]);
-      if (pix1 < hw) unpack8(__ldg(reinterpret_cast<const uint4*>(b + (static_cast<size_t>(g) * hw + pix1) * 8)), t);
-      else {
+      if (pix1 < hw) {
+        if constexpr (SPLIT) load8_split(b + (static_cast<size_t>(g) * hw + pix1) * 8, static_cast<size_t>(src_c8 >> 1) * hw * 8, t);
+        else unpack8(__ldg(reinterpret_cast<const uint4*>(b + (static_cast<size_t>(g) * hw + pix1) * 8)), t);
+      } else {
 #pragma unroll
         for (int j = 0; j < 8; ++j) t[j] = 0.f;
       }
@@ -435,6 +447,24 @@ __global__ void __launch_bounds__(kBitDecThreads) bit_decoder_kernel(const __nv_
     }
   }
   __nv_bfloat16* o = dst + static_cast<size_t>(img) * dst_c8 * hw * 8;
+  if constexpr (SPLIT) {
+    const size_t lo_off = static_cast<size_t>(dst_c8 >> 1) * hw * 8;
+#pragma unroll
+    for (int g = 0; g < 4; ++g) {
+      uint4 qh, ql;
+      if (pix0 < hw) {
+        split8(reinterpret_cast<const float*>(x0.v + 4 * g), qh, ql);
+        *reinterpret_cast<uint4*>(o + (static_cast<size_t>(g) * hw + pix0) * 8) = qh;
+        *reinterpret_cast<uint4*>(o + (static_cast<size_t>(g) * hw + pix0) * 8 + lo_off) = ql;
+      }
+      if (pix1 < hw) {
+        split8(reinterpret_cast<const float*>(x1.v + 4 * g), qh, ql);
+        *reinterpret_cast<uint4*>(o + (static_cast<size_t>(g) * hw + pix1) * 8) = qh;
+        *reinterpret_cast<uint4*>(o + (static_cast<size_t>(g) * hw + pix1) * 8 + lo_off) = ql;
+      }
+    }
+    return;
+  }
 #pragma unroll
   for (int g = 0; g < 4; ++g) {
     if (pix0 < hw) *reinterpret_cast<uint4*>(o + (static_cast<size_t>(g) * hw + pix0) * 8) = pack8(reinterpret_cast<const float*>(x0.v + 4 * g));

@@ -99,6 +99,7 @@ struct PackOp {
 
 struct PoolOp {
   int src, dst, c;
+  int split = 0;              // split precision (lowering.Program.precision): src, dst hold hi and lo planes
 };
 
 struct GraphOp {
@@ -148,6 +149,7 @@ struct AbsDiffOp {
   int src, dst, c;
   int signed_diff = 0;
   int add = -1;
+  int split = 0;
 };
 
 struct GateOp {
@@ -155,6 +157,7 @@ struct GateOp {
   std::vector<float> w;      // w1 [hid][c] | w2 [c][hid] | ws [c] (mode 1)
   float* w_dev = nullptr;
   float* partial = nullptr;  // [imgs][ranges][c]
+  int split = 0;
 };
 
 struct BitOp {
@@ -167,6 +170,7 @@ struct BitOp {
   size_t coef_smem = 0;
   float* coef = nullptr;       // [2*chunk][n_dec][A | Bm]
   size_t mixer_smem = 0;
+  int split = 0;               // the feature map holds hi and lo planes (the token path is fp32 either way)
 };
 
 struct ChanAttnOp {
@@ -205,6 +209,7 @@ struct VffmOp {
 
 struct SumOp {
   int src[5], n, dst;
+  int split = 0;
 };
 
 struct SegHeadOp {
@@ -436,8 +441,9 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const Tensor& td = plan->tensors[k.dst];
       const size_t total = (size_t)td.mult * plan->chunk * (k.c / 8) * td.h * td.w;
       const int blocks = (int)std::min<size_t>((total + 255) / 256, 148 * 16);
-      stcd::maxpool3x3s2_s2d_kernel<<<blocks, 256, 0, st>>>((const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr,
-                                                            td.mult * plan->chunk, k.c / 8, td.c / 8, td.h, td.w);
+      auto kern = k.split ? stcd::maxpool3x3s2_s2d_kernel<true> : stcd::maxpool3x3s2_s2d_kernel<false>;
+      kern<<<blocks, 256, 0, st>>>((const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, td.mult * plan->chunk, k.c / 8, td.c / 8, td.h,
+                                   td.w);
       CUDA_TRY(cudaGetLastError());
     } else if (o.kind == 5) {
       const GraphOp& k = plan->graphs[o.idx];
@@ -467,10 +473,12 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
     } else if (o.kind == 10) {
       const AbsDiffOp& k = plan->absdiffs[o.idx];
       const Tensor& td = plan->tensors[k.dst];
-      const size_t vecs = td.bytes / 16;           // 16-byte vectors per stream (dst holds one stream)
-      stcd::absdiff_kernel<<<(unsigned)std::max<size_t>(1, std::min<size_t>((vecs + 255) / 256, 148 * 16)), 256, 0, st>>>(
+      const size_t vecs = td.bytes / 16 / (k.split ? 2 : 1);     // 16-byte (hi) vectors per stream (dst holds one stream)
+      const int plane_vecs = (td.c / 16) * td.h * td.w;            // split: vectors of one plane of one image
+      auto kern = k.split ? stcd::absdiff_kernel<true> : stcd::absdiff_kernel<false>;
+      kern<<<(unsigned)std::max<size_t>(1, std::min<size_t>((vecs + 255) / 256, 148 * 16)), 256, 0, st>>>(
           (const __nv_bfloat16*)plan->tensors[k.src].ptr, (__nv_bfloat16*)td.ptr, vecs, k.signed_diff,
-          k.add >= 0 ? (const __nv_bfloat16*)plan->tensors[k.add].ptr : nullptr);
+          k.add >= 0 ? (const __nv_bfloat16*)plan->tensors[k.add].ptr : nullptr, plane_vecs);
       CUDA_TRY(cudaGetLastError());
     } else if (o.kind == 11) {
       const GateOp& k = plan->gates[o.idx];
@@ -478,13 +486,14 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const Tensor& td = plan->tensors[k.dst];
       const int B = ts.mult * plan->chunk, hw = ts.h * ts.w;
       const int n_items = B * (k.c / 8) * k.ranges;   // one warp each
-      stcd::chan_sum_kernel<<<(n_items + 7) / 8, 256, 0, st>>>((const __nv_bfloat16*)ts.ptr, k.partial, k.c, ts.c / 8, hw, k.ranges, n_items);
+      (k.split ? stcd::chan_sum_kernel<true> : stcd::chan_sum_kernel<false>)<<<(n_items + 7) / 8, 256, 0, st>>>(
+          (const __nv_bfloat16*)ts.ptr, k.partial, k.c, ts.c / 8, hw, k.ranges, n_items);
       // ~2048 (pixel, channel group) items per CTA: enough CTAs to fill the machine on every level of the pyramid
       const int ppb = std::max(32, std::min(stcd::kGateMaxPix, 2048 / (k.c / 8)));
       const float* w1 = k.w_dev;
       const float* w2 = w1 + (size_t)k.hid * k.c;
       const float* ws = k.mode == 1 ? w2 + (size_t)k.c * k.hid : nullptr;
-      stcd::gate_apply_kernel<<<dim3((hw + ppb - 1) / ppb, B), 256, 0, st>>>(
+      (k.split ? stcd::gate_apply_kernel<true> : stcd::gate_apply_kernel<false>)<<<dim3((hw + ppb - 1) / ppb, B), 256, 0, st>>>(
           (const __nv_bfloat16*)ts.ptr, k.res >= 0 ? (const __nv_bfloat16*)plan->tensors[k.res].ptr : nullptr, (__nv_bfloat16*)td.ptr,
           k.dst2 >= 0 ? (__nv_bfloat16*)plan->tensors[k.dst2].ptr : nullptr, k.partial, w1, w2, ws, k.c, k.hid, ts.c / 8,
           k.res >= 0 ? plan->tensors[k.res].c / 8 : 0, td.c / 8, k.dst2 >= 0 ? plan->tensors[k.dst2].c / 8 : 0, ts.h, ts.w, k.ranges, k.mode,
@@ -562,14 +571,16 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const float* pos = conv_a + stcd::kBitL * stcd::kBitC;
       const float* enc = pos + 2 * stcd::kBitL * stcd::kBitC;
       const float* dec = enc + (size_t)k.d.n_enc * stcd::bit_enc_size(k.d.inner_enc);
-      stcd::bit_tokenizer_kernel<<<imgs, 256, 0, st>>>((const __nv_bfloat16*)ts.ptr, conv_a, k.tokens, ts.c / 8, hw);
+      (k.split ? stcd::bit_tokenizer_kernel<true> : stcd::bit_tokenizer_kernel<false>)<<<imgs, 256, 0, st>>>(
+          (const __nv_bfloat16*)ts.ptr, conv_a, k.tokens, ts.c / 8, hw);
       const float scale = 1.f / sqrtf((float)stcd::kBitC);     // dim ** -0.5 with dim = 32 (help_funcs.py:74,118), not dim_head
       stcd::bit_token_mixer_kernel<<<plan->chunk, 256, k.mixer_smem, st>>>(k.tokens, pos, enc, k.tok_mixed, plan->chunk, k.d.n_enc,
                                                                           k.d.inner_enc, scale);
       stcd::bit_coef_kernel<<<dim3(plan->chunk, k.d.n_dec), 256, k.coef_smem, st>>>(k.tok_mixed, dec, k.coef, plan->chunk, k.d.n_dec,
                                                                                    k.d.inner_dec, scale);
-      stcd::bit_decoder_kernel<<<dim3((hw + 2 * stcd::kBitDecThreads - 1) / (2 * stcd::kBitDecThreads), imgs), stcd::kBitDecThreads, 0, st>>>((const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, dec, k.coef,
-                                                                            ts.c / 8, td.c / 8, hw, k.d.n_dec, k.d.inner_dec, k.d.softmax);
+      (k.split ? stcd::bit_decoder_kernel<true> : stcd::bit_decoder_kernel<false>)<<<
+          dim3((hw + 2 * stcd::kBitDecThreads - 1) / (2 * stcd::kBitDecThreads), imgs), stcd::kBitDecThreads, 0, st>>>(
+          (const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, dec, k.coef, ts.c / 8, td.c / 8, hw, k.d.n_dec, k.d.inner_dec, k.d.softmax);
       CUDA_TRY(cudaGetLastError());
     } else if (o.kind == 12) {
       const SumOp& k = plan->sums[o.idx];
@@ -577,8 +588,10 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       stcd::AddNParams ap;
       ap.n = k.n;
       for (int i = 0; i < 5; ++i) ap.src[i] = i < k.n ? (const __nv_bfloat16*)plan->tensors[k.src[i]].ptr : nullptr;
-      const size_t vecs = td.bytes / 16;
-      stcd::add_n_kernel<<<(unsigned)std::max<size_t>(1, std::min<size_t>((vecs + 255) / 256, 148 * 16)), 256, 0, st>>>(ap, (__nv_bfloat16*)td.ptr, vecs);
+      const size_t vecs = td.bytes / 16 / (k.split ? 2 : 1);     // (hi) vectors
+      auto kern = k.split ? stcd::add_n_kernel<true> : stcd::add_n_kernel<false>;
+      kern<<<(unsigned)std::max<size_t>(1, std::min<size_t>((vecs + 255) / 256, 148 * 16)), 256, 0, st>>>(ap, (__nv_bfloat16*)td.ptr, vecs,
+                                                                                                        (td.c / 16) * td.h * td.w);
       CUDA_TRY(cudaGetLastError());
     } else if (o.kind == 7) {
       const LayerNormOp& k = plan->lns[o.idx];
@@ -691,12 +704,16 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
 #undef STCD_PACK_U8
       } else if (k.s2d) {
         __nv_bfloat16* dp = (__nv_bfloat16*)t.ptr;
+#define STCD_PACK_S2D(CIN)                                                                                                   \
+  (k.split ? stcd::input_pack_s2d_kernel<CIN, true> : stcd::input_pack_s2d_kernel<CIN, false>)<<<blocks, 256, 0, st>>>( \
+      x1, x2, dp, plan->chunk, n_valid, t.h, t.w)
         switch (k.cin) {
-          case 1: stcd::input_pack_s2d_kernel<1><<<blocks, 256, 0, st>>>(x1, x2, dp, plan->chunk, n_valid, t.h, t.w); break;
-          case 2: stcd::input_pack_s2d_kernel<2><<<blocks, 256, 0, st>>>(x1, x2, dp, plan->chunk, n_valid, t.h, t.w); break;
-          case 3: stcd::input_pack_s2d_kernel<3><<<blocks, 256, 0, st>>>(x1, x2, dp, plan->chunk, n_valid, t.h, t.w); break;
-          default: stcd::input_pack_s2d_kernel<4><<<blocks, 256, 0, st>>>(x1, x2, dp, plan->chunk, n_valid, t.h, t.w); break;
+          case 1: STCD_PACK_S2D(1); break;
+          case 2: STCD_PACK_S2D(2); break;
+          case 3: STCD_PACK_S2D(3); break;
+          default: STCD_PACK_S2D(4); break;
         }
+#undef STCD_PACK_S2D
       } else if (!k.split && k.cin <= 4 && hw % 4 == 0 && (reinterpret_cast<uintptr_t>(x1) | reinterpret_cast<uintptr_t>(x2)) % 16 == 0) {
         __nv_bfloat16* dp = (__nv_bfloat16*)t.ptr;
         const int blocks4 = (int)std::min<size_t>((total / 4 + 255) / 256, 148 * 8);
@@ -905,18 +922,19 @@ int stcd_plan_add_input_pack_split(stcd_plan* plan, int dst_tensor, int cin) {
   return (int)plan->ops.size() - 1;
 }
 
-int stcd_plan_add_input_pack_s2d(stcd_plan* plan, int dst_tensor, int cin) {
+static int add_input_pack_s2d(stcd_plan* plan, int dst_tensor, int cin, int split) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad dst tensor %d", dst_tensor);
   const Tensor& t = plan->tensors[dst_tensor];
-  if (t.mult != 2 || t.c != 16 || cin < 1 || cin > 4)
-    return -fail(STCD_ERR_INVALID, "space-to-depth input pack needs a [2*chunk][2][h][w][8] tensor and cin <= 4 (got mult=%d c=%d cin=%d)",
-                 t.mult, t.c, cin);
+  if (t.mult != 2 || t.c != (split ? 32 : 16) || cin < 1 || cin > 4)
+    return -fail(STCD_ERR_INVALID, "space-to-depth input pack needs a [2*chunk][%d][h][w][8] tensor and cin <= 4 (got mult=%d c=%d cin=%d)",
+                 split ? 4 : 2, t.mult, t.c, cin);
   PackOp k;
   k.dst = dst_tensor;
   k.cin = cin;
   k.s2d = 1;
+  k.split = split;
   plan->packs.push_back(k);
   plan->ops.push_back({1, (int)plan->packs.size() - 1});
   plan->in_c = cin;
@@ -924,6 +942,8 @@ int stcd_plan_add_input_pack_s2d(stcd_plan* plan, int dst_tensor, int cin) {
   plan->in_w = 2 * t.w;
   return (int)plan->ops.size() - 1;
 }
+
+int stcd_plan_add_input_pack_s2d(stcd_plan* plan, int dst_tensor, int cin) { return add_input_pack_s2d(plan, dst_tensor, cin, 0); }
 
 int stcd_plan_add_input_pack_u8(stcd_plan* plan, int dst_tensor, int cin, int s2d, const float* mean, const float* std_) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
@@ -943,18 +963,24 @@ int stcd_plan_add_input_pack_u8(stcd_plan* plan, int dst_tensor, int cin, int s2
   return r;
 }
 
-int stcd_plan_add_maxpool_s2d(stcd_plan* plan, int src_tensor, int dst_tensor, int c) {
+static int add_maxpool_s2d(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int split) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad tensor id");
   const Tensor& ts = plan->tensors[src_tensor];
   const Tensor& td = plan->tensors[dst_tensor];
-  if (c < 8 || (c % 8) || ts.c != 4 * c || td.c < c || ts.h != td.h || ts.w != td.w || ts.mult != td.mult)
+  if (c < 8 || (c % 8) || ts.c != (split ? 8 : 4) * c || td.c < (split ? 2 : 1) * c || ts.h != td.h || ts.w != td.w || ts.mult != td.mult)
     return -fail(STCD_ERR_INVALID, "max-pool: src [%d*chunk,%d,%d,%d] must be the space-to-depth form of dst [%d*chunk,%d,%d,%d] (c=%d)",
                  ts.mult, ts.h, ts.w, ts.c, td.mult, td.h, td.w, td.c, c);
-  plan->pools.push_back({src_tensor, dst_tensor, c});
+  PoolOp k{src_tensor, dst_tensor, c};
+  k.split = split;
+  plan->pools.push_back(k);
   plan->ops.push_back({3, (int)plan->pools.size() - 1});
   return (int)plan->ops.size() - 1;
+}
+
+int stcd_plan_add_maxpool_s2d(stcd_plan* plan, int src_tensor, int dst_tensor, int c) {
+  return add_maxpool_s2d(plan, src_tensor, dst_tensor, c, 0);
 }
 
 int stcd_plan_add_graph_conv(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int k, int dilation, int r, const float* relpos) {
@@ -1153,8 +1179,8 @@ int stcd_plan_add_subdiff(stcd_plan* plan, int src_tensor, int add, int dst_tens
   return r;
 }
 
-int stcd_plan_add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst_tensor, int dst_s2d, int c, int hid, const float* w1,
-                               const float* w2, const float* ws, int mode) {
+static int add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst_tensor, int dst_s2d, int c, int hid, const float* w1,
+                            const float* w2, const float* ws, int mode, int split) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor) || (res >= 0 && !valid_tensor(plan, res)) ||
@@ -1171,8 +1197,9 @@ int stcd_plan_add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst
   }
   if (dst_s2d >= 0) {
     const Tensor& t2 = plan->tensors[dst_s2d];
-    if ((ts.h % 2) || (ts.w % 2) || t2.h != ts.h / 2 || t2.w != ts.w / 2 || t2.c != 4 * c || t2.mult != ts.mult)
-      return -fail(STCD_ERR_INVALID, "channel gate: space-to-depth copy must be [%d*chunk,%d,%d,%d]", ts.mult, ts.h / 2, ts.w / 2, 4 * c);
+    if ((ts.h % 2) || (ts.w % 2) || t2.h != ts.h / 2 || t2.w != ts.w / 2 || t2.c != (split ? 8 : 4) * c || t2.mult != ts.mult)
+      return -fail(STCD_ERR_INVALID, "channel gate: space-to-depth copy must be [%d*chunk,%d,%d,%d]", ts.mult, ts.h / 2, ts.w / 2,
+                   (split ? 8 : 4) * c);
   }
   GateOp k;
   k.src = src_tensor;
@@ -1186,12 +1213,18 @@ int stcd_plan_add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst
   k.w.assign(w1, w1 + (size_t)hid * c);
   k.w.insert(k.w.end(), w2, w2 + (size_t)c * hid);
   if (mode == 1) k.w.insert(k.w.end(), ws, ws + c);
+  k.split = split;
   plan->gates.push_back(std::move(k));
   plan->ops.push_back({11, (int)plan->gates.size() - 1});
   return (int)plan->ops.size() - 1;
 }
 
-int stcd_plan_add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* d) {
+int stcd_plan_add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst_tensor, int dst_s2d, int c, int hid, const float* w1,
+                               const float* w2, const float* ws, int mode) {
+  return add_channel_gate(plan, src_tensor, res, dst_tensor, dst_s2d, c, hid, w1, w2, ws, mode, 0);
+}
+
+static int add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* d, int split) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!d || !valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor) || !d->conv_a || !d->pos || !d->enc || !d->dec)
@@ -1204,8 +1237,9 @@ int stcd_plan_add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tenso
     return -fail(STCD_ERR_INVALID, "BIT transformer: depths %d/%d, inner dims %d/%d out of range", d->n_enc, d->n_dec, d->inner_enc, d->inner_dec);
   const Tensor& ts = plan->tensors[src_tensor];
   const Tensor& td = plan->tensors[dst_tensor];
-  if (ts.mult != 2 || td.mult != 2 || ts.c != stcd::kBitC || td.c != stcd::kBitC || ts.h != td.h || ts.w != td.w)
-    return -fail(STCD_ERR_INVALID, "BIT transformer: src and dst must be [2*chunk,h,w,32] (both streams)");
+  const int cs = (split ? 2 : 1) * stcd::kBitC;      // stored channels (split: hi and lo planes)
+  if (ts.mult != 2 || td.mult != 2 || ts.c != cs || td.c != cs || ts.h != td.h || ts.w != td.w)
+    return -fail(STCD_ERR_INVALID, "BIT transformer: src and dst must be [2*chunk,h,w,%d] (both streams)", cs);
   BitOp k;
   k.src = src_tensor;
   k.dst = dst_tensor;
@@ -1217,9 +1251,14 @@ int stcd_plan_add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tenso
   k.d.conv_a = k.d.pos = k.d.enc = k.d.dec = nullptr;
   k.mixer_smem = sizeof(float) * (size_t)(8 * 3 * d->inner_enc);
   k.coef_smem = sizeof(float) * (size_t)(2 * 8 * d->inner_dec);
+  k.split = split;
   plan->bits.push_back(std::move(k));
   plan->ops.push_back({13, (int)plan->bits.size() - 1});
   return (int)plan->ops.size() - 1;
+}
+
+int stcd_plan_add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* d) {
+  return add_bit_transformer(plan, src_tensor, dst_tensor, d, 0);
 }
 
 int stcd_plan_add_channel_attention(stcd_plan* plan, const int* src_tensors, const int* src_streams, const int* src_c, int n_src,
@@ -1350,6 +1389,60 @@ int stcd_plan_add_sum(stcd_plan* plan, const int* src_tensors, int n, int dst_te
   return (int)plan->ops.size() - 1;
 }
 
+// ---- split precision forms of the ResNet-family ops (stem pack and max-pool, feature differences, sums, SE gates, BIT's token
+// path).  Like the ones above, they reject tensors that do not store twice their logical channels in multiples of 16.
+int stcd_plan_add_input_pack_s2d_split(stcd_plan* plan, int dst_tensor, int cin) { return add_input_pack_s2d(plan, dst_tensor, cin, 1); }
+
+int stcd_plan_add_maxpool_s2d_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c) {
+  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (valid_tensor(plan, dst_tensor) && !split_planes(plan->tensors[dst_tensor], c))
+    return -fail(STCD_ERR_INVALID, "split max-pool: dst must store 2 x %d channels in multiples of 16 (got %d)", c, plan->tensors[dst_tensor].c);
+  return add_maxpool_s2d(plan, src_tensor, dst_tensor, c, 1);      // src: 8c (4 classes x 2 planes)
+}
+
+// elementwise ops without a logical channel count: every tensor must hold two planes of a multiple of 8 channels
+static bool split_even(stcd_plan* plan, int t) { return !valid_tensor(plan, t) || plan->tensors[t].c % 16 == 0; }
+
+int stcd_plan_add_absdiff_split(stcd_plan* plan, int src_tensor, int dst_tensor) {
+  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (!split_even(plan, src_tensor) || !split_even(plan, dst_tensor))
+    return -fail(STCD_ERR_INVALID, "split abs-diff: src / dst must store hi and lo planes (channels a multiple of 16)");
+  const int r = stcd_plan_add_absdiff(plan, src_tensor, dst_tensor);
+  if (r >= 0) plan->absdiffs.back().split = 1;
+  return r;
+}
+
+int stcd_plan_add_subdiff_split(stcd_plan* plan, int src_tensor, int add, int dst_tensor) {
+  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (!split_even(plan, src_tensor) || !split_even(plan, dst_tensor) || (add >= 0 && !split_even(plan, add)))
+    return -fail(STCD_ERR_INVALID, "split signed diff: src / addend / dst must store hi and lo planes (channels a multiple of 16)");
+  const int r = stcd_plan_add_subdiff(plan, src_tensor, add, dst_tensor);
+  if (r >= 0) plan->absdiffs.back().split = 1;
+  return r;
+}
+
+int stcd_plan_add_sum_split(stcd_plan* plan, const int* src_tensors, int n, int dst_tensor) {
+  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (!split_even(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "split sum: dst must store hi and lo planes (channels a multiple of 16)");
+  const int r = stcd_plan_add_sum(plan, src_tensors, n, dst_tensor);     // sources: the destination's shape
+  if (r >= 0) plan->sums.back().split = 1;
+  return r;
+}
+
+int stcd_plan_add_channel_gate_split(stcd_plan* plan, int src_tensor, int res, int dst_tensor, int dst_s2d, int c, int hid, const float* w1,
+                                     const float* w2, const float* ws, int mode) {
+  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  for (int t : {src_tensor, dst_tensor, res})
+    if (valid_tensor(plan, t) && !split_planes(plan->tensors[t], c))
+      return -fail(STCD_ERR_INVALID, "split channel gate: src / res / dst must store 2 x %d channels in multiples of 16 (tensor %d has %d)", c,
+                   t, plan->tensors[t].c);
+  return add_channel_gate(plan, src_tensor, res, dst_tensor, dst_s2d, c, hid, w1, w2, ws, mode, 1);    // space-to-depth copy: 8c
+}
+
+int stcd_plan_add_bit_transformer_split(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* d) {
+  return add_bit_transformer(plan, src_tensor, dst_tensor, d, 1);
+}
+
 int stcd_plan_add_seg_head(stcd_plan* plan, const stcd_seghead_desc* d) {
   if (!plan || !d) return -fail(STCD_ERR_STATE, "plan/desc is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
@@ -1400,8 +1493,8 @@ int stcd_plan_add_conv(stcd_plan* plan, const stcd_conv_desc* d) {
   if (2 * mt * d->n_tile > 512)
     return -fail(STCD_ERR_INVALID, "double-buffered accumulators need %d TMEM columns (> 512)", 2 * mt * d->n_tile);
   if (d->pair && (plan->chunk < 1)) return -fail(STCD_ERR_INVALID, "pair op on an empty chunk");
-  if (d->split && (d->out0_s2d || d->fold_cs || d->xf_cs))
-    return -fail(STCD_ERR_INVALID, "split precision: no space-to-depth, folded or horizontally folded stores");
+  if (d->split && (d->fold_cs || d->xf_cs))
+    return -fail(STCD_ERR_INVALID, "split precision: no folded or horizontally folded stores");
   if (d->xf_cs) {
     bool ok = d->xf_cs >= 16 && d->xf_cs % 16 == 0 && d->n_tile == 3 * d->xf_cs && d->cout_pad == d->n_tile && d->cout <= d->xf_cs &&
               d->n_phase == 1 && d->osy == 1 && d->osx == 1 && !d->out0_s2d && !d->fold_cs;
@@ -1455,9 +1548,10 @@ int stcd_plan_add_conv(stcd_plan* plan, const stcd_conv_desc* d) {
     if (d->out0 < 0 || d->out0_coff || (ho % 2) || (wo % 2) || !valid_tensor(plan, d->out0))
       return -fail(STCD_ERR_INVALID, "space-to-depth out0 needs a tensor, even output dims and no channel offset");
     const Tensor& t = plan->tensors[d->out0];
-    if (t.h != ho / 2 || t.w != wo / 2 || t.c != 4 * d->cout || t.mult != out_imgs)
-      return -fail(STCD_ERR_INVALID, "space-to-depth out0 tensor is [%d*chunk,%d,%d,%d], op writes [%d*chunk,%d,%d,4*%d]", t.mult, t.h, t.w,
-                   t.c, out_imgs, ho / 2, wo / 2, d->cout);
+    // split precision: hi of parity class k at k*cout, lo at 4*cout + k*cout
+    if (t.h != ho / 2 || t.w != wo / 2 || t.c != (d->split ? 8 : 4) * d->cout || t.mult != out_imgs)
+      return -fail(STCD_ERR_INVALID, "space-to-depth out0 tensor is [%d*chunk,%d,%d,%d], op writes [%d*chunk,%d,%d,%d*%d]", t.mult, t.h, t.w,
+                   t.c, out_imgs, ho / 2, wo / 2, d->split ? 8 : 4, d->cout);
   } else if (check_out(d->out0, ho, wo, d->out0_coff, out_imgs, "out0")) return -STCD_ERR_INVALID;
   if (check_out(d->out_raw, ho, wo, 0, out_imgs, "out_raw")) return -STCD_ERR_INVALID;
   if (check_out(d->res, ho, wo, 0, out_imgs, "res")) return -STCD_ERR_INVALID;

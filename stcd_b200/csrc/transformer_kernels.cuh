@@ -496,7 +496,9 @@ constexpr int kGateMaxC = 512;
 constexpr int kGateMaxH = 32;
 
 // one warp per (pixel range, 8-channel group, image): lanes stride over the range's pixels, butterfly reduce (fixed order)
+// SPLIT: src holds hi + lo planes (lo at src_c8/2 groups) and the sums run over hi + lo.
 constexpr int kGateRangePix = 512;
+template <bool SPLIT>
 __global__ void __launch_bounds__(256) chan_sum_kernel(const __nv_bfloat16* __restrict__ src, float* __restrict__ partial, int C,
                                                        int src_c8, int hw, int ranges, int n_items) {
   const int item = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -510,7 +512,8 @@ __global__ void __launch_bounds__(256) chan_sum_kernel(const __nv_bfloat16* __re
 #pragma unroll 4
   for (int px = p0 + lane; px < p1; px += 32) {
     float v[8];
-    unpack8(__ldg(reinterpret_cast<const uint4*>(base + static_cast<size_t>(px) * 8)), v);
+    if constexpr (SPLIT) load8_split(base + static_cast<size_t>(px) * 8, static_cast<size_t>(src_c8 >> 1) * hw * 8, v);
+    else unpack8(__ldg(reinterpret_cast<const uint4*>(base + static_cast<size_t>(px) * 8)), v);
 #pragma unroll
     for (int j = 0; j < 8; ++j) s[j] += v[j];
   }
@@ -529,7 +532,10 @@ __global__ void __launch_bounds__(256) chan_sum_kernel(const __nv_bfloat16* __re
 
 // grid (pixel blocks, B), 256 threads.  Every CTA redoes the two tiny FC layers of its image (C x hid MACs, warp-cooperative),
 // then applies its pixels: work items are (channel group, pixel) so small maps with many channels still fill the CTA.
+// SPLIT: src, res, dst and dst2 hold hi + lo planes (lo at half the stored channel groups; dst2's lo plane of class k, group g at
+// 4*g8 + k*g8 + g).  Reads are hi + lo, the gate and the output are formed in fp32 as above and written as hi and lo.
 constexpr int kGateMaxPix = 1024;
+template <bool SPLIT>
 __global__ void __launch_bounds__(256) gate_apply_kernel(const __nv_bfloat16* __restrict__ src, const __nv_bfloat16* __restrict__ res,
                                                          __nv_bfloat16* __restrict__ dst, __nv_bfloat16* __restrict__ dst2,
                                                          const float* __restrict__ partial, const float* __restrict__ w1,
@@ -561,12 +567,14 @@ __global__ void __launch_bounds__(256) gate_apply_kernel(const __nv_bfloat16* __
   const int p_begin = blockIdx.x * pix_per_block;
   const int n_pix = min(hw, p_begin + pix_per_block) - p_begin;
   const __nv_bfloat16* sb = src + static_cast<size_t>(b) * src_c8 * hw * 8;
+  const size_t s_lo = static_cast<size_t>(src_c8 >> 1) * hw * 8;      // split: offset of the lo plane
   if (mode == 1) {                                       // spatial gate per pixel: sigmoid(ws . x_pixel)
     for (int i = threadIdx.x; i < n_pix; i += blockDim.x) {
       float a = 0.f;
       for (int g = 0; g < g8; ++g) {
         float v[8];
-        unpack8(__ldg(reinterpret_cast<const uint4*>(sb + (static_cast<size_t>(g) * hw + p_begin + i) * 8)), v);
+        if constexpr (SPLIT) load8_split(sb + (static_cast<size_t>(g) * hw + p_begin + i) * 8, s_lo, v);
+        else unpack8(__ldg(reinterpret_cast<const uint4*>(sb + (static_cast<size_t>(g) * hw + p_begin + i) * 8)), v);
 #pragma unroll
         for (int j = 0; j < 8; ++j) a = fmaf(v[j], __ldg(ws + g * 8 + j), a);
       }
@@ -578,16 +586,35 @@ __global__ void __launch_bounds__(256) gate_apply_kernel(const __nv_bfloat16* __
   for (int it = threadIdx.x; it < n_pix * g8; it += blockDim.x) {
     const int g = it / n_pix, i = it - g * n_pix, pix = p_begin + i;
     float v[8];
-    unpack8(__ldg(reinterpret_cast<const uint4*>(sb + (static_cast<size_t>(g) * hw + pix) * 8)), v);
+    if constexpr (SPLIT) load8_split(sb + (static_cast<size_t>(g) * hw + pix) * 8, s_lo, v);
+    else unpack8(__ldg(reinterpret_cast<const uint4*>(sb + (static_cast<size_t>(g) * hw + pix) * 8)), v);
     if (mode == 0) {
       float rv[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-      if (res != nullptr) unpack8(__ldg(reinterpret_cast<const uint4*>(res + ((static_cast<size_t>(b) * res_c8 + g) * hw + pix) * 8)), rv);
+      if constexpr (SPLIT) {
+        if (res != nullptr)
+          load8_split(res + ((static_cast<size_t>(b) * res_c8 + g) * hw + pix) * 8, static_cast<size_t>(res_c8 >> 1) * hw * 8, rv);
+      } else if (res != nullptr) unpack8(__ldg(reinterpret_cast<const uint4*>(res + ((static_cast<size_t>(b) * res_c8 + g) * hw + pix) * 8)), rv);
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = fmaxf(fmaf(v[j], s_gate[g * 8 + j], rv[j]), 0.f);
     } else {
       const float gs = s_gs[i];
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = v[j] * (1.f + s_gate[g * 8 + j] + gs);
+    }
+    if constexpr (SPLIT) {
+      uint4 qh, ql;
+      split8(v, qh, ql);
+      __nv_bfloat16* o = dst + ((static_cast<size_t>(b) * dst_c8 + g) * hw + pix) * 8;
+      *reinterpret_cast<uint4*>(o) = qh;
+      *reinterpret_cast<uint4*>(o + static_cast<size_t>(dst_c8 >> 1) * hw * 8) = ql;
+      if (dst2 != nullptr) {
+        const int y = pix / w, x = pix - y * w;
+        __nv_bfloat16* o2 = dst2 + ((static_cast<size_t>(b) * dst2_c8 + ((y & 1) * 2 + (x & 1)) * g8 + g) * hw2 +
+                                    static_cast<size_t>(y >> 1) * w2h + (x >> 1)) * 8;
+        *reinterpret_cast<uint4*>(o2) = qh;
+        *reinterpret_cast<uint4*>(o2 + static_cast<size_t>(dst2_c8 >> 1) * hw2 * 8) = ql;
+      }
+      continue;
     }
     const uint4 q = pack8(v);
     *reinterpret_cast<uint4*>(dst + ((static_cast<size_t>(b) * dst_c8 + g) * hw + pix) * 8) = q;
@@ -600,12 +627,31 @@ __global__ void __launch_bounds__(256) gate_apply_kernel(const __nv_bfloat16* __
 }
 
 // dst = sum of up to 5 tensors (Dblock: x + d1 + d2 + d3 + d4, models/DTCDSCN.py:65-71), elementwise over 16-byte vectors
+// SPLIT: every tensor holds hi + lo planes; vecs counts the hi vectors and plane_vecs the vectors of one plane of one image (as in
+// absdiff_kernel).  The fp32 sum of the hi + lo values, in source order, is written as hi and lo.
 struct AddNParams {
   const __nv_bfloat16* src[5];
   int n;
 };
-__global__ void __launch_bounds__(256) add_n_kernel(const AddNParams p, __nv_bfloat16* __restrict__ dst, size_t vecs) {
+template <bool SPLIT>
+__global__ void __launch_bounds__(256) add_n_kernel(const AddNParams p, __nv_bfloat16* __restrict__ dst, size_t vecs, int plane_vecs) {
   for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < vecs; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
+    if constexpr (SPLIT) {
+      const size_t hv = i + (i / plane_vecs) * plane_vecs;            // hi vector; its lo vector is plane_vecs further
+      const size_t lo_off = static_cast<size_t>(plane_vecs) * 8;
+      float a[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+      for (int k = 0; k < p.n; ++k) {
+        float v[8];
+        load8_split(p.src[k] + hv * 8, lo_off, v);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) a[j] += v[j];
+      }
+      uint4 qh, ql;
+      split8(a, qh, ql);
+      reinterpret_cast<uint4*>(dst)[hv] = qh;
+      reinterpret_cast<uint4*>(dst)[hv + plane_vecs] = ql;
+      continue;
+    }
     float a[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     for (int k = 0; k < p.n; ++k) {
       float v[8];

@@ -102,6 +102,7 @@ class _Dblock(nn.Module):
 class CDNet_model(PlannedModule):
     """models/DTCDSCN.py:176-313."""
     default_chunk_pairs = 16
+    supports_precision_path = True
 
     def __init__(self, in_channels: int = 3, block=None, layers: Sequence[int] = (3, 4, 6, 3), num_classes: int = 2):
         super().__init__()
@@ -154,7 +155,7 @@ class CDNet_model(PlannedModule):
         return nn.Sequential(*layers)
 
     def lower(self, h: int, w: int) -> L.Program:
-        return lower_dtcdscn(self.state_dict(), self.inchannels, self.layers, self.num_classes, h, w)
+        return lower_dtcdscn(self.state_dict(), self.inchannels, self.layers, self.num_classes, h, w, precision=self.plan_precision)
 
     @torch.no_grad()
     def forward(self, x: torch.Tensor, y: torch.Tensor) -> torch.Tensor:
@@ -175,13 +176,15 @@ def dilated_taps(weight: torch.Tensor, d: int, h: int, w: int) -> List:
     return [(0, 0, taps)]
 
 
-def lower_dtcdscn(sd: Dict[str, torch.Tensor], in_channels: int, layers: Sequence[int], num_classes: int, h: int, w: int) -> L.Program:
-    """state_dict of the reference CDNet_model -> fused-op Program (eval mode)."""
+def lower_dtcdscn(sd: Dict[str, torch.Tensor], in_channels: int, layers: Sequence[int], num_classes: int, h: int, w: int,
+                  precision: str = "bf16") -> L.Program:
+    """state_dict of the reference CDNet_model -> fused-op Program (eval mode).  precision "split": every op carries (hi, lo) bf16
+    planes (lowering.Program.precision)."""
     if h % 32 or w % 32:
         raise ValueError(f"DTCDSCN lowering needs H and W divisible by 32 (got {h}x{w}): the reference's skip additions "
                          "do not line up otherwise")
     sd = {k: v.detach().to("cpu", torch.float32) for k, v in sd.items()}
-    p = L.Program(model="CDNet34", in_channels=in_channels, h=h, w=w)
+    p = L.Program(model="CDNet34", in_channels=in_channels, h=h, w=w, precision=precision)
 
     def bn(prefix: str, c: int, bias=None):
         return L.fold_bn(bias, L.bn_params(sd, prefix), c)
@@ -192,14 +195,14 @@ def lower_dtcdscn(sd: Dict[str, torch.Tensor], in_channels: int, layers: Sequenc
     # ---------------- stem (:246-249): space-to-depth pack, 4x4 conv, BN, ReLU (stored space-to-depth), max-pool
     hh, ww = h // 2, w // 2
     p.tensor("in", 2, hh, ww, 16)
-    p.ops.append(L.InputPackSpec("pack", "in", in_channels, s2d=True))
+    p.ops.append(L.InputPackSpec("pack", "in", in_channels, s2d=True, split=p.split))
     f1s = p.tensor("f1s", 2, hh // 2, ww // 2, 4 * 64)
     sc, sh = bn("firstbn", 64)
     L.add_conv(p, "firstconv", [L.Segment("in", 4 * in_channels)], stem_s2d_taps(sd["firstconv.weight"]), 64, hh, ww, 1, sc, sh,
                pair=True, relu=True, out0=f1s, out0_s2d=True, macs_per_pair=2 * hh * ww * 64 * in_channels * 49)
     hh, ww = hh // 2, ww // 2
     x = p.tensor("p1", 2, hh, ww, 64)
-    p.ops.append(L.MaxPoolS2DSpec("firstmaxpool", f1s, x, 64))
+    p.ops.append(L.MaxPoolS2DSpec("firstmaxpool", f1s, x, 64, split=p.split))
     x_s2d = None                      # space-to-depth copy of x (what a stride-2 conv reads)
     cin = 64
 
@@ -240,14 +243,14 @@ def lower_dtcdscn(sd: Dict[str, torch.Tensor], in_channels: int, layers: Sequenc
             o = p.tensor(f"{pre}.o", 2, hh, ww, cout)
             o_s2d = p.tensor(f"{pre}.o_s2d", 2, hh // 2, ww // 2, 4 * cout) if (last_of_layer and li < 3) else None
             p.ops.append(L.ChannelGateSpec(f"{pre}.se", u, o, cout, f32(sd[f"{pre}.se.fc.0.weight"]), f32(sd[f"{pre}.se.fc.2.weight"]),
-                                           mode=0, res=ident, dst_s2d=o_s2d))
+                                           mode=0, res=ident, dst_s2d=o_s2d, split=p.split))
             x, x_s2d, cin = o, o_s2d, cout
         feats.append((x, cout, hh, ww))
 
     # ---------------- centre: Dblock on e4_x - e4_y (:294; Dblock.forward :65-71)
     e4, c4, hh, ww = feats[3]
     dsum = [p.tensor("e4.diff", 1, hh, ww, c4)]
-    p.ops.append(L.AbsDiffSpec("e4.diff", e4, dsum[0], c4, signed=True))
+    p.ops.append(L.AbsDiffSpec("e4.diff", e4, dsum[0], c4, signed=True, split=p.split))
     cur = dsum[0]
     for i, dil in enumerate((1, 2, 4, 8)):
         nm = f"dblock_master.dilate{i + 1}"
@@ -259,7 +262,7 @@ def lower_dtcdscn(sd: Dict[str, torch.Tensor], in_channels: int, layers: Sequenc
         dsum.append(o)
         cur = o
     x = p.tensor("dblock_master.o", 1, hh, ww, c4)
-    p.ops.append(L.SumSpec("dblock_master.sum", dsum, x))
+    p.ops.append(L.SumSpec("dblock_master.sum", dsum, x, split=p.split))
     cin = c4
 
     # ---------------- decoder on the differences (:296-299)
@@ -278,7 +281,7 @@ def lower_dtcdscn(sd: Dict[str, torch.Tensor], in_channels: int, layers: Sequenc
         w2g[:mid] = f32(sd[f"{nm}.scse.channel_excitation.2.weight"].reshape(mid, hid))
         wsg[:mid] = f32(sd[f"{nm}.scse.spatial_se.0.weight"].reshape(mid))
         t2 = p.tensor(f"{nm}.t2", 1, hh, ww, midp)
-        p.ops.append(L.ChannelGateSpec(f"{nm}.scse", t1, t2, midp, w1g, w2g, mode=1, ws=wsg))
+        p.ops.append(L.ChannelGateSpec(f"{nm}.scse", t1, t2, midp, w1g, w2g, mode=1, ws=wsg, split=p.split))
         t3 = p.tensor(f"{nm}.t3", 1, 2 * hh, 2 * ww, midp)
         sc, sh = bn(f"{nm}.norm2", mid, sd[f"{nm}.deconv2.bias"])
         L.add_conv(p, f"{nm}.deconv2", [L.Segment(t2, mid)], L.convT_phase_taps(sd[f"{nm}.deconv2.weight"], 2, 1), mid, hh, ww, 1, sc, sh,
@@ -291,7 +294,7 @@ def lower_dtcdscn(sd: Dict[str, torch.Tensor], in_channels: int, layers: Sequenc
         if di < 3:
             e, ce, _, _ = feats[2 - di]
             d = p.tensor(f"{nm}.d", 1, hh, ww, cout)
-            p.ops.append(L.AbsDiffSpec(f"{nm}.skip", e, d, ce, signed=True, add=o))
+            p.ops.append(L.AbsDiffSpec(f"{nm}.skip", e, d, ce, signed=True, add=o, split=p.split))
             o = d
         x, cin = o, cout
 

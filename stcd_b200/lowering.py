@@ -132,7 +132,7 @@ class InputPackSpec:
     name: str
     dst: str
     cin: int
-    s2d: bool = False            # space-to-depth: dst is [h/2, w/2] with channel (py*2 + px)*cin + c
+    s2d: bool = False            # space-to-depth: dst is [h/2, w/2] with channel (py*2 + px)*cin + c (split: lo plane at 16 + that)
     # (mean, std) per channel: the plan's inputs are uint8 HWC images and the pack kernel applies the reference
     # loader's ToTensor + Normalize (data/dataset.py:196-203) before the bf16 rounding; None: fp32 NCHW inputs
     u8_norm: Optional[Tuple[Tuple[float, ...], Tuple[float, ...]]] = None
@@ -153,6 +153,7 @@ class MaxPoolS2DSpec:
     src: str
     dst: str
     c: int
+    split: bool = False          # split precision: src holds hi of class k at k*c and lo at 4c + k*c; the max over hi + lo picks a pair
 
 
 @dataclass
@@ -239,6 +240,7 @@ class AbsDiffSpec:
     c: int
     signed: bool = False         # True: (add +) src[T1] - src[T2], no abs (DTCDSCN: decoder(..) + e_x - e_y, models/DTCDSCN.py:294-300)
     add: Optional[str] = None
+    split: bool = False          # split precision: reads hi + lo, writes both planes
 
 
 @dataclass
@@ -256,6 +258,7 @@ class ChannelGateSpec:
     res: Optional[str] = None
     ws: Optional[np.ndarray] = None   # float32 [c]
     dst_s2d: Optional[str] = None
+    split: bool = False          # split precision: reads src / res as hi + lo, writes both planes (dst_s2d: lo of class k at 4c + k*c)
 
 
 @dataclass
@@ -280,6 +283,7 @@ class BitTransformerSpec:
     dec: np.ndarray              # float32 [n_dec, bit_dec_size]
     softmax: bool = True
     macs_per_pair: int = 0
+    split: bool = False          # split precision: the map is read as hi + lo and written as both planes (the token path is fp32)
 
 
 def bit_enc_fields(c: int, inner: int, mlp: int):
@@ -410,6 +414,7 @@ class SumSpec:
     name: str
     srcs: List[str]
     dst: str
+    split: bool = False          # split precision: the fp32 sum of hi + lo values, written as both planes
 
 
 @dataclass
@@ -946,8 +951,6 @@ def add_conv(
         raise ValueError(f"{name}: act_pre needs the second affine")
     split = prog.split
     if split:
-        if out0_s2d:
-            raise NotImplementedError(f"{name}: split precision has no space-to-depth store")
         fold = False                # folded / horizontally folded forms keep their specialised bf16 epilogues
         segs, phase_taps = _split_operands(prog, name, segs, phase_taps)
         parts = _k_partition(prog, name, segs, phase_taps, cout, pair, max_kc)
@@ -1150,16 +1153,16 @@ def op_bytes_per_pair(prog: Program, op) -> int:
         return 2 * (op.cin * prog.h * prog.w * in_b + t.h * t.w * t.c * 2)
     if isinstance(op, MaxPoolS2DSpec):
         t = T[op.dst]
-        return 2 * (4 * op.c + op.c) * t.h * t.w * 2
+        return 2 * (4 * op.c + op.c) * t.h * t.w * 2 * (2 if op.split else 1)
     if isinstance(op, SegHeadSpec):
         t = T[op.src]
         return (2 + (op.diff_src is not None)) * op.c * t.h * t.w * 2 + 3 * t.h * t.w * 4
     if isinstance(op, AbsDiffSpec):
         t = T[op.dst]
-        return (3 + (op.add is not None)) * op.c * t.h * t.w * 2
+        return (3 + (op.add is not None)) * op.c * t.h * t.w * 2 * (2 if op.split else 1)
     if isinstance(op, ChannelGateSpec):
         t = T[op.src]
-        return t.mult * op.c * t.h * t.w * 2 * (3 + (op.mode == 1) + (op.res is not None) + (op.dst_s2d is not None))
+        return t.mult * op.c * t.h * t.w * 2 * (3 + (op.mode == 1) + (op.res is not None) + (op.dst_s2d is not None)) * (2 if op.split else 1)
     if isinstance(op, SumSpec):
         t = T[op.dst]
         return t.mult * t.c * t.h * t.w * 2 * (len(op.srcs) + 1)
@@ -1177,7 +1180,7 @@ def op_bytes_per_pair(prog: Program, op) -> int:
         return t.mult * op.c * t.h * t.w * 2 * 5
     if isinstance(op, BitTransformerSpec):
         t = T[op.src]
-        return t.mult * op.c * t.h * t.w * 2 * 3            # tokenizer read + decoder read + write
+        return t.mult * op.c * t.h * t.w * 2 * 3 * (2 if op.split else 1)      # tokenizer read + decoder read + write
     if isinstance(op, EcamHeadSpec):
         t = T[op.srcs[0]]
         return 2 * 4 * op.c * t.h * t.w * 2 + op.n_class * t.h * t.w * 4

@@ -39,7 +39,7 @@ class PlannedModule(nn.Module):
         if self.precision not in ("bf16", "tf32"):
             raise ValueError(f"precision must be 'bf16' or 'tf32', got {self.precision!r}")
         if self.precision == "tf32" and not self.supports_precision_path:
-            raise NotImplementedError(f"{type(self).__name__} has no 'tf32' precision path (implemented: the FC-Siam family, SNUNet-CD and ChangeFormerV6)")
+            raise NotImplementedError(f"{type(self).__name__} has no 'tf32' precision path (implemented: the FC-Siam family, SNUNet-CD, ChangeFormerV6, BIT and DTCDSCN)")
         return "split" if self.precision == "tf32" else "bf16"
 
     def __init__(self):

@@ -60,9 +60,10 @@ class Plan:
                               f"uint8 input pack {op.name}")
                 self.u8 = True
             elif isinstance(op, InputPackSpec):
-                if op.split and op.s2d:
-                    raise NotImplementedError("split precision has no space-to-depth input pack")
-                add = lib.stcd_plan_add_input_pack_split if op.split else (lib.stcd_plan_add_input_pack_s2d if op.s2d else lib.stcd_plan_add_input_pack)
+                if op.s2d:
+                    add = lib.stcd_plan_add_input_pack_s2d_split if op.split else lib.stcd_plan_add_input_pack_s2d
+                else:
+                    add = lib.stcd_plan_add_input_pack_split if op.split else lib.stcd_plan_add_input_pack
                 _lib.check_id(add(h, ids[op.dst], op.cin), f"input pack {op.name}")
             elif isinstance(op, GraphConvSpec):
                 rp = None if op.relpos is None else np.ascontiguousarray(op.relpos, np.float32)
@@ -70,16 +71,18 @@ class Plan:
                               f"graph conv {op.name}")
             elif isinstance(op, AbsDiffSpec):
                 if op.signed:
-                    r = lib.stcd_plan_add_subdiff(h, ids[op.src], -1 if op.add is None else ids[op.add], ids[op.dst])
+                    add = lib.stcd_plan_add_subdiff_split if op.split else lib.stcd_plan_add_subdiff
+                    r = add(h, ids[op.src], -1 if op.add is None else ids[op.add], ids[op.dst])
                 else:
-                    r = lib.stcd_plan_add_absdiff(h, ids[op.src], ids[op.dst])
+                    add = lib.stcd_plan_add_absdiff_split if op.split else lib.stcd_plan_add_absdiff
+                    r = add(h, ids[op.src], ids[op.dst])
                 _lib.check_id(r, f"diff {op.name}")
             elif isinstance(op, ChannelGateSpec):
                 w1, w2 = np.ascontiguousarray(op.w1, np.float32), np.ascontiguousarray(op.w2, np.float32)
                 ws = None if op.ws is None else np.ascontiguousarray(op.ws, np.float32)
-                _lib.check_id(lib.stcd_plan_add_channel_gate(h, ids[op.src], -1 if op.res is None else ids[op.res], ids[op.dst],
-                                                             -1 if op.dst_s2d is None else ids[op.dst_s2d], op.c, w1.shape[0],
-                                                             _fptr(w1), _fptr(w2), _fptr(ws), op.mode), f"channel gate {op.name}")
+                add = lib.stcd_plan_add_channel_gate_split if op.split else lib.stcd_plan_add_channel_gate
+                _lib.check_id(add(h, ids[op.src], -1 if op.res is None else ids[op.res], ids[op.dst], -1 if op.dst_s2d is None else ids[op.dst_s2d],
+                                  op.c, w1.shape[0], _fptr(w1), _fptr(w2), _fptr(ws), op.mode), f"channel gate {op.name}")
             elif isinstance(op, BitTransformerSpec):
                 d = _lib.BitDesc()
                 d.c, d.token_len, d.heads, d.mlp = op.c, op.token_len, op.heads, op.mlp
@@ -88,7 +91,8 @@ class Plan:
                 if len(op.enc) == 0:
                     keep[2] = np.zeros(1, np.float32)
                 d.conv_a, d.pos, d.enc, d.dec = (_fptr(a) for a in keep)
-                _lib.check_id(lib.stcd_plan_add_bit_transformer(h, ids[op.src], ids[op.dst], C.byref(d)), f"BIT transformer {op.name}")
+                add = lib.stcd_plan_add_bit_transformer_split if op.split else lib.stcd_plan_add_bit_transformer
+                _lib.check_id(add(h, ids[op.src], ids[op.dst], C.byref(d)), f"BIT transformer {op.name}")
             elif isinstance(op, ChannelAttentionSpec):
                 n = len(op.srcs)
                 ts = (C.c_int * n)(*[ids[s_[0]] for s_ in op.srcs])
@@ -113,7 +117,8 @@ class Plan:
                                                      _fptr(prm)), f"VFFM {op.name}")
             elif isinstance(op, SumSpec):
                 arr = (C.c_int * len(op.srcs))(*[ids[s_] for s_ in op.srcs])
-                _lib.check_id(lib.stcd_plan_add_sum(h, arr, len(op.srcs), ids[op.dst]), f"sum {op.name}")
+                add = lib.stcd_plan_add_sum_split if op.split else lib.stcd_plan_add_sum
+                _lib.check_id(add(h, arr, len(op.srcs), ids[op.dst]), f"sum {op.name}")
             elif isinstance(op, LayerNormSpec):
                 g, b = np.ascontiguousarray(op.gamma, np.float32), np.ascontiguousarray(op.beta, np.float32)
                 add = lib.stcd_plan_add_layernorm_split if op.split else lib.stcd_plan_add_layernorm
@@ -130,7 +135,8 @@ class Plan:
                 add = lib.stcd_plan_add_bilinear_up_split if op.split else lib.stcd_plan_add_bilinear_up
                 _lib.check_id(add(h, ids[op.src], ids[op.dst], op.c, op.scale), f"bilinear {op.name}")
             elif isinstance(op, MaxPoolS2DSpec):
-                _lib.check_id(lib.stcd_plan_add_maxpool_s2d(h, ids[op.src], ids[op.dst], op.c), f"maxpool {op.name}")
+                add = lib.stcd_plan_add_maxpool_s2d_split if op.split else lib.stcd_plan_add_maxpool_s2d
+                _lib.check_id(add(h, ids[op.src], ids[op.dst], op.c), f"maxpool {op.name}")
             elif isinstance(op, SegHeadSpec):
                 d = _lib.SegHeadDesc()
                 d.src, d.c, d.bias, d.out_ext = ids[op.src], op.c, float(op.bias), op.out_ext

@@ -1,12 +1,13 @@
-"""Step time of config C5 (ChangeFormerV6, 32 pairs of 256 x 256, chunk 32) at bf16 and on the precision path ("tf32": split-bf16
-operands), measured in one process on one GPU.
+"""Step time of a bench.py workload (default changeformer_v6_256_b32, config C5: ChangeFormerV6, 32 pairs of 256 x 256, chunk 32)
+at bf16 and on the precision path ("tf32": split-bf16 operands), measured in one process on one GPU.  The net, batch and chunk
+are bench.py's (WORKLOADS, build_net).
 
-    python tools/precision_step.py [--reps 3] [--window 2.0] [--profile-dir DIR]
+    python tools/precision_step.py [--workload changeformer_v6_256_b32] [--reps 3] [--window 2.0] [--profile-dir DIR]
 
 * the card's name, power limit and max SM clock (nvidia-smi, read-only query);
 * the two precisions alternate, each repeated --reps times; a timed window is >= --window seconds of back-to-back steps on
-  device-resident inputs between two CUDA events after a synchronise (inputs 2 x 25 MB: the working set is the plan's ~GB of
-  activations, far beyond the 126 MB L2);
+  device-resident inputs between two CUDA events after a synchronise (C5's inputs are 2 x 25 MB: the working set is the plan's
+  ~GB of activations, far beyond the 126 MB L2);
 * per-op device time of one step of each precision (the plan's own CUDA events around every launch), summed by op kind;
 * a separate torch.profiler pass over tf32 steps: per-kernel device time of the split kernels (template argument `true`) and
   of the conv kernel.
@@ -24,9 +25,8 @@ sys.path.insert(0, ROOT)
 
 import torch  # noqa: E402
 
-from stcd_b200 import changeformer, lowering as L, synth  # noqa: E402
-
-PAIRS, CHUNK = 32, 32
+import bench  # noqa: E402
+from stcd_b200 import lowering as L, synth  # noqa: E402
 
 
 def card() -> str:
@@ -46,7 +46,7 @@ def window(net, a, b, seconds: float, est_ms: float) -> float:
     e1.synchronize()
     ms = e0.elapsed_time(e1)
     assert ms >= seconds * 1e3 * 0.9, f"window too short: {ms:.0f} ms"
-    return n * PAIRS / (ms / 1e3)
+    return n * a.shape[0] / (ms / 1e3)
 
 
 def op_kind(prog, name: str) -> str:
@@ -58,6 +58,7 @@ def op_kind(prog, name: str) -> str:
 
 def main() -> None:
     ap = argparse.ArgumentParser()
+    ap.add_argument("--workload", default="changeformer_v6_256_b32", choices=sorted(bench.WORKLOADS))
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--window", type=float, default=2.0)
     ap.add_argument("--profile-dir", default=None, help="also export the profiler trace there")
@@ -66,9 +67,11 @@ def main() -> None:
         raise SystemExit("needs a CUDA device (no CPU timing)")
     print(card())
     print(torch.cuda.get_device_name(0))
-    net = synth.prepare_(changeformer.ChangeFormerV6(3, 2, embed_dim=256).eval(), "ChangeFormerV6").cuda()
-    net.chunk_pairs = CHUNK
-    x1, x2 = synth.image_pairs(PAIRS, 256, 256)
+    wl = bench.WORKLOADS[args.workload]
+    print(f"{args.workload}: {wl['desc']}")
+    net = bench.build_net(wl).cuda()
+    net.chunk_pairs = wl.get("chunk", net.default_chunk_pairs)
+    x1, x2 = synth.image_pairs(wl["batch"], wl["h"], wl["w"])
     a, b = x1.cuda(), x2.cuda()
     est = {}
     for prec in ("bf16", "tf32"):                       # warm-up: plans, modules, clocks
@@ -91,7 +94,7 @@ def main() -> None:
             print(f"rep {rep} {prec}: {rates[prec][-1]:.1f} pairs/s")
     med = {p: sorted(v)[len(v) // 2] for p, v in rates.items()}
     spread = {p: (max(v) - min(v)) / med[p] for p, v in rates.items()}
-    print(f"C5 bf16: {med['bf16']:.1f} pairs/s (spread {100 * spread['bf16']:.1f} %), tf32: {med['tf32']:.1f} pairs/s "
+    print(f"{args.workload} bf16: {med['bf16']:.1f} pairs/s (spread {100 * spread['bf16']:.1f} %), tf32: {med['tf32']:.1f} pairs/s "
           f"(spread {100 * spread['tf32']:.1f} %); tf32 step / bf16 step = {med['bf16'] / med['tf32']:.2f}x")
 
     # per-op device time of one step (the plan's CUDA events around every launch), by op kind
