@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define STCD_ABI_VERSION 20
+#define STCD_ABI_VERSION 21
 
 enum stcd_status {
   STCD_OK = 0,
@@ -55,12 +55,24 @@ int stcd_device_count(void);
 /* activations stay resident in the 126 MB L2.                                                 */
 
 /* device = -1 creates a VALIDATION plan: every stcd_plan_add_* call checks and records its descriptor exactly as on a
- * device, stcd_plan_finalize returns STCD_ERR_NO_DEVICE (host-side tests of the lowering run without a GPU). */
-int stcd_plan_create(int device, int chunk_pairs, stcd_plan** out);
+ * device, stcd_plan_finalize returns STCD_ERR_NO_DEVICE (host-side tests of the lowering run without a GPU).
+ *
+ * precision: STCD_PRECISION_BF16 or STCD_PRECISION_SPLIT, for every op of the plan.  Split precision is the tolerance class
+ * the north star calls "tf32": logits within 1e-3 of the fp32 reference; the reference itself computes in fp32,
+ * models/SNUNet.py:116-152.  In a split plan every tensor stores 2x its logical channels, a multiple of 16
+ * (stcd_plan_add_tensor refuses any other count): a hi plane bf16(v) in channel groups [0, c8/2) and a lo plane
+ * bf16(v - hi) in [c8/2, c8).  A conv's K-program (built by the host) reads each logical source as the three segments
+ * (hi, lo, hi) against the weights (Whi, Whi, Wlo); its epilogue writes both planes of out0 / out_raw / out_pool / out_diff
+ * and reads the residual as hi + lo.  A space-to-depth out0 stores 8*cout channels: hi of parity class k at k*cout, lo at
+ * 4*cout + k*cout; fold_cs and xf_cs are refused.  The other ops read hi + lo, compute in fp32 and write hi = bf16(v),
+ * lo = bf16(v - hi); their comments give the layouts as "split plan:" lines.  Graph conv, channel attention, spatial gate,
+ * global-local gate, CSAM gate, VFFM, seg head and the uint8 input pack have no split form and are refused. */
+enum stcd_precision { STCD_PRECISION_BF16 = 0, STCD_PRECISION_SPLIT = 1 };
+int stcd_plan_create(int device, int chunk_pairs, int precision, stcd_plan** out);
 void stcd_plan_destroy(stcd_plan* plan);
 
 /* Declare an activation tensor of img_mult*chunk_pairs images, bf16 [img][c/8][h][w][8].
- * Returns id >= 0, or <0. */
+ * split plan: c is a multiple of 16 (two planes of 8-channel groups).  Returns id >= 0, or <0. */
 int stcd_plan_add_tensor(stcd_plan* plan, int img_mult, int h, int w, int c, int dtype);
 
 /* Activation tensors are stored channel-chunked: bf16 [img][c/8][h][w][8] ("NC8HW8"), so that a
@@ -167,13 +179,6 @@ typedef struct stcd_conv_desc {
    * blocks across neighbouring pixels.  Tiles are 8 x 16 input positions with 14 output columns (the library's choice;
    * hg / wg stay the output dims).  Single phase, stride-1 sources, osy = osx = 1, no space-to-depth / folded store. */
   int32_t xf_cs;
-  /* Split precision (the tolerance class the north star calls "tf32": logits within 1e-3 of the fp32 reference; the reference
-   * itself computes in fp32, models/SNUNet.py:116-152).  split = 1: every bf16 tensor this op touches stores 2x its logical
-   * channels -- a hi plane bf16(v) in channel groups [0, c8/2) and a lo plane bf16(v - hi) in [c8/2, c8) -- the K-program
-   * (built by the host) reads each logical source as the three segments (hi, lo, hi) against the weights (Whi, Whi, Wlo), the
-   * epilogue writes both planes of out0 / out_raw / out_pool / out_diff and reads the residual as hi + lo.  A space-to-depth
-   * out0 stores 8*cout channels: hi of parity class k at k*cout, lo at 4*cout + k*cout.  Not combined with fold_cs or xf_cs. */
-  int32_t split;
 } stcd_conv_desc;
 
 /* returns op index >= 0, or <0 */
@@ -181,31 +186,33 @@ int stcd_plan_add_conv(stcd_plan* plan, const stcd_conv_desc* desc);
 
 /* x1, x2 (fp32 NCHW [n_pairs, cin, h, w], the reference's input layout: data/dataset.py:196-203)
  * -> bf16 [2*chunk][2][h][w][8] (cin <= 8 real channels, 16 stored) with the T1 images first, then
- * the T2 images. */
+ * the T2 images.
+ * split plan: dst has 16 stored channels, [0, 8) = bf16(x), [8, 16) = bf16(x - bf16(x)); cin <= 8. */
 int stcd_plan_add_input_pack(stcd_plan* plan, int dst_tensor, int cin);
-
-/* Split-precision variant (see stcd_conv_desc.split): dst has 16 stored channels, [0, 8) = bf16(x), [8, 16) = bf16(x - bf16(x));
- * cin <= 8. */
-int stcd_plan_add_input_pack_split(stcd_plan* plan, int dst_tensor, int cin);
 
 /* Space-to-depth variant for the 7x7 stride-2 ResNet stem (smp/encoders/resnet.py:50): x1, x2 fp32 NCHW
  * [n_pairs, cin, 2h, 2w] -> bf16 [2*chunk][2][h][w][8] with channel (py*2 + px)*cin + c holding
- * x[c][2y + py][2x + px] (4*cin <= 16); the stem then runs as a 4x4 stride-1 conv. */
+ * x[c][2y + py][2x + px] (4*cin <= 16); the stem then runs as a 4x4 stride-1 conv.
+ * split plan: dst stores 32 channels, the hi plane in [0, 16) (channel (py*2 + px)*cin + c), the lo plane in [16, 32). */
 int stcd_plan_add_input_pack_s2d(stcd_plan* plan, int dst_tensor, int cin);
 
 /* uint8 input pipeline (SURVEY.md §8(f)-1; reference: data/dataset.py:196-203, ToTensor + Normalize on the host).
  * Same as stcd_plan_add_input_pack / _s2d, but the plan's inputs become uint8 HWC images [n_pairs, H, W, cin] and
  * the pack kernel evaluates ((u / 255) - mean[c]) / std[c] in fp32 (IEEE ops, the reference's expression) before
  * the bf16 rounding: bit-identical to packing the host-normalised fp32 tensor, at a quarter of the PCIe bytes.
- * A plan built with this op is run with stcd_forward_u8 / stcd_forward_host_u8.  mean, std: HOST float[cin]. */
+ * A plan built with this op is run with stcd_forward_u8 / stcd_forward_host_u8.  mean, std: HOST float[cin].
+ * Refused in a split plan. */
 int stcd_plan_add_input_pack_u8(stcd_plan* plan, int dst_tensor, int cin, int s2d, const float* mean, const float* std_);
 
 /* nn.MaxPool2d(kernel_size=3, stride=2, padding=1) (smp/encoders/resnet.py:51) over a feature map stored
- * space-to-depth (src: [h][w] pixels x 4c channels = the (2h x 2w) map) -> dst [h][w] x c channels. */
+ * space-to-depth (src: [h][w] pixels x 4c channels = the (2h x 2w) map) -> dst [h][w] x c channels.
+ * split plan: src stores 8c channels (hi of parity class k at k*c, lo at 4c + k*c), dst 2c; the max over hi + lo selects the
+ *   winning (hi, lo) pair (first maximum in the kernel's window order). */
 int stcd_plan_add_maxpool_s2d(stcd_plan* plan, int src_tensor, int dst_tensor, int c);
 
 /* dst = |src[T1 images] - src[T2 images]| (torch.abs(f1 - f2), FFCTLCD.forward, decoders/unet/model.py:412): src holds
- * both temporal streams (mult 2), dst one stream with the same [h][w][c] (any layout: elementwise). */
+ * both temporal streams (mult 2), dst one stream with the same [h][w][c] (any layout: elementwise).
+ * split plan (subdiff too): every tensor stores hi and lo planes. */
 int stcd_plan_add_absdiff(stcd_plan* plan, int src_tensor, int dst_tensor);
 /* the signed variant dst = (add) + src[T1] - src[T2] (DTCDSCN: decoder(...) + e_x - e_y, models/DTCDSCN.py:294-300);
  * add_or_neg: a one-stream tensor of dst's shape, or -1 */
@@ -215,7 +222,8 @@ int stcd_plan_add_subdiff(stcd_plan* plan, int src_tensor, int add_or_neg, int d
  * w1 HOST fp32 [hid][c], w2 HOST fp32 [c][hid] (bias-free: SELayer :14-19, SCSEBlock.channel_excitation :153-158).
  *   mode 0 (SEBasicBlock tail, :93-109):  dst = relu(src * g + res)        res_or_neg: tensor id or -1
  *   mode 1 (DecoderBlock, :129-135):       dst = src * (1 + g + sigmoid(ws . src_pixel))   ws HOST fp32 [c] (spatial_se :160-162)
- * dst_s2d_or_neg >= 0 also writes the space-to-depth copy.  c <= 512, hid <= 32. */
+ * dst_s2d_or_neg >= 0 also writes the space-to-depth copy.  c <= 512, hid <= 32.
+ * split plan: src, res, dst store 2c channels; the space-to-depth copy 8c (hi of parity class k at k*c, lo at 4c + k*c). */
 int stcd_plan_add_channel_gate(stcd_plan* plan, int src_tensor, int res_or_neg, int dst_tensor, int dst_s2d_or_neg, int c, int hid,
                                const float* w1, const float* w2, const float* ws_or_null, int mode);
 
@@ -226,7 +234,8 @@ int stcd_plan_add_channel_gate(stcd_plan* plan, int src_tensor, int res_or_neg, 
  *   enc row: ln1_g[c] ln1_b[c] Wqkv[3*inner_enc][c] Wout[c][inner_enc] bout[c] ln2_g[c] ln2_b[c] W1[mlp][c] b1[mlp] W2[c][mlp] b2[c]
  *   dec row: ln1_g[c] ln1_b[c] Wq[inner_dec][c] Wk[..][c] Wv[..][c] Wout^T[inner_dec][c] bout[c] ln2_g[c] ln2_b[c]
  *            W1^T[c][mlp] b1[mlp] W2^T[mlp][c] b2[c]
- * (torch Linear layouts [out][in]; the decoder's to_out and feed-forward weights transposed). */
+ * (torch Linear layouts [out][in]; the decoder's to_out and feed-forward weights transposed).
+ * split plan: src and dst store 64 channels (2 x 32); the token path itself is fp32 in both precisions. */
 typedef struct {
   int32_t c, token_len, heads, mlp;
   int32_t n_enc, n_dec, inner_enc, inner_dec;
@@ -269,7 +278,8 @@ int stcd_plan_add_csam_gate(stcd_plan* plan, int src_tensor, int dst_tensor, int
 int stcd_plan_add_vffm(stcd_plan* plan, int low_tensor, int high_tensor, int mixed_tensor, int local_tensor, int dst_tensor, int c,
                        int inter, const float* prm);
 
-/* dst = sum of n <= 5 plan tensors of identical shape (Dblock.forward: x + d1 + d2 + d3 + d4, models/DTCDSCN.py:65-71) */
+/* dst = sum of n <= 5 plan tensors of identical shape (Dblock.forward: x + d1 + d2 + d3 + d4, models/DTCDSCN.py:65-71).
+ * split plan: every tensor stores hi and lo planes. */
 int stcd_plan_add_sum(stcd_plan* plan, const int* src_tensors, int n, int dst_tensor);
 
 /* SegCD's tail (segmentation_models_pytorch/decoders/unet/model.py:321-330) as one op over the decoder
@@ -297,7 +307,8 @@ int stcd_plan_add_graph_conv(stcd_plan* plan, int src_tensor, int dst_tensor, in
                              const float* relative_pos);
 
 /* F.interpolate(x, scale_factor=scale, mode="bilinear", align_corners=False) between two plan tensors
- * (ChangeVIG.py:246-262); dst is [scale*h][scale*w], first c channels. */
+ * (ChangeVIG.py:246-262); dst is [scale*h][scale*w], first c channels.
+ * split plan: src and dst store 2c channels. */
 int stcd_plan_add_bilinear_up(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int scale);
 
 /* MiT / ChangeFormer encoder ops between plan tensors (models/ChangeFormer.py).
@@ -306,51 +317,26 @@ int stcd_plan_add_bilinear_up(stcd_plan* plan, int src_tensor, int dst_tensor, i
  *   gamma, beta: HOST fp32 [c].
  * sr_attention: softmax(q k^T * scale) v per head (:338-358); q, dst [imgs][h][w][c], kv [imgs][hk][wk][2c] with
  *   k = channels [0, c), v = [c, 2c); hk*wk <= 64 keys, c / heads in {64, 80}.
- * dwconv3x3: depth-wise 3x3 (padding 1) + bias, then GELU if gelu != 0 (:283-289,512-523); weight HOST fp32 [c][9]. */
+ * dwconv3x3: depth-wise 3x3 (padding 1) + bias, then GELU if gelu != 0 (:283-289,512-523); weight HOST fp32 [c][9].
+ * split plan:
+ *   layernorm: src and dst store 2c channels; the space-to-depth copy stores 8c: hi of parity class k, channel ch at k*c + ch,
+ *     lo at 4c + k*c + ch.
+ *   sr_attention: q and dst store 2c, kv 4c (k hi [0, c), v hi [c, 2c), k lo [2c, 3c), v lo [3c, 4c)); exactly 64 keys.
+ *     S = Qhi Khi^T + Qlo Khi^T + Qhi Klo^T, fp32 softmax, P split into hi + lo, O = Phi Vhi + Plo Vhi + Phi Vlo, normalised
+ *     by the fp32 row sum.
+ *   dwconv3x3: src and dst store 2c channels. */
 int stcd_plan_add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d_or_neg, int c, const float* gamma,
                             const float* beta, float eps);
 int stcd_plan_add_sr_attention(stcd_plan* plan, int q_tensor, int kv_tensor, int dst_tensor, int c, int heads, float scale);
 int stcd_plan_add_dwconv3x3(stcd_plan* plan, int src_tensor, int dst_tensor, int c, const float* weight, const float* bias,
                             int gelu);
 
-/* Split-precision variants (see stcd_conv_desc.split), same arguments as the functions above.  Every tensor holds a value as
- * hi + lo bf16 planes: a tensor of c logical channels stores 2c (a multiple of 16), the hi plane in channels [0, c) and the lo
- * plane in [c, 2c), hi = bf16(v), lo = bf16(v - hi).  The kernels read hi + lo, compute in fp32 and write both planes.
- * layernorm_split: src and dst store 2c channels; the space-to-depth copy stores 8c: hi of parity class k, channel ch at
- *   k*c + ch, lo at 4c + k*c + ch.
- * sr_attention_split: q and dst store 2c, kv 4c (k hi [0, c), v hi [c, 2c), k lo [2c, 3c), v lo [3c, 4c)); exactly 64 keys.
- *   S = Qhi Khi^T + Qlo Khi^T + Qhi Klo^T, fp32 softmax, P split into hi + lo, O = Phi Vhi + Plo Vhi + Phi Vlo, normalised by
- *   the fp32 row sum.
- * dwconv3x3_split, bilinear_up_split: src and dst store 2c channels. */
-int stcd_plan_add_layernorm_split(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d_or_neg, int c, const float* gamma,
-                                  const float* beta, float eps);
-int stcd_plan_add_sr_attention_split(stcd_plan* plan, int q_tensor, int kv_tensor, int dst_tensor, int c, int heads, float scale);
-int stcd_plan_add_dwconv3x3_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, const float* weight, const float* bias,
-                                  int gelu);
-int stcd_plan_add_bilinear_up_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int scale);
-
-/* Split-precision variants of the ResNet-family ops (BIT, DTCDSCN), same arguments as the functions above and the same hi + lo
- * layout; each reads hi + lo, computes in fp32 in the order of its bf16 form and writes hi = bf16(v), lo = bf16(v - hi).
- * input_pack_s2d_split: dst stores 32 channels, the hi plane in [0, 16) (channel (py*2 + px)*cin + c), the lo plane in [16, 32).
- * maxpool_s2d_split: src stores 8c channels (hi of parity class k at k*c, lo at 4c + k*c), dst 2c; the max over hi + lo selects
- *   the winning (hi, lo) pair (first maximum in the kernel's window order).
- * absdiff_split, subdiff_split, sum_split: every tensor stores hi and lo planes (channels a multiple of 16).
- * channel_gate_split: src, res, dst store 2c channels; the space-to-depth copy 8c (as layernorm_split's).
- * bit_transformer_split: src and dst store 64 channels (2 x 32); the token path itself is fp32 in both forms. */
-int stcd_plan_add_input_pack_s2d_split(stcd_plan* plan, int dst_tensor, int cin);
-int stcd_plan_add_maxpool_s2d_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c);
-int stcd_plan_add_absdiff_split(stcd_plan* plan, int src_tensor, int dst_tensor);
-int stcd_plan_add_subdiff_split(stcd_plan* plan, int src_tensor, int add_or_neg, int dst_tensor);
-int stcd_plan_add_sum_split(stcd_plan* plan, const int* src_tensors, int n, int dst_tensor);
-int stcd_plan_add_channel_gate_split(stcd_plan* plan, int src_tensor, int res_or_neg, int dst_tensor, int dst_s2d_or_neg, int c,
-                                     int hid, const float* w1, const float* w2, const float* ws_or_null, int mode);
-int stcd_plan_add_bit_transformer_split(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* desc);
-
 /* SNUNet's ECAM tail (models/SNUNet.py:144-149: two ChannelAttention blocks :46-59 + conv_final)
  * over four activation tensors of `c` channels each, as one fused op writing external output
  * `out_ext` (fp32 NCHW [n, n_class, h, w]).  All weight pointers are HOST fp32, copied at add time:
  * ca_fc1 [r][4c], ca_fc2 [4c][r], ca1_fc1 [r1][c], ca1_fc2 [c][r1], w_final [n_class][4c],
- * b_final [n_class].  Limits: c % 8 == 0, c <= 64, r, r1 <= 16, n_class <= 4. */
+ * b_final [n_class].  Limits: c % 8 == 0, c <= 64, r, r1 <= 16, n_class <= 4.
+ * split plan: each source stores 2c channels (hi plane, lo plane) and is read as hi + lo. */
 typedef struct stcd_ecam_desc {
   int32_t src[4];
   int32_t c, n_class, r, r1;
@@ -361,7 +347,6 @@ typedef struct stcd_ecam_desc {
   const float* w_final;
   const float* b_final;
   int32_t out_ext;
-  int32_t split;      /* split precision: each source stores 2c channels (hi plane, lo plane) and is read as hi + lo */
 } stcd_ecam_desc;
 int stcd_plan_add_ecam_head(stcd_plan* plan, const stcd_ecam_desc* desc);
 

@@ -145,7 +145,6 @@ class ConvDesc(C.Structure):
         ("fold_cs", C.c_int32), ("fold_cout", C.c_int32),
         ("act_pre", C.c_int32), ("act_alpha", C.c_float),
         ("xf_cs", C.c_int32),
-        ("split", C.c_int32),
     ]
 
 
@@ -170,23 +169,22 @@ class EcamDesc(C.Structure):
         ("ca1_fc1", C.POINTER(C.c_float)), ("ca1_fc2", C.POINTER(C.c_float)),
         ("w_final", C.POINTER(C.c_float)), ("b_final", C.POINTER(C.c_float)),
         ("out_ext", C.c_int32),
-        ("split", C.c_int32),
     ]
 
 
-ABI_VERSION = 20
+ABI_VERSION = 21
+PRECISION_BF16, PRECISION_SPLIT = 0, 1        # enum stcd_precision
 
 # every symbol include/stcd_b200.h declares: (name, restype, argtypes)
 SYMBOLS = [
     ("stcd_last_error", C.c_char_p, []),
     ("stcd_abi_version", C.c_int, []),
     ("stcd_device_count", C.c_int, []),
-    ("stcd_plan_create", C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    ("stcd_plan_create", C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
     ("stcd_plan_destroy", None, [C.c_void_p]),
     ("stcd_plan_add_tensor", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     ("stcd_plan_add_conv", C.c_int, [C.c_void_p, C.POINTER(ConvDesc)]),
     ("stcd_plan_add_input_pack", C.c_int, [C.c_void_p, C.c_int, C.c_int]),
-    ("stcd_plan_add_input_pack_split", C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     ("stcd_plan_add_input_pack_s2d", C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     ("stcd_plan_add_input_pack_u8", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     ("stcd_plan_add_maxpool_s2d", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
@@ -210,19 +208,6 @@ SYMBOLS = [
     ("stcd_plan_add_sr_attention", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float]),
     ("stcd_plan_add_dwconv3x3", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int]),
     ("stcd_plan_add_bilinear_up", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]),
-    ("stcd_plan_add_layernorm_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float),
-                                                C.c_float]),
-    ("stcd_plan_add_sr_attention_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float]),
-    ("stcd_plan_add_dwconv3x3_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int]),
-    ("stcd_plan_add_bilinear_up_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]),
-    ("stcd_plan_add_input_pack_s2d_split", C.c_int, [C.c_void_p, C.c_int, C.c_int]),
-    ("stcd_plan_add_maxpool_s2d_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
-    ("stcd_plan_add_absdiff_split", C.c_int, [C.c_void_p, C.c_int, C.c_int]),
-    ("stcd_plan_add_subdiff_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int]),
-    ("stcd_plan_add_sum_split", C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_int, C.c_int]),
-    ("stcd_plan_add_channel_gate_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float),
-                                                   C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int]),
-    ("stcd_plan_add_bit_transformer_split", C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     ("stcd_plan_add_ecam_head", C.c_int, [C.c_void_p, C.c_void_p]),
     ("stcd_plan_finalize", C.c_int, [C.c_void_p]),
     ("stcd_plan_tensor_copy", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.c_int]),

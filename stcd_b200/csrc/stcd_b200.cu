@@ -94,12 +94,10 @@ struct PackOp {
   int s2d = 0;
   int u8 = 0;                 // inputs are uint8 HWC, normalised in the pack kernel
   stcd::NormParams norm;
-  int split = 0;              // split precision: channels [8, 16) = lo parts of channels [0, 8)
 };
 
 struct PoolOp {
   int src, dst, c;
-  int split = 0;              // split precision (lowering.Program.precision): src, dst hold hi and lo planes
 };
 
 struct GraphOp {
@@ -118,10 +116,8 @@ struct GraphOp {
   float* ysq = nullptr;        // r > 1
 };
 
-// split: split precision (lowering.Program.precision), every tensor of the op holds a hi and a lo plane
 struct BilinearOp {
   int src, dst, c, scale;
-  int split = 0;
 };
 
 struct LayerNormOp {
@@ -129,27 +125,23 @@ struct LayerNormOp {
   float eps;
   std::vector<float> gb;   // gamma | beta
   float* gb_dev = nullptr;
-  int split = 0;
 };
 
 struct AttentionOp {
   int q, kv, dst, c, heads;
   float scale;
-  int split = 0;
 };
 
 struct DWConvOp {
   int src, dst, c, gelu;
   std::vector<float> wb;   // weight [c][9] | bias [c]
   float* wb_dev = nullptr;
-  int split = 0;
 };
 
 struct AbsDiffOp {
   int src, dst, c;
   int signed_diff = 0;
   int add = -1;
-  int split = 0;
 };
 
 struct GateOp {
@@ -157,7 +149,6 @@ struct GateOp {
   std::vector<float> w;      // w1 [hid][c] | w2 [c][hid] | ws [c] (mode 1)
   float* w_dev = nullptr;
   float* partial = nullptr;  // [imgs][ranges][c]
-  int split = 0;
 };
 
 struct BitOp {
@@ -170,7 +161,6 @@ struct BitOp {
   size_t coef_smem = 0;
   float* coef = nullptr;       // [2*chunk][n_dec][A | Bm]
   size_t mixer_smem = 0;
-  int split = 0;               // the feature map holds hi and lo planes (the token path is fp32 either way)
 };
 
 struct ChanAttnOp {
@@ -209,7 +199,6 @@ struct VffmOp {
 
 struct SumOp {
   int src[5], n, dst;
-  int split = 0;
 };
 
 struct SegHeadOp {
@@ -239,6 +228,7 @@ struct Op {
 struct stcd_plan {
   int device = 0;
   int chunk = 0;
+  int split = 0;             // STCD_PRECISION_SPLIT: every tensor holds a hi and a lo plane, every op runs its split form
   bool finalized = false;
   std::vector<Tensor> tensors;
   std::vector<ConvOp> convs;
@@ -441,7 +431,7 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const Tensor& td = plan->tensors[k.dst];
       const size_t total = (size_t)td.mult * plan->chunk * (k.c / 8) * td.h * td.w;
       const int blocks = (int)std::min<size_t>((total + 255) / 256, 148 * 16);
-      auto kern = k.split ? stcd::maxpool3x3s2_s2d_kernel<true> : stcd::maxpool3x3s2_s2d_kernel<false>;
+      auto kern = plan->split ? stcd::maxpool3x3s2_s2d_kernel<true> : stcd::maxpool3x3s2_s2d_kernel<false>;
       kern<<<blocks, 256, 0, st>>>((const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, td.mult * plan->chunk, k.c / 8, td.c / 8, td.h,
                                    td.w);
       CUDA_TRY(cudaGetLastError());
@@ -473,9 +463,9 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
     } else if (o.kind == 10) {
       const AbsDiffOp& k = plan->absdiffs[o.idx];
       const Tensor& td = plan->tensors[k.dst];
-      const size_t vecs = td.bytes / 16 / (k.split ? 2 : 1);     // 16-byte (hi) vectors per stream (dst holds one stream)
+      const size_t vecs = td.bytes / 16 / (plan->split ? 2 : 1); // 16-byte (hi) vectors per stream (dst holds one stream)
       const int plane_vecs = (td.c / 16) * td.h * td.w;            // split: vectors of one plane of one image
-      auto kern = k.split ? stcd::absdiff_kernel<true> : stcd::absdiff_kernel<false>;
+      auto kern = plan->split ? stcd::absdiff_kernel<true> : stcd::absdiff_kernel<false>;
       kern<<<(unsigned)std::max<size_t>(1, std::min<size_t>((vecs + 255) / 256, 148 * 16)), 256, 0, st>>>(
           (const __nv_bfloat16*)plan->tensors[k.src].ptr, (__nv_bfloat16*)td.ptr, vecs, k.signed_diff,
           k.add >= 0 ? (const __nv_bfloat16*)plan->tensors[k.add].ptr : nullptr, plane_vecs);
@@ -486,14 +476,14 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const Tensor& td = plan->tensors[k.dst];
       const int B = ts.mult * plan->chunk, hw = ts.h * ts.w;
       const int n_items = B * (k.c / 8) * k.ranges;   // one warp each
-      (k.split ? stcd::chan_sum_kernel<true> : stcd::chan_sum_kernel<false>)<<<(n_items + 7) / 8, 256, 0, st>>>(
+      (plan->split ? stcd::chan_sum_kernel<true> : stcd::chan_sum_kernel<false>)<<<(n_items + 7) / 8, 256, 0, st>>>(
           (const __nv_bfloat16*)ts.ptr, k.partial, k.c, ts.c / 8, hw, k.ranges, n_items);
       // ~2048 (pixel, channel group) items per CTA: enough CTAs to fill the machine on every level of the pyramid
       const int ppb = std::max(32, std::min(stcd::kGateMaxPix, 2048 / (k.c / 8)));
       const float* w1 = k.w_dev;
       const float* w2 = w1 + (size_t)k.hid * k.c;
       const float* ws = k.mode == 1 ? w2 + (size_t)k.c * k.hid : nullptr;
-      (k.split ? stcd::gate_apply_kernel<true> : stcd::gate_apply_kernel<false>)<<<dim3((hw + ppb - 1) / ppb, B), 256, 0, st>>>(
+      (plan->split ? stcd::gate_apply_kernel<true> : stcd::gate_apply_kernel<false>)<<<dim3((hw + ppb - 1) / ppb, B), 256, 0, st>>>(
           (const __nv_bfloat16*)ts.ptr, k.res >= 0 ? (const __nv_bfloat16*)plan->tensors[k.res].ptr : nullptr, (__nv_bfloat16*)td.ptr,
           k.dst2 >= 0 ? (__nv_bfloat16*)plan->tensors[k.dst2].ptr : nullptr, k.partial, w1, w2, ws, k.c, k.hid, ts.c / 8,
           k.res >= 0 ? plan->tensors[k.res].c / 8 : 0, td.c / 8, k.dst2 >= 0 ? plan->tensors[k.dst2].c / 8 : 0, ts.h, ts.w, k.ranges, k.mode,
@@ -571,14 +561,14 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const float* pos = conv_a + stcd::kBitL * stcd::kBitC;
       const float* enc = pos + 2 * stcd::kBitL * stcd::kBitC;
       const float* dec = enc + (size_t)k.d.n_enc * stcd::bit_enc_size(k.d.inner_enc);
-      (k.split ? stcd::bit_tokenizer_kernel<true> : stcd::bit_tokenizer_kernel<false>)<<<imgs, 256, 0, st>>>(
+      (plan->split ? stcd::bit_tokenizer_kernel<true> : stcd::bit_tokenizer_kernel<false>)<<<imgs, 256, 0, st>>>(
           (const __nv_bfloat16*)ts.ptr, conv_a, k.tokens, ts.c / 8, hw);
       const float scale = 1.f / sqrtf((float)stcd::kBitC);     // dim ** -0.5 with dim = 32 (help_funcs.py:74,118), not dim_head
       stcd::bit_token_mixer_kernel<<<plan->chunk, 256, k.mixer_smem, st>>>(k.tokens, pos, enc, k.tok_mixed, plan->chunk, k.d.n_enc,
                                                                           k.d.inner_enc, scale);
       stcd::bit_coef_kernel<<<dim3(plan->chunk, k.d.n_dec), 256, k.coef_smem, st>>>(k.tok_mixed, dec, k.coef, plan->chunk, k.d.n_dec,
                                                                                    k.d.inner_dec, scale);
-      (k.split ? stcd::bit_decoder_kernel<true> : stcd::bit_decoder_kernel<false>)<<<
+      (plan->split ? stcd::bit_decoder_kernel<true> : stcd::bit_decoder_kernel<false>)<<<
           dim3((hw + 2 * stcd::kBitDecThreads - 1) / (2 * stcd::kBitDecThreads), imgs), stcd::kBitDecThreads, 0, st>>>(
           (const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, dec, k.coef, ts.c / 8, td.c / 8, hw, k.d.n_dec, k.d.inner_dec, k.d.softmax);
       CUDA_TRY(cudaGetLastError());
@@ -588,8 +578,8 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       stcd::AddNParams ap;
       ap.n = k.n;
       for (int i = 0; i < 5; ++i) ap.src[i] = i < k.n ? (const __nv_bfloat16*)plan->tensors[k.src[i]].ptr : nullptr;
-      const size_t vecs = td.bytes / 16 / (k.split ? 2 : 1);     // (hi) vectors
-      auto kern = k.split ? stcd::add_n_kernel<true> : stcd::add_n_kernel<false>;
+      const size_t vecs = td.bytes / 16 / (plan->split ? 2 : 1); // (hi) vectors
+      auto kern = plan->split ? stcd::add_n_kernel<true> : stcd::add_n_kernel<false>;
       kern<<<(unsigned)std::max<size_t>(1, std::min<size_t>((vecs + 255) / 256, 148 * 16)), 256, 0, st>>>(ap, (__nv_bfloat16*)td.ptr, vecs,
                                                                                                         (td.c / 16) * td.h * td.w);
       CUDA_TRY(cudaGetLastError());
@@ -602,7 +592,7 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       __nv_bfloat16* d2 = k.dst2 >= 0 ? (__nv_bfloat16*)plan->tensors[k.dst2].ptr : nullptr;
       // 4 threads per pixel (a warp = 8 pixels x 4 channel slices)
       const unsigned blocks = (unsigned)std::max<size_t>(1, std::min<size_t>((total * 4 + 255) / 256, 148 * 16));
-      auto kern = k.split ? stcd::layernorm_kernel<true> : stcd::layernorm_kernel<false>;
+      auto kern = plan->split ? stcd::layernorm_kernel<true> : stcd::layernorm_kernel<false>;
       kern<<<blocks, 256, 0, st>>>((const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, d2, k.gb_dev, k.gb_dev + k.c, B, k.c, ts.c / 8,
                                    td.c / 8, k.dst2 >= 0 ? plan->tensors[k.dst2].c / 8 : 0, ts.h, ts.w, k.eps);
       CUDA_TRY(cudaGetLastError());
@@ -614,7 +604,7 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const int B = tq.mult * plan->chunk, N = tq.h * tq.w, NK = tk.h * tk.w, D = k.c / k.heads;
       const dim3 grid((N + 255) / 256, k.heads, B);                       // two queries per thread
       const bool use_mma = NK == 64 && env_int("STCD_ATTN_MMA", 1);        // every stage of the 256 x 256 configurations
-      if (k.split)                                                          // split precision: tensor-core kernel only (NK == 64)
+      if (plan->split)                                                     // split precision: tensor-core kernel only (NK == 64)
         (D == 64 ? stcd::sr_attention_mma_kernel<64, true> : stcd::sr_attention_mma_kernel<80, true>)<<<dim3((N + 63) / 64, k.heads, B), 128, 0, st>>>(
             (const __nv_bfloat16*)tq.ptr, (const __nv_bfloat16*)tk.ptr, (__nv_bfloat16*)td.ptr, k.c, tq.c / 8, tk.c / 8, td.c / 8, N, k.scale);
       else if (use_mma && D == 64)
@@ -639,7 +629,7 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const int items = ((ts.w + 3) / 4) * ts.h;                        // one thread per 4 horizontally adjacent pixels
       const dim3 grid((unsigned)std::max(1, (items + 127) / 128), (unsigned)(k.c / 8), (unsigned)B);
       (void)hwp;
-      auto kern = k.split ? stcd::dwconv3x3_kernel<true> : stcd::dwconv3x3_kernel<false>;
+      auto kern = plan->split ? stcd::dwconv3x3_kernel<true> : stcd::dwconv3x3_kernel<false>;
       kern<<<grid, 128, 0, st>>>((const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, k.wb_dev, k.wb_dev + (size_t)k.c * 9, B, k.c / 8,
                                  ts.c / 8, td.c / 8, ts.h, ts.w, k.gelu);
       CUDA_TRY(cudaGetLastError());
@@ -649,7 +639,7 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       const Tensor& td = plan->tensors[k.dst];
       const int B = ts.mult * plan->chunk;
       const size_t total = (size_t)B * (k.c / 8) * td.h * td.w;
-      auto kern = k.split ? stcd::bilinear_up_kernel<true> : stcd::bilinear_up_kernel<false>;
+      auto kern = plan->split ? stcd::bilinear_up_kernel<true> : stcd::bilinear_up_kernel<false>;
       kern<<<(unsigned)std::max<size_t>(1, std::min<size_t>((total + 255) / 256, 148 * 16)), 256, 0, st>>>(
           (const __nv_bfloat16*)ts.ptr, (__nv_bfloat16*)td.ptr, B, k.c / 8, ts.c / 8, td.c / 8, ts.h, ts.w, k.scale);
       CUDA_TRY(cudaGetLastError());
@@ -705,7 +695,7 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
       } else if (k.s2d) {
         __nv_bfloat16* dp = (__nv_bfloat16*)t.ptr;
 #define STCD_PACK_S2D(CIN)                                                                                                   \
-  (k.split ? stcd::input_pack_s2d_kernel<CIN, true> : stcd::input_pack_s2d_kernel<CIN, false>)<<<blocks, 256, 0, st>>>( \
+  (plan->split ? stcd::input_pack_s2d_kernel<CIN, true> : stcd::input_pack_s2d_kernel<CIN, false>)<<<blocks, 256, 0, st>>>( \
       x1, x2, dp, plan->chunk, n_valid, t.h, t.w)
         switch (k.cin) {
           case 1: STCD_PACK_S2D(1); break;
@@ -714,7 +704,7 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
           default: STCD_PACK_S2D(4); break;
         }
 #undef STCD_PACK_S2D
-      } else if (!k.split && k.cin <= 4 && hw % 4 == 0 && (reinterpret_cast<uintptr_t>(x1) | reinterpret_cast<uintptr_t>(x2)) % 16 == 0) {
+      } else if (!plan->split && k.cin <= 4 && hw % 4 == 0 && (reinterpret_cast<uintptr_t>(x1) | reinterpret_cast<uintptr_t>(x2)) % 16 == 0) {
         __nv_bfloat16* dp = (__nv_bfloat16*)t.ptr;
         const int blocks4 = (int)std::min<size_t>((total / 4 + 255) / 256, 148 * 8);
         switch (k.cin) {
@@ -724,7 +714,7 @@ int run_chunk(stcd_plan* plan, const void* x1v, const void* x2v, int n_valid, fl
           default: stcd::input_pack4_kernel<4><<<blocks4, 256, 0, st>>>(x1, x2, dp, plan->chunk, n_valid, t.c / 8, hw); break;
         }
       } else
-        stcd::input_pack_kernel<<<blocks, 256, 0, st>>>(x1, x2, (__nv_bfloat16*)t.ptr, plan->chunk, n_valid, k.cin, t.c / 8, hw, k.split);
+        stcd::input_pack_kernel<<<blocks, 256, 0, st>>>(x1, x2, (__nv_bfloat16*)t.ptr, plan->chunk, n_valid, k.cin, t.c / 8, hw, plan->split);
       CUDA_TRY(cudaGetLastError());
     }
     ++op_i;
@@ -778,10 +768,12 @@ int stcd_device_count(void) {
   return ok;
 }
 
-int stcd_plan_create(int device, int chunk_pairs, stcd_plan** out) {
+int stcd_plan_create(int device, int chunk_pairs, int precision, stcd_plan** out) {
   if (!out) return fail(STCD_ERR_INVALID, "out is NULL");
   *out = nullptr;
   if (chunk_pairs < 1 || chunk_pairs > 4096) return fail(STCD_ERR_INVALID, "chunk_pairs %d out of range", chunk_pairs);
+  if (precision != STCD_PRECISION_BF16 && precision != STCD_PRECISION_SPLIT)
+    return fail(STCD_ERR_INVALID, "precision %d is neither STCD_PRECISION_BF16 (0) nor STCD_PRECISION_SPLIT (1)", precision);
   if (device != -1) {          // device -1: a validation plan (descriptors are checked and recorded, finalize refuses)
     int r = check_sm100(device);
     if (r) return r;
@@ -789,6 +781,7 @@ int stcd_plan_create(int device, int chunk_pairs, stcd_plan** out) {
   stcd_plan* p = new stcd_plan();
   p->device = device;
   p->chunk = chunk_pairs;
+  p->split = precision == STCD_PRECISION_SPLIT;
   *out = p;
   return STCD_OK;
 }
@@ -877,6 +870,8 @@ int stcd_plan_add_tensor(stcd_plan* plan, int img_mult, int h, int w, int c, int
   if (img_mult < 1 || img_mult > 2 || h < 1 || w < 1 || c < 8 || (c % 8) != 0 || dtype != STCD_BF16)
     return -fail(STCD_ERR_INVALID, "bad tensor decl mult=%d h=%d w=%d c=%d dtype=%d (c must be a multiple of 8, bf16)",
                  img_mult, h, w, c, dtype);
+  if (plan->split && (c % 16))
+    return -fail(STCD_ERR_INVALID, "split plan: tensor channels %d not a multiple of 16 (a hi and a lo plane of 8-channel groups)", c);
   Tensor t;
   t.mult = img_mult;
   t.h = h;
@@ -893,6 +888,9 @@ int stcd_plan_add_input_pack(stcd_plan* plan, int dst_tensor, int cin) {
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad dst tensor %d", dst_tensor);
   const Tensor& t = plan->tensors[dst_tensor];
+  if (plan->split && (t.mult != 2 || t.c != 16 || cin < 1 || cin > 8))
+    return -fail(STCD_ERR_INVALID, "split input pack needs a [2*chunk][2][h][w][8] tensor (hi plane, lo plane) and cin <= 8 (got mult=%d c=%d cin=%d)",
+                 t.mult, t.c, cin);
   if (t.mult != 2 || (t.c != 8 && t.c != 16) || cin < 1 || cin > t.c)
     return -fail(STCD_ERR_INVALID, "input pack needs a [2*chunk][1 or 2][h][w][8] tensor and cin <= its channels (got mult=%d c=%d cin=%d)",
                  t.mult, t.c, cin);
@@ -904,37 +902,18 @@ int stcd_plan_add_input_pack(stcd_plan* plan, int dst_tensor, int cin) {
   return (int)plan->ops.size() - 1;
 }
 
-int stcd_plan_add_input_pack_split(stcd_plan* plan, int dst_tensor, int cin) {
+int stcd_plan_add_input_pack_s2d(stcd_plan* plan, int dst_tensor, int cin) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad dst tensor %d", dst_tensor);
   const Tensor& t = plan->tensors[dst_tensor];
-  if (t.mult != 2 || t.c != 16 || cin < 1 || cin > 8)
-    return -fail(STCD_ERR_INVALID, "split input pack needs a [2*chunk][2][h][w][8] tensor (hi plane, lo plane) and cin <= 8 (got mult=%d c=%d cin=%d)",
-                 t.mult, t.c, cin);
-  PackOp k{dst_tensor, cin};
-  k.split = 1;
-  plan->packs.push_back(k);
-  plan->ops.push_back({1, (int)plan->packs.size() - 1});
-  plan->in_c = cin;
-  plan->in_h = t.h;
-  plan->in_w = t.w;
-  return (int)plan->ops.size() - 1;
-}
-
-static int add_input_pack_s2d(stcd_plan* plan, int dst_tensor, int cin, int split) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
-  if (!valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad dst tensor %d", dst_tensor);
-  const Tensor& t = plan->tensors[dst_tensor];
-  if (t.mult != 2 || t.c != (split ? 32 : 16) || cin < 1 || cin > 4)
+  if (t.mult != 2 || t.c != (plan->split ? 32 : 16) || cin < 1 || cin > 4)
     return -fail(STCD_ERR_INVALID, "space-to-depth input pack needs a [2*chunk][%d][h][w][8] tensor and cin <= 4 (got mult=%d c=%d cin=%d)",
-                 split ? 4 : 2, t.mult, t.c, cin);
+                 plan->split ? 4 : 2, t.mult, t.c, cin);
   PackOp k;
   k.dst = dst_tensor;
   k.cin = cin;
   k.s2d = 1;
-  k.split = split;
   plan->packs.push_back(k);
   plan->ops.push_back({1, (int)plan->packs.size() - 1});
   plan->in_c = cin;
@@ -943,10 +922,14 @@ static int add_input_pack_s2d(stcd_plan* plan, int dst_tensor, int cin, int spli
   return (int)plan->ops.size() - 1;
 }
 
-int stcd_plan_add_input_pack_s2d(stcd_plan* plan, int dst_tensor, int cin) { return add_input_pack_s2d(plan, dst_tensor, cin, 0); }
+// entry points of ops that have no split form start with this: a split plan refuses them
+static int refuse_split(const stcd_plan* plan, const char* op) {
+  return plan && plan->split ? -fail(STCD_ERR_INVALID, "%s has no split form (split plan)", op) : 0;
+}
 
 int stcd_plan_add_input_pack_u8(stcd_plan* plan, int dst_tensor, int cin, int s2d, const float* mean, const float* std_) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (int r = refuse_split(plan, "uint8 input pack")) return r;
   if (!mean || !std_) return -fail(STCD_ERR_INVALID, "mean/std are NULL");
   if (cin < 1 || cin > 4) return -fail(STCD_ERR_INVALID, "uint8 input pack: cin %d not in [1, 4]", cin);
   for (int c = 0; c < cin; ++c)
@@ -963,28 +946,36 @@ int stcd_plan_add_input_pack_u8(stcd_plan* plan, int dst_tensor, int cin, int s2
   return r;
 }
 
-static int add_maxpool_s2d(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int split) {
+// split plan: each tensor (ids >= 0, already validated) stores an op's c logical channels twice over, the hi plane first and the
+// lo plane at half its stored channels
+static int check_split_planes(const stcd_plan* plan, const char* op, std::initializer_list<int> tensor_ids, int c) {
+  if (!plan->split) return 0;
+  for (int id : tensor_ids)
+    if (id >= 0 && plan->tensors[id].c < 2 * c)
+      return -fail(STCD_ERR_INVALID, "split %s: tensor %d stores %d channels, not the 2 x %d of a hi and a lo plane", op, id,
+                   plan->tensors[id].c, c);
+  return 0;
+}
+
+int stcd_plan_add_maxpool_s2d(stcd_plan* plan, int src_tensor, int dst_tensor, int c) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad tensor id");
+  if (int r = check_split_planes(plan, "max-pool", {dst_tensor}, c)) return r;
   const Tensor& ts = plan->tensors[src_tensor];
   const Tensor& td = plan->tensors[dst_tensor];
-  if (c < 8 || (c % 8) || ts.c != (split ? 8 : 4) * c || td.c < (split ? 2 : 1) * c || ts.h != td.h || ts.w != td.w || ts.mult != td.mult)
+  // split plan: src stores 8c (4 parity classes x 2 planes)
+  if (c < 8 || (c % 8) || ts.c != (plan->split ? 8 : 4) * c || td.c < c || ts.h != td.h || ts.w != td.w || ts.mult != td.mult)
     return -fail(STCD_ERR_INVALID, "max-pool: src [%d*chunk,%d,%d,%d] must be the space-to-depth form of dst [%d*chunk,%d,%d,%d] (c=%d)",
                  ts.mult, ts.h, ts.w, ts.c, td.mult, td.h, td.w, td.c, c);
-  PoolOp k{src_tensor, dst_tensor, c};
-  k.split = split;
-  plan->pools.push_back(k);
+  plan->pools.push_back({src_tensor, dst_tensor, c});
   plan->ops.push_back({3, (int)plan->pools.size() - 1});
   return (int)plan->ops.size() - 1;
 }
 
-int stcd_plan_add_maxpool_s2d(stcd_plan* plan, int src_tensor, int dst_tensor, int c) {
-  return add_maxpool_s2d(plan, src_tensor, dst_tensor, c, 0);
-}
-
 int stcd_plan_add_graph_conv(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int k, int dilation, int r, const float* relpos) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (int e = refuse_split(plan, "graph conv")) return e;
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad tensor id");
   const Tensor& ts = plan->tensors[src_tensor];
@@ -1008,22 +999,23 @@ int stcd_plan_add_graph_conv(stcd_plan* plan, int src_tensor, int dst_tensor, in
   return (int)plan->ops.size() - 1;
 }
 
-static int add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d, int c, const float* gamma, const float* beta,
-                         float eps, int split) {
+int stcd_plan_add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d, int c, const float* gamma, const float* beta,
+                            float eps) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor) || (dst_s2d >= 0 && !valid_tensor(plan, dst_s2d)) || !gamma || !beta)
     return -fail(STCD_ERR_INVALID, "layer norm: bad tensor id / NULL gamma, beta");
+  if (int r = check_split_planes(plan, "layer norm", {src_tensor, dst_tensor}, c)) return r;
   const Tensor& ts = plan->tensors[src_tensor];
   const Tensor& td = plan->tensors[dst_tensor];
   if (c < 8 || (c % 8) || ts.c < c || td.c < c || ts.h != td.h || ts.w != td.w || ts.mult != td.mult || !(eps > 0.f))
     return -fail(STCD_ERR_INVALID, "layer norm: src [%d*chunk,%d,%d,%d] / dst [%d*chunk,%d,%d,%d] must match and hold c=%d channels", ts.mult,
                  ts.h, ts.w, ts.c, td.mult, td.h, td.w, td.c, c);
-  if (dst_s2d >= 0) {
+  if (dst_s2d >= 0) {      // split plan: 8c (4 parity classes x 2 planes)
     const Tensor& t2 = plan->tensors[dst_s2d];
-    if ((ts.h % 2) || (ts.w % 2) || t2.h != ts.h / 2 || t2.w != ts.w / 2 || t2.c != (split ? 8 : 4) * c || t2.mult != ts.mult)
+    if ((ts.h % 2) || (ts.w % 2) || t2.h != ts.h / 2 || t2.w != ts.w / 2 || t2.c != (plan->split ? 8 : 4) * c || t2.mult != ts.mult)
       return -fail(STCD_ERR_INVALID, "layer norm: space-to-depth copy must be [%d*chunk,%d,%d,%d]", ts.mult, ts.h / 2, ts.w / 2,
-                   (split ? 8 : 4) * c);
+                   (plan->split ? 8 : 4) * c);
   }
   LayerNormOp k;
   k.src = src_tensor;
@@ -1033,15 +1025,9 @@ static int add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int ds
   k.eps = eps;
   k.gb.assign(gamma, gamma + c);
   k.gb.insert(k.gb.end(), beta, beta + c);
-  k.split = split;
   plan->lns.push_back(std::move(k));
   plan->ops.push_back({7, (int)plan->lns.size() - 1});
   return (int)plan->ops.size() - 1;
-}
-
-int stcd_plan_add_layernorm(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d, int c, const float* gamma, const float* beta,
-                            float eps) {
-  return add_layernorm(plan, src_tensor, dst_tensor, dst_s2d, c, gamma, beta, eps, 0);
 }
 
 int stcd_plan_add_sr_attention(stcd_plan* plan, int q_tensor, int kv_tensor, int dst_tensor, int c, int heads, float scale) {
@@ -1053,8 +1039,12 @@ int stcd_plan_add_sr_attention(stcd_plan* plan, int q_tensor, int kv_tensor, int
   const Tensor& td = plan->tensors[dst_tensor];
   if (heads < 1 || c < 8 || (c % heads) || ((c / heads) != 64 && (c / heads) != 80))
     return -fail(STCD_ERR_INVALID, "attention: c=%d heads=%d: head dim must be 64 or 80", c, heads);
-  if (tq.c != c || td.c != c || tk.c != 2 * c || tq.h != td.h || tq.w != td.w || tq.mult != td.mult || tq.mult != tk.mult)
-    return -fail(STCD_ERR_INVALID, "attention: q/dst must be [m*chunk,h,w,%d] and kv [m*chunk,hk,wk,%d]", c, 2 * c);
+  const int cs = plan->split ? 2 * c : c;        // stored channels of q and dst (split plan: hi and lo planes)
+  if (tq.c != cs || td.c != cs || tk.c != 2 * cs || tq.h != td.h || tq.w != td.w || tq.mult != td.mult || tq.mult != tk.mult)
+    return -fail(STCD_ERR_INVALID, "attention: q/dst must be [m*chunk,h,w,%d] and kv [m*chunk,hk,wk,%d]%s", cs, 2 * cs,
+                 plan->split ? " (hi and lo planes)" : "");
+  if (plan->split && tk.h * tk.w != 64)
+    return -fail(STCD_ERR_INVALID, "split attention: %d keys (the tensor-core kernel takes exactly 64)", tk.h * tk.w);
   if (tk.h * tk.w > stcd::kAttnMaxKeys) return -fail(STCD_ERR_INVALID, "attention: %d keys (max %d)", tk.h * tk.w, stcd::kAttnMaxKeys);
   plan->attns.push_back({q_tensor, kv_tensor, dst_tensor, c, heads, scale});
   plan->ops.push_back({8, (int)plan->attns.size() - 1});
@@ -1065,6 +1055,7 @@ int stcd_plan_add_dwconv3x3(stcd_plan* plan, int src_tensor, int dst_tensor, int
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor) || !weight || !bias) return -fail(STCD_ERR_INVALID, "dw conv: bad tensor id / NULL weights");
+  if (int r = check_split_planes(plan, "dw conv", {src_tensor, dst_tensor}, c)) return r;
   const Tensor& ts = plan->tensors[src_tensor];
   const Tensor& td = plan->tensors[dst_tensor];
   if (c < 8 || (c % 8) || ts.c < c || td.c < c || ts.h != td.h || ts.w != td.w || ts.mult != td.mult)
@@ -1086,6 +1077,7 @@ int stcd_plan_add_bilinear_up(stcd_plan* plan, int src_tensor, int dst_tensor, i
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad tensor id");
+  if (int r = check_split_planes(plan, "bilinear up", {src_tensor, dst_tensor}, c)) return r;
   const Tensor& ts = plan->tensors[src_tensor];
   const Tensor& td = plan->tensors[dst_tensor];
   if (c < 8 || (c % 8) || ts.c < c || td.c < c || scale < 1 || scale > 32 || td.h != ts.h * scale || td.w != ts.w * scale || ts.mult != td.mult)
@@ -1094,61 +1086,6 @@ int stcd_plan_add_bilinear_up(stcd_plan* plan, int src_tensor, int dst_tensor, i
   plan->bilinears.push_back({src_tensor, dst_tensor, c, scale});
   plan->ops.push_back({6, (int)plan->bilinears.size() - 1});
   return (int)plan->ops.size() - 1;
-}
-
-// ---- split precision (lowering.Program.precision "split"): the same ops on tensors that hold a hi and a lo plane.  Every
-// tensor must store its logical channels twice over (hi plane first, lo plane at half the stored channels), in multiples of 16.
-static bool split_planes(const Tensor& t, int c) { return t.c % 16 == 0 && t.c / 2 >= c; }
-
-int stcd_plan_add_layernorm_split(stcd_plan* plan, int src_tensor, int dst_tensor, int dst_s2d, int c, const float* gamma,
-                                  const float* beta, float eps) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  if (valid_tensor(plan, src_tensor) && valid_tensor(plan, dst_tensor) &&
-      (!split_planes(plan->tensors[src_tensor], c) || !split_planes(plan->tensors[dst_tensor], c)))
-    return -fail(STCD_ERR_INVALID, "split layer norm: src / dst must store 2 x %d channels in multiples of 16 (got %d, %d)", c,
-                 plan->tensors[src_tensor].c, plan->tensors[dst_tensor].c);
-  return add_layernorm(plan, src_tensor, dst_tensor, dst_s2d, c, gamma, beta, eps, 1);     // space-to-depth copy: 8c (4 classes x 2 planes)
-}
-
-int stcd_plan_add_sr_attention_split(stcd_plan* plan, int q_tensor, int kv_tensor, int dst_tensor, int c, int heads, float scale) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
-  if (!valid_tensor(plan, q_tensor) || !valid_tensor(plan, kv_tensor) || !valid_tensor(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "bad tensor id");
-  const Tensor& tq = plan->tensors[q_tensor];
-  const Tensor& tk = plan->tensors[kv_tensor];
-  const Tensor& td = plan->tensors[dst_tensor];
-  if (heads < 1 || c < 8 || (c % heads) || ((c / heads) != 64 && (c / heads) != 80))
-    return -fail(STCD_ERR_INVALID, "split attention: c=%d heads=%d: head dim must be 64 or 80", c, heads);
-  if (tq.c != 2 * c || td.c != 2 * c || tk.c != 4 * c || tq.h != td.h || tq.w != td.w || tq.mult != td.mult || tq.mult != tk.mult)
-    return -fail(STCD_ERR_INVALID, "split attention: q/dst must be [m*chunk,h,w,2 x %d] and kv [m*chunk,hk,wk,2 x %d] (hi and lo planes)", c, 2 * c);
-  if (tk.h * tk.w != 64) return -fail(STCD_ERR_INVALID, "split attention: %d keys (the tensor-core kernel takes exactly 64)", tk.h * tk.w);
-  AttentionOp k{q_tensor, kv_tensor, dst_tensor, c, heads, scale};
-  k.split = 1;
-  plan->attns.push_back(k);
-  plan->ops.push_back({8, (int)plan->attns.size() - 1});
-  return (int)plan->ops.size() - 1;
-}
-
-int stcd_plan_add_dwconv3x3_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, const float* weight, const float* bias, int gelu) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  if (valid_tensor(plan, src_tensor) && valid_tensor(plan, dst_tensor) &&
-      (!split_planes(plan->tensors[src_tensor], c) || !split_planes(plan->tensors[dst_tensor], c)))
-    return -fail(STCD_ERR_INVALID, "split dw conv: src / dst must store 2 x %d channels in multiples of 16 (got %d, %d)", c,
-                 plan->tensors[src_tensor].c, plan->tensors[dst_tensor].c);
-  const int r = stcd_plan_add_dwconv3x3(plan, src_tensor, dst_tensor, c, weight, bias, gelu);
-  if (r >= 0) plan->dws.back().split = 1;
-  return r;
-}
-
-int stcd_plan_add_bilinear_up_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int scale) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  if (valid_tensor(plan, src_tensor) && valid_tensor(plan, dst_tensor) &&
-      (!split_planes(plan->tensors[src_tensor], c) || !split_planes(plan->tensors[dst_tensor], c)))
-    return -fail(STCD_ERR_INVALID, "split bilinear up: src / dst must store 2 x %d channels in multiples of 16 (got %d, %d)", c,
-                 plan->tensors[src_tensor].c, plan->tensors[dst_tensor].c);
-  const int r = stcd_plan_add_bilinear_up(plan, src_tensor, dst_tensor, c, scale);
-  if (r >= 0) plan->bilinears.back().split = 1;
-  return r;
 }
 
 int stcd_plan_add_absdiff(stcd_plan* plan, int src_tensor, int dst_tensor) {
@@ -1179,13 +1116,14 @@ int stcd_plan_add_subdiff(stcd_plan* plan, int src_tensor, int add, int dst_tens
   return r;
 }
 
-static int add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst_tensor, int dst_s2d, int c, int hid, const float* w1,
-                            const float* w2, const float* ws, int mode, int split) {
+int stcd_plan_add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst_tensor, int dst_s2d, int c, int hid, const float* w1,
+                               const float* w2, const float* ws, int mode) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor) || (res >= 0 && !valid_tensor(plan, res)) ||
       (dst_s2d >= 0 && !valid_tensor(plan, dst_s2d)) || !w1 || !w2 || (mode == 1 && !ws) || mode < 0 || mode > 1)
     return -fail(STCD_ERR_INVALID, "channel gate: bad tensor id / NULL weights / mode");
+  if (int r = check_split_planes(plan, "channel gate", {src_tensor, res, dst_tensor}, c)) return r;
   const Tensor& ts = plan->tensors[src_tensor];
   const Tensor& td = plan->tensors[dst_tensor];
   if (c < 8 || (c % 8) || c > stcd::kGateMaxC || hid < 1 || hid > stcd::kGateMaxH || ts.c < c || td.c < c || ts.h != td.h || ts.w != td.w ||
@@ -1195,11 +1133,11 @@ static int add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst_te
     const Tensor& tr = plan->tensors[res];
     if (tr.h != ts.h || tr.w != ts.w || tr.c < c || tr.mult != ts.mult) return -fail(STCD_ERR_INVALID, "channel gate: residual shape");
   }
-  if (dst_s2d >= 0) {
+  if (dst_s2d >= 0) {      // split plan: 8c (4 parity classes x 2 planes)
     const Tensor& t2 = plan->tensors[dst_s2d];
-    if ((ts.h % 2) || (ts.w % 2) || t2.h != ts.h / 2 || t2.w != ts.w / 2 || t2.c != (split ? 8 : 4) * c || t2.mult != ts.mult)
+    if ((ts.h % 2) || (ts.w % 2) || t2.h != ts.h / 2 || t2.w != ts.w / 2 || t2.c != (plan->split ? 8 : 4) * c || t2.mult != ts.mult)
       return -fail(STCD_ERR_INVALID, "channel gate: space-to-depth copy must be [%d*chunk,%d,%d,%d]", ts.mult, ts.h / 2, ts.w / 2,
-                   (split ? 8 : 4) * c);
+                   (plan->split ? 8 : 4) * c);
   }
   GateOp k;
   k.src = src_tensor;
@@ -1213,18 +1151,12 @@ static int add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst_te
   k.w.assign(w1, w1 + (size_t)hid * c);
   k.w.insert(k.w.end(), w2, w2 + (size_t)c * hid);
   if (mode == 1) k.w.insert(k.w.end(), ws, ws + c);
-  k.split = split;
   plan->gates.push_back(std::move(k));
   plan->ops.push_back({11, (int)plan->gates.size() - 1});
   return (int)plan->ops.size() - 1;
 }
 
-int stcd_plan_add_channel_gate(stcd_plan* plan, int src_tensor, int res, int dst_tensor, int dst_s2d, int c, int hid, const float* w1,
-                               const float* w2, const float* ws, int mode) {
-  return add_channel_gate(plan, src_tensor, res, dst_tensor, dst_s2d, c, hid, w1, w2, ws, mode, 0);
-}
-
-static int add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* d, int split) {
+int stcd_plan_add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* d) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!d || !valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor) || !d->conv_a || !d->pos || !d->enc || !d->dec)
@@ -1237,7 +1169,7 @@ static int add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tensor, 
     return -fail(STCD_ERR_INVALID, "BIT transformer: depths %d/%d, inner dims %d/%d out of range", d->n_enc, d->n_dec, d->inner_enc, d->inner_dec);
   const Tensor& ts = plan->tensors[src_tensor];
   const Tensor& td = plan->tensors[dst_tensor];
-  const int cs = (split ? 2 : 1) * stcd::kBitC;      // stored channels (split: hi and lo planes)
+  const int cs = (plan->split ? 2 : 1) * stcd::kBitC;      // stored channels (split plan: hi and lo planes)
   if (ts.mult != 2 || td.mult != 2 || ts.c != cs || td.c != cs || ts.h != td.h || ts.w != td.w)
     return -fail(STCD_ERR_INVALID, "BIT transformer: src and dst must be [2*chunk,h,w,%d] (both streams)", cs);
   BitOp k;
@@ -1251,19 +1183,15 @@ static int add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tensor, 
   k.d.conv_a = k.d.pos = k.d.enc = k.d.dec = nullptr;
   k.mixer_smem = sizeof(float) * (size_t)(8 * 3 * d->inner_enc);
   k.coef_smem = sizeof(float) * (size_t)(2 * 8 * d->inner_dec);
-  k.split = split;
   plan->bits.push_back(std::move(k));
   plan->ops.push_back({13, (int)plan->bits.size() - 1});
   return (int)plan->ops.size() - 1;
 }
 
-int stcd_plan_add_bit_transformer(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* d) {
-  return add_bit_transformer(plan, src_tensor, dst_tensor, d, 0);
-}
-
 int stcd_plan_add_channel_attention(stcd_plan* plan, const int* src_tensors, const int* src_streams, const int* src_c, int n_src,
                                     int dst_tensor, int hid, const float* fc1, const float* fc2) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (int r = refuse_split(plan, "channel attention")) return r;
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!src_tensors || !src_streams || !src_c || n_src < 1 || n_src > 4 || !valid_tensor(plan, dst_tensor) || !fc1 || !fc2 || hid < 1 ||
       hid > stcd::kCaMaxH)
@@ -1299,6 +1227,7 @@ int stcd_plan_add_channel_attention(stcd_plan* plan, const int* src_tensors, con
 
 int stcd_plan_add_spatial_gate(stcd_plan* plan, int src_tensor, int dst_tensor, int c, const float* w, const float* scale, const float* shift) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (int r = refuse_split(plan, "spatial gate")) return r;
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor) || !w || !scale || !shift)
     return -fail(STCD_ERR_INVALID, "spatial gate: bad tensor id / NULL weights");
@@ -1320,6 +1249,7 @@ int stcd_plan_add_spatial_gate(stcd_plan* plan, int src_tensor, int dst_tensor, 
 
 int stcd_plan_add_global_local_gate(stcd_plan* plan, int src_tensor, int dst_tensor, int c, const float* prm) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (int r = refuse_split(plan, "global-local gate")) return r;
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, src_tensor) || !valid_tensor(plan, dst_tensor) || !prm) return -fail(STCD_ERR_INVALID, "global-local gate: bad tensor id / NULL weights");
   const Tensor& ts = plan->tensors[src_tensor];
@@ -1338,6 +1268,7 @@ int stcd_plan_add_global_local_gate(stcd_plan* plan, int src_tensor, int dst_ten
 }
 
 int stcd_plan_add_csam_gate(stcd_plan* plan, int src_tensor, int dst_tensor, int c, int hid, const float* prm) {
+  if (int r = refuse_split(plan, "csam gate")) return r;
   if (hid < 1 || hid > stcd::kGlMaxC / 4) return -fail(STCD_ERR_INVALID, "csam gate: hid=%d (1..%d)", hid, stcd::kGlMaxC / 4);
   const int r = stcd_plan_add_global_local_gate(plan, src_tensor, dst_tensor, c, prm);   // same tensors and checks; weights replaced below
   if (r < 0) return r;
@@ -1349,6 +1280,7 @@ int stcd_plan_add_csam_gate(stcd_plan* plan, int src_tensor, int dst_tensor, int
 
 int stcd_plan_add_vffm(stcd_plan* plan, int low, int high, int mixed, int local, int dst, int c, int inter, const float* prm) {
   if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
+  if (int r = refuse_split(plan, "VFFM")) return r;
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   const int ids[5] = {low, high, mixed, local, dst};
   for (int id : ids)
@@ -1389,62 +1321,9 @@ int stcd_plan_add_sum(stcd_plan* plan, const int* src_tensors, int n, int dst_te
   return (int)plan->ops.size() - 1;
 }
 
-// ---- split precision forms of the ResNet-family ops (stem pack and max-pool, feature differences, sums, SE gates, BIT's token
-// path).  Like the ones above, they reject tensors that do not store twice their logical channels in multiples of 16.
-int stcd_plan_add_input_pack_s2d_split(stcd_plan* plan, int dst_tensor, int cin) { return add_input_pack_s2d(plan, dst_tensor, cin, 1); }
-
-int stcd_plan_add_maxpool_s2d_split(stcd_plan* plan, int src_tensor, int dst_tensor, int c) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  if (valid_tensor(plan, dst_tensor) && !split_planes(plan->tensors[dst_tensor], c))
-    return -fail(STCD_ERR_INVALID, "split max-pool: dst must store 2 x %d channels in multiples of 16 (got %d)", c, plan->tensors[dst_tensor].c);
-  return add_maxpool_s2d(plan, src_tensor, dst_tensor, c, 1);      // src: 8c (4 classes x 2 planes)
-}
-
-// elementwise ops without a logical channel count: every tensor must hold two planes of a multiple of 8 channels
-static bool split_even(stcd_plan* plan, int t) { return !valid_tensor(plan, t) || plan->tensors[t].c % 16 == 0; }
-
-int stcd_plan_add_absdiff_split(stcd_plan* plan, int src_tensor, int dst_tensor) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  if (!split_even(plan, src_tensor) || !split_even(plan, dst_tensor))
-    return -fail(STCD_ERR_INVALID, "split abs-diff: src / dst must store hi and lo planes (channels a multiple of 16)");
-  const int r = stcd_plan_add_absdiff(plan, src_tensor, dst_tensor);
-  if (r >= 0) plan->absdiffs.back().split = 1;
-  return r;
-}
-
-int stcd_plan_add_subdiff_split(stcd_plan* plan, int src_tensor, int add, int dst_tensor) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  if (!split_even(plan, src_tensor) || !split_even(plan, dst_tensor) || (add >= 0 && !split_even(plan, add)))
-    return -fail(STCD_ERR_INVALID, "split signed diff: src / addend / dst must store hi and lo planes (channels a multiple of 16)");
-  const int r = stcd_plan_add_subdiff(plan, src_tensor, add, dst_tensor);
-  if (r >= 0) plan->absdiffs.back().split = 1;
-  return r;
-}
-
-int stcd_plan_add_sum_split(stcd_plan* plan, const int* src_tensors, int n, int dst_tensor) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  if (!split_even(plan, dst_tensor)) return -fail(STCD_ERR_INVALID, "split sum: dst must store hi and lo planes (channels a multiple of 16)");
-  const int r = stcd_plan_add_sum(plan, src_tensors, n, dst_tensor);     // sources: the destination's shape
-  if (r >= 0) plan->sums.back().split = 1;
-  return r;
-}
-
-int stcd_plan_add_channel_gate_split(stcd_plan* plan, int src_tensor, int res, int dst_tensor, int dst_s2d, int c, int hid, const float* w1,
-                                     const float* w2, const float* ws, int mode) {
-  if (!plan) return -fail(STCD_ERR_STATE, "plan is NULL");
-  for (int t : {src_tensor, dst_tensor, res})
-    if (valid_tensor(plan, t) && !split_planes(plan->tensors[t], c))
-      return -fail(STCD_ERR_INVALID, "split channel gate: src / res / dst must store 2 x %d channels in multiples of 16 (tensor %d has %d)", c,
-                   t, plan->tensors[t].c);
-  return add_channel_gate(plan, src_tensor, res, dst_tensor, dst_s2d, c, hid, w1, w2, ws, mode, 1);    // space-to-depth copy: 8c
-}
-
-int stcd_plan_add_bit_transformer_split(stcd_plan* plan, int src_tensor, int dst_tensor, const stcd_bit_desc* d) {
-  return add_bit_transformer(plan, src_tensor, dst_tensor, d, 1);
-}
-
 int stcd_plan_add_seg_head(stcd_plan* plan, const stcd_seghead_desc* d) {
   if (!plan || !d) return -fail(STCD_ERR_STATE, "plan/desc is NULL");
+  if (int r = refuse_split(plan, "seg head")) return r;
   if (plan->finalized) return -fail(STCD_ERR_STATE, "plan already finalized");
   if (!valid_tensor(plan, d->src) || !d->weight || d->out_ext < 0) return -fail(STCD_ERR_INVALID, "seg head: bad src / NULL weight / out_ext");
   const Tensor& t = plan->tensors[d->src];
@@ -1493,7 +1372,7 @@ int stcd_plan_add_conv(stcd_plan* plan, const stcd_conv_desc* d) {
   if (2 * mt * d->n_tile > 512)
     return -fail(STCD_ERR_INVALID, "double-buffered accumulators need %d TMEM columns (> 512)", 2 * mt * d->n_tile);
   if (d->pair && (plan->chunk < 1)) return -fail(STCD_ERR_INVALID, "pair op on an empty chunk");
-  if (d->split && (d->fold_cs || d->xf_cs))
+  if (plan->split && (d->fold_cs || d->xf_cs))
     return -fail(STCD_ERR_INVALID, "split precision: no folded or horizontally folded stores");
   if (d->xf_cs) {
     bool ok = d->xf_cs >= 16 && d->xf_cs % 16 == 0 && d->n_tile == 3 * d->xf_cs && d->cout_pad == d->n_tile && d->cout <= d->xf_cs &&
@@ -1534,9 +1413,7 @@ int stcd_plan_add_conv(stcd_plan* plan, const stcd_conv_desc* d) {
     if (id < 0) return 0;
     if (!valid_tensor(plan, id)) return fail(STCD_ERR_INVALID, "bad %s tensor %d", name, id);
     const Tensor& t = plan->tensors[id];
-    if (d->split && (t.c % 16))
-      return fail(STCD_ERR_INVALID, "split precision: %s tensor %d needs a hi and a lo plane (channels %d not a multiple of 16)", name, id, t.c);
-    if (t.h != hh || t.w != ww || (d->split ? t.c / 2 : t.c) < coff + (d->fold_cs ? d->fold_cout : d->cout) || t.mult != mult)
+    if (t.h != hh || t.w != ww || (plan->split ? t.c / 2 : t.c) < coff + (d->fold_cs ? d->fold_cout : d->cout) || t.mult != mult)
       return fail(STCD_ERR_INVALID, "%s tensor %d is [%d*chunk,%d,%d,%d], op writes [%d*chunk,%d,%d,%d+%d]", name, id,
                   t.mult, t.h, t.w, t.c, mult, hh, ww, coff, d->cout);
     return 0;
@@ -1549,9 +1426,9 @@ int stcd_plan_add_conv(stcd_plan* plan, const stcd_conv_desc* d) {
       return -fail(STCD_ERR_INVALID, "space-to-depth out0 needs a tensor, even output dims and no channel offset");
     const Tensor& t = plan->tensors[d->out0];
     // split precision: hi of parity class k at k*cout, lo at 4*cout + k*cout
-    if (t.h != ho / 2 || t.w != wo / 2 || t.c != (d->split ? 8 : 4) * d->cout || t.mult != out_imgs)
+    if (t.h != ho / 2 || t.w != wo / 2 || t.c != (plan->split ? 8 : 4) * d->cout || t.mult != out_imgs)
       return -fail(STCD_ERR_INVALID, "space-to-depth out0 tensor is [%d*chunk,%d,%d,%d], op writes [%d*chunk,%d,%d,%d*%d]", t.mult, t.h, t.w,
-                   t.c, out_imgs, ho / 2, wo / 2, d->split ? 8 : 4, d->cout);
+                   t.c, out_imgs, ho / 2, wo / 2, plan->split ? 8 : 4, d->cout);
   } else if (check_out(d->out0, ho, wo, d->out0_coff, out_imgs, "out0")) return -STCD_ERR_INVALID;
   if (check_out(d->out_raw, ho, wo, 0, out_imgs, "out_raw")) return -STCD_ERR_INVALID;
   if (check_out(d->res, ho, wo, 0, out_imgs, "res")) return -STCD_ERR_INVALID;
@@ -1637,7 +1514,7 @@ int stcd_plan_add_ecam_head(stcd_plan* plan, const stcd_ecam_desc* d) {
   for (int k = 0; k < 4; ++k) {
     if (!valid_tensor(plan, d->src[k])) return -fail(STCD_ERR_INVALID, "ecam head: bad src tensor %d", d->src[k]);
     const Tensor& t = plan->tensors[d->src[k]];
-    if (t.mult != 1 || t.c != (d->split ? 2 : 1) * d->c || (k && (t.h != h || t.w != w)))
+    if (t.mult != 1 || t.c != (plan->split ? 2 : 1) * d->c || (k && (t.h != h || t.w != w)))
       return -fail(STCD_ERR_INVALID, "ecam head: src %d is [%d*chunk,%d,%d,%d], need [chunk,%d,%d,%d]", k, t.mult, t.h, t.w, t.c, h, w, d->c);
     h = t.h;
     w = t.w;
@@ -1926,8 +1803,8 @@ int stcd_plan_finalize(stcd_plan* plan) {
     // epilogue finishes together (slot <= 16 KB), up to kMaxRSlots blocks ahead, when >= 2 slots (32 KB when there is room)
     // fit beside >= 2 A stages; else the epilogue loads the residual itself
     p.res_slots = 0;
-    p.split = d.split ? 1 : 0;
-    if (d.res >= 0 && d.n_phase == 1 && d.osy == 1 && d.osx == 1 && !d.split && env_int("STCD_RES_SMEM", 1)) {
+    p.split = plan->split;
+    if (d.res >= 0 && d.n_phase == 1 && d.osy == 1 && d.osx == 1 && !plan->split && env_int("STCD_RES_SMEM", 1)) {
       const Tensor& tr = plan->tensors[d.res];
       const int ms = d.pair ? 2 : 1;
       p.res_ch = xf ? d.xf_cs : d.n_tile;
@@ -1988,7 +1865,7 @@ int stcd_plan_finalize(stcd_plan* plan) {
     op.threads = stcd::kConvThreads;
     // plans that run one CTA per SM anyway take the eight-epilogue-warp instance when there is one (>= 2 column steps to share)
     const bool want8 = !(tune_flags & 2) && occ == 1 && (xf ? (d.xf_cs >= 32 && env_int("STCD_XF_EPI8", 1) != 0) : d.n_tile >= 32) && env_int("STCD_EPI8", 1) != 0;
-    for (int i = 0; i < n_kernels && !force_generic && !d.split; ++i)     // split precision lives in the generic instances
+    for (int i = 0; i < n_kernels && !force_generic && !plan->split; ++i)     // split precision lives in the generic instances
       if (kernels[i].mt == op.mt && kernels[i].ms == (d.pair ? 2 : 1) && kernels[i].epi == op.epi && (kernels[i].ne == 4 || want8)) {
         if (op.fn && kernels[i].ne == 4) continue;       // an eight-warp instance found earlier wins
         op.fn = kernels[i].fn;
@@ -2196,7 +2073,7 @@ int stcd_plan_finalize(stcd_plan* plan) {
     memset(&q, 0, sizeof(q));
     for (int k = 0; k < 4; ++k) q.src[k] = (const __nv_bfloat16*)plan->tensors[d.src[k]].ptr;
     q.c = d.c;
-    q.split = d.split ? 1 : 0;
+    q.split = plan->split;
     q.hw = e.hw;
     q.n_img = plan->chunk;
     q.n_class = d.n_class;

@@ -36,7 +36,8 @@ class Plan:
         self.device = int(device)
         self.u8 = False                      # set by _build when the input op takes uint8 HWC images
         self._h = C.c_void_p()
-        _lib.check(self.lib.stcd_plan_create(self.device, self.chunk, C.byref(self._h)), "stcd_plan_create")
+        precision = _lib.PRECISION_SPLIT if prog.split else _lib.PRECISION_BF16
+        _lib.check(self.lib.stcd_plan_create(self.device, self.chunk, precision, C.byref(self._h)), "stcd_plan_create")
         try:
             self._build()
         except Exception:
@@ -51,7 +52,7 @@ class Plan:
             ids[name] = _lib.check_id(lib.stcd_plan_add_tensor(h, t.mult, t.h, t.w, t.c, 0), f"tensor {name}")
         self.tensor_ids = ids
         for op in prog.ops:
-            if isinstance(op, InputPackSpec) and op.u8_norm is not None and op.split:
+            if isinstance(op, InputPackSpec) and op.u8_norm is not None and prog.split:
                 raise NotImplementedError("split precision takes fp32 inputs (forward_uint8 is the bf16 path's loader fusion)")
             if isinstance(op, InputPackSpec) and op.u8_norm is not None:
                 mean = (C.c_float * op.cin)(*op.u8_norm[0][: op.cin])
@@ -60,10 +61,7 @@ class Plan:
                               f"uint8 input pack {op.name}")
                 self.u8 = True
             elif isinstance(op, InputPackSpec):
-                if op.s2d:
-                    add = lib.stcd_plan_add_input_pack_s2d_split if op.split else lib.stcd_plan_add_input_pack_s2d
-                else:
-                    add = lib.stcd_plan_add_input_pack_split if op.split else lib.stcd_plan_add_input_pack
+                add = lib.stcd_plan_add_input_pack_s2d if op.s2d else lib.stcd_plan_add_input_pack
                 _lib.check_id(add(h, ids[op.dst], op.cin), f"input pack {op.name}")
             elif isinstance(op, GraphConvSpec):
                 rp = None if op.relpos is None else np.ascontiguousarray(op.relpos, np.float32)
@@ -71,18 +69,16 @@ class Plan:
                               f"graph conv {op.name}")
             elif isinstance(op, AbsDiffSpec):
                 if op.signed:
-                    add = lib.stcd_plan_add_subdiff_split if op.split else lib.stcd_plan_add_subdiff
-                    r = add(h, ids[op.src], -1 if op.add is None else ids[op.add], ids[op.dst])
+                    r = lib.stcd_plan_add_subdiff(h, ids[op.src], -1 if op.add is None else ids[op.add], ids[op.dst])
                 else:
-                    add = lib.stcd_plan_add_absdiff_split if op.split else lib.stcd_plan_add_absdiff
-                    r = add(h, ids[op.src], ids[op.dst])
+                    r = lib.stcd_plan_add_absdiff(h, ids[op.src], ids[op.dst])
                 _lib.check_id(r, f"diff {op.name}")
             elif isinstance(op, ChannelGateSpec):
                 w1, w2 = np.ascontiguousarray(op.w1, np.float32), np.ascontiguousarray(op.w2, np.float32)
                 ws = None if op.ws is None else np.ascontiguousarray(op.ws, np.float32)
-                add = lib.stcd_plan_add_channel_gate_split if op.split else lib.stcd_plan_add_channel_gate
-                _lib.check_id(add(h, ids[op.src], -1 if op.res is None else ids[op.res], ids[op.dst], -1 if op.dst_s2d is None else ids[op.dst_s2d],
-                                  op.c, w1.shape[0], _fptr(w1), _fptr(w2), _fptr(ws), op.mode), f"channel gate {op.name}")
+                _lib.check_id(lib.stcd_plan_add_channel_gate(h, ids[op.src], -1 if op.res is None else ids[op.res], ids[op.dst],
+                                                             -1 if op.dst_s2d is None else ids[op.dst_s2d], op.c, w1.shape[0], _fptr(w1),
+                                                             _fptr(w2), _fptr(ws), op.mode), f"channel gate {op.name}")
             elif isinstance(op, BitTransformerSpec):
                 d = _lib.BitDesc()
                 d.c, d.token_len, d.heads, d.mlp = op.c, op.token_len, op.heads, op.mlp
@@ -91,8 +87,7 @@ class Plan:
                 if len(op.enc) == 0:
                     keep[2] = np.zeros(1, np.float32)
                 d.conv_a, d.pos, d.enc, d.dec = (_fptr(a) for a in keep)
-                add = lib.stcd_plan_add_bit_transformer_split if op.split else lib.stcd_plan_add_bit_transformer
-                _lib.check_id(add(h, ids[op.src], ids[op.dst], C.byref(d)), f"BIT transformer {op.name}")
+                _lib.check_id(lib.stcd_plan_add_bit_transformer(h, ids[op.src], ids[op.dst], C.byref(d)), f"BIT transformer {op.name}")
             elif isinstance(op, ChannelAttentionSpec):
                 n = len(op.srcs)
                 ts = (C.c_int * n)(*[ids[s_[0]] for s_ in op.srcs])
@@ -117,26 +112,22 @@ class Plan:
                                                      _fptr(prm)), f"VFFM {op.name}")
             elif isinstance(op, SumSpec):
                 arr = (C.c_int * len(op.srcs))(*[ids[s_] for s_ in op.srcs])
-                add = lib.stcd_plan_add_sum_split if op.split else lib.stcd_plan_add_sum
-                _lib.check_id(add(h, arr, len(op.srcs), ids[op.dst]), f"sum {op.name}")
+                _lib.check_id(lib.stcd_plan_add_sum(h, arr, len(op.srcs), ids[op.dst]), f"sum {op.name}")
             elif isinstance(op, LayerNormSpec):
                 g, b = np.ascontiguousarray(op.gamma, np.float32), np.ascontiguousarray(op.beta, np.float32)
-                add = lib.stcd_plan_add_layernorm_split if op.split else lib.stcd_plan_add_layernorm
-                _lib.check_id(add(h, ids[op.src], ids[op.dst], -1 if op.dst_s2d is None else ids[op.dst_s2d], op.c, _fptr(g), _fptr(b),
-                                  float(op.eps)), f"layer norm {op.name}")
+                _lib.check_id(lib.stcd_plan_add_layernorm(h, ids[op.src], ids[op.dst], -1 if op.dst_s2d is None else ids[op.dst_s2d], op.c,
+                                                          _fptr(g), _fptr(b), float(op.eps)), f"layer norm {op.name}")
             elif isinstance(op, AttentionSpec):
-                add = lib.stcd_plan_add_sr_attention_split if op.split else lib.stcd_plan_add_sr_attention
-                _lib.check_id(add(h, ids[op.q], ids[op.kv], ids[op.dst], op.c, op.heads, float(op.scale)), f"attention {op.name}")
+                _lib.check_id(lib.stcd_plan_add_sr_attention(h, ids[op.q], ids[op.kv], ids[op.dst], op.c, op.heads, float(op.scale)),
+                              f"attention {op.name}")
             elif isinstance(op, DWConvSpec):
                 wt, b = np.ascontiguousarray(op.weight, np.float32), np.ascontiguousarray(op.bias, np.float32)
-                add = lib.stcd_plan_add_dwconv3x3_split if op.split else lib.stcd_plan_add_dwconv3x3
-                _lib.check_id(add(h, ids[op.src], ids[op.dst], op.c, _fptr(wt), _fptr(b), 1 if op.gelu else 0), f"dw conv {op.name}")
+                _lib.check_id(lib.stcd_plan_add_dwconv3x3(h, ids[op.src], ids[op.dst], op.c, _fptr(wt), _fptr(b), 1 if op.gelu else 0),
+                              f"dw conv {op.name}")
             elif isinstance(op, BilinearUpSpec):
-                add = lib.stcd_plan_add_bilinear_up_split if op.split else lib.stcd_plan_add_bilinear_up
-                _lib.check_id(add(h, ids[op.src], ids[op.dst], op.c, op.scale), f"bilinear {op.name}")
+                _lib.check_id(lib.stcd_plan_add_bilinear_up(h, ids[op.src], ids[op.dst], op.c, op.scale), f"bilinear {op.name}")
             elif isinstance(op, MaxPoolS2DSpec):
-                add = lib.stcd_plan_add_maxpool_s2d_split if op.split else lib.stcd_plan_add_maxpool_s2d
-                _lib.check_id(add(h, ids[op.src], ids[op.dst], op.c), f"maxpool {op.name}")
+                _lib.check_id(lib.stcd_plan_add_maxpool_s2d(h, ids[op.src], ids[op.dst], op.c), f"maxpool {op.name}")
             elif isinstance(op, SegHeadSpec):
                 d = _lib.SegHeadDesc()
                 d.src, d.c, d.bias, d.out_ext = ids[op.src], op.c, float(op.bias), op.out_ext
@@ -204,7 +195,6 @@ class Plan:
         d.out0_s2d = 1 if op.out0_s2d else 0
         d.fold_cs, d.fold_cout = op.fold_cs, op.fold_cout
         d.xf_cs = op.xf_cs
-        d.split = 1 if op.split else 0
         _lib.check_id(self.lib.stcd_plan_add_conv(self._h, C.byref(d)), f"conv {op.name}")
 
     def _add_ecam(self, op: EcamHeadSpec) -> None:
@@ -217,7 +207,6 @@ class Plan:
                 (op.ca_fc1, op.ca_fc2, op.ca1_fc1, op.ca1_fc2, op.w_final, op.b_final)]
         d.ca_fc1, d.ca_fc2, d.ca1_fc1, d.ca1_fc2, d.w_final, d.b_final = (_fptr(a) for a in keep)
         d.out_ext = op.out_ext
-        d.split = 1 if op.split else 0
         _lib.check_id(self.lib.stcd_plan_add_ecam_head(self._h, C.byref(d)), f"ecam head {op.name}")
 
     # ------------------------------------------------------------------ queries

@@ -3,6 +3,7 @@ every compute entry point fails loudly (no CPU fallback)."""
 import ctypes as C
 import re
 
+import numpy as np
 import pytest
 import torch
 
@@ -33,13 +34,14 @@ def test_struct_layouts_match_header():
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="CPU-only behaviour")
-def test_no_gpu_fails_loudly():
+def test_no_gpu_fails_loudly_at_either_precision():
     lib = _lib.lib()
     assert lib.stcd_device_count() == 0
     h = C.c_void_p()
-    rc = lib.stcd_plan_create(0, 4, C.byref(h))
-    assert rc == 3 and not h.value          # STCD_ERR_NO_DEVICE
-    assert b"no CPU fallback" in lib.stcd_last_error()
+    for precision in (_lib.PRECISION_BF16, _lib.PRECISION_SPLIT):
+        rc = lib.stcd_plan_create(0, 4, precision, C.byref(h))
+        assert rc == 3 and not h.value          # STCD_ERR_NO_DEVICE
+        assert b"no CPU fallback" in lib.stcd_last_error()
     cm = (C.c_int64 * 4)()
     buf = (C.c_uint8 * 16)()
     rc = lib.stcd_confusion_add_batch(buf, 3, 0.0, buf, 1, 1, 16, 2, cm, None, None)
@@ -57,6 +59,46 @@ def test_argument_validation_without_gpu():
     assert lib.stcd_confusion_add_batch(buf, 9, 0.0, buf, 1, 1, 16, 2, cm, None, None) == 1
     assert lib.stcd_confusion_add_batch(buf, 0, 0.0, buf, 1, 1, 16, 3, cm, None, None) == 1
     assert lib.stcd_forward(None, None, None, 1, None, 0, None) == 4      # STCD_ERR_STATE
+
+
+def test_plan_precision():
+    """The precision is declared once, for the whole plan: a split plan declares only two-plane tensors (channels a multiple
+    of 16) and refuses the ops that have no split form, all of which a bf16 plan accepts."""
+    lib = _lib.lib()
+    h = C.c_void_p()
+    for bad in (-1, 2):
+        assert lib.stcd_plan_create(-1, 1, bad, C.byref(h)) == 1 and not h.value     # STCD_ERR_INVALID
+        assert b"precision" in lib.stcd_last_error()
+    z, ones = np.zeros(1 << 16, np.float32), np.ones(16, np.float32)
+    f = lambda a: a.ctypes.data_as(C.POINTER(C.c_float))  # noqa: E731
+    for precision in (_lib.PRECISION_BF16, _lib.PRECISION_SPLIT):
+        split = precision == _lib.PRECISION_SPLIT
+        _lib.check(lib.stcd_plan_create(-1, 1, precision, C.byref(h)), "create")
+        try:
+            t = lambda mult, c: lib.stcd_plan_add_tensor(h, mult, 16, 16, c, 0)  # noqa: E731
+            assert (t(1, 24) < 0) == split
+            a, b, c = t(1, 32), t(1, 32), t(1, 32)
+            pair16 = t(2, 16)
+            seg = _lib.SegHeadDesc(pair16, 16, f(z), 0.0, 0, -1)
+            calls = [
+                ("graph conv", lambda: lib.stcd_plan_add_graph_conv(h, a, b, 32, 9, 1, 1, None)),
+                ("channel attention", lambda: lib.stcd_plan_add_channel_attention(h, (C.c_int * 1)(a), (C.c_int * 1)(0), (C.c_int * 1)(32),
+                                                                                  1, b, 8, f(z), f(z))),
+                ("spatial gate", lambda: lib.stcd_plan_add_spatial_gate(h, a, b, 32, f(z), f(ones), f(z))),
+                ("global-local gate", lambda: lib.stcd_plan_add_global_local_gate(h, a, b, 32, f(z))),
+                ("csam gate", lambda: lib.stcd_plan_add_csam_gate(h, a, b, 32, 8, f(z))),
+                ("VFFM", lambda: lib.stcd_plan_add_vffm(h, a, b, a, b, c, 32, 8, f(z))),
+                ("seg head", lambda: lib.stcd_plan_add_seg_head(h, C.byref(seg))),
+                ("uint8 input pack", lambda: lib.stcd_plan_add_input_pack_u8(h, pair16, 3, 0, f(z), f(ones))),
+            ]
+            for name, call in calls:
+                rc = call()
+                if split:
+                    assert rc < 0 and f"{name} has no split form" in lib.stcd_last_error().decode(), name
+                else:
+                    assert rc >= 0, (name, lib.stcd_last_error())
+        finally:
+            lib.stcd_plan_destroy(h)
 
 
 # every registry family at a small legal size: the library's own descriptor checks run on the lowered programs without a

@@ -98,31 +98,31 @@ def test_split_program_passes_the_library_checks(chunk):
     plan.close()
 
 
-def test_split_entry_points_reject_bad_tensors():
-    """Split bandwidth ops need tensors that store twice their logical channels (multiples of 16); split attention needs
-    exactly 64 keys."""
+def test_split_plan_rejects_bad_tensors():
+    """In a split plan the bandwidth ops need tensors that store twice their logical channels; attention needs exactly 64
+    keys."""
     import ctypes as C
     import numpy as np
     lib = _lib.lib()
     h = C.c_void_p()
-    _lib.check(lib.stcd_plan_create(-1, 1, C.byref(h)), "create")
+    _lib.check(lib.stcd_plan_create(-1, 1, _lib.PRECISION_SPLIT, C.byref(h)), "create")
     try:
         t = lambda mult, hh, ww, c: lib.stcd_plan_add_tensor(h, mult, hh, ww, c, 0)  # noqa: E731
         one, two = t(2, 16, 16, 64), t(2, 16, 16, 128)
         g = np.ones(64, np.float32)
         gp = g.ctypes.data_as(C.POINTER(C.c_float))
         w9 = np.ones(64 * 9, np.float32).ctypes.data_as(C.POINTER(C.c_float))
-        assert lib.stcd_plan_add_layernorm_split(h, one, two, -1, 64, gp, gp, 1e-6) < 0
-        assert lib.stcd_plan_add_layernorm_split(h, two, two, -1, 64, gp, gp, 1e-6) >= 0
-        assert lib.stcd_plan_add_dwconv3x3_split(h, two, one, 64, w9, gp, 1) < 0
-        assert lib.stcd_plan_add_dwconv3x3_split(h, two, two, 64, w9, gp, 1) >= 0
+        assert lib.stcd_plan_add_layernorm(h, one, two, -1, 64, gp, gp, 1e-6) < 0
+        assert lib.stcd_plan_add_layernorm(h, two, two, -1, 64, gp, gp, 1e-6) >= 0
+        assert lib.stcd_plan_add_dwconv3x3(h, two, one, 64, w9, gp, 1) < 0
+        assert lib.stcd_plan_add_dwconv3x3(h, two, two, 64, w9, gp, 1) >= 0
         up = t(2, 32, 32, 128)
-        assert lib.stcd_plan_add_bilinear_up_split(h, one, up, 64, 2) < 0
-        assert lib.stcd_plan_add_bilinear_up_split(h, two, up, 64, 2) >= 0
+        assert lib.stcd_plan_add_bilinear_up(h, one, up, 64, 2) < 0
+        assert lib.stcd_plan_add_bilinear_up(h, two, up, 64, 2) >= 0
         kv64, kv16 = t(2, 8, 8, 256), t(2, 4, 4, 256)
-        assert lib.stcd_plan_add_sr_attention_split(h, two, kv16, two, 64, 1, 0.125) < 0          # 16 keys
-        assert lib.stcd_plan_add_sr_attention_split(h, one, kv64, one, 64, 1, 0.125) < 0          # single-plane q / dst
-        assert lib.stcd_plan_add_sr_attention_split(h, two, kv64, two, 64, 1, 0.125) >= 0
+        assert lib.stcd_plan_add_sr_attention(h, two, kv16, two, 64, 1, 0.125) < 0          # 16 keys
+        assert lib.stcd_plan_add_sr_attention(h, one, kv64, one, 64, 1, 0.125) < 0          # single-plane q / dst
+        assert lib.stcd_plan_add_sr_attention(h, two, kv64, two, 64, 1, 0.125) >= 0
     finally:
         lib.stcd_plan_destroy(h)
 

@@ -14,10 +14,10 @@ def _f(a):
     return np.ascontiguousarray(a, np.float32).ctypes.data_as(C.POINTER(C.c_float))
 
 
-def test_new_plan_ops_reject_bad_arguments():
+def test_bf16_plan_ops_reject_bad_arguments():
     lib = _lib.lib()
     h = C.c_void_p()
-    _lib.check(lib.stcd_plan_create(0, 2, C.byref(h)), "stcd_plan_create")
+    _lib.check(lib.stcd_plan_create(0, 2, _lib.PRECISION_BF16, C.byref(h)), "stcd_plan_create")
     try:
         pair32 = _lib.check_id(lib.stcd_plan_add_tensor(h, 2, 16, 16, 32, 0), "tensor")       # [2*chunk, 16, 16, 32]
         one32 = _lib.check_id(lib.stcd_plan_add_tensor(h, 1, 16, 16, 32, 0), "tensor")

@@ -1,7 +1,7 @@
 """BIT (BASE_Transformer s4 / dd8 / dd8_dedim8, the ResNet-18 baseline) and DTCDSCN on the precision path
 (``net.precision = "tf32"``: split-bf16 operands, lowering.Program.precision) without a GPU: the split programs through the
 emulator against the fp32 oracle, the bf16 programs left as they were, and the library's own descriptor checks (validation
-plans, the split entry points' tensor checks, split convs with a space-to-depth store)."""
+plans, the split plan's tensor checks, split convs with a space-to-depth store)."""
 import ctypes as C
 import dataclasses
 
@@ -91,33 +91,31 @@ def test_split_program_passes_the_library_checks(name, chunk):
     plan.close()
 
 
-def test_split_entry_points_reject_single_plane_tensors():
+def test_split_plan_rejects_single_plane_tensors():
     lib = _lib.lib()
     h = C.c_void_p()
-    _lib.check(lib.stcd_plan_create(-1, 1, C.byref(h)), "create")
+    _lib.check(lib.stcd_plan_create(-1, 1, _lib.PRECISION_SPLIT, C.byref(h)), "create")
     try:
         t = lambda mult, hh, ww, c: lib.stcd_plan_add_tensor(h, mult, hh, ww, c, 0)  # noqa: E731
         f = lambda a: a.ctypes.data_as(C.POINTER(C.c_float))  # noqa: E731
         # input pack: 32 stored channels (hi [0, 16), lo [16, 32))
-        assert lib.stcd_plan_add_input_pack_s2d_split(h, t(2, 16, 16, 16), 3) < 0
-        assert lib.stcd_plan_add_input_pack_s2d_split(h, t(2, 16, 16, 32), 3) >= 0
+        assert lib.stcd_plan_add_input_pack_s2d(h, t(2, 16, 16, 16), 3) < 0
+        assert lib.stcd_plan_add_input_pack_s2d(h, t(2, 16, 16, 32), 3) >= 0
         # max-pool: src 8c, dst 2c
         s4, s8, d1, d2 = t(2, 8, 8, 256), t(2, 8, 8, 512), t(2, 8, 8, 64), t(2, 8, 8, 128)
-        assert lib.stcd_plan_add_maxpool_s2d_split(h, s4, d2, 64) < 0
-        assert lib.stcd_plan_add_maxpool_s2d_split(h, s8, d1, 64) < 0
-        assert lib.stcd_plan_add_maxpool_s2d_split(h, s8, d2, 64) >= 0
-        # differences and sums: channel counts that cannot hold two planes of 8-channel groups
-        a24, b24, a32, b32 = t(2, 8, 8, 24), t(1, 8, 8, 24), t(2, 8, 8, 32), t(1, 8, 8, 32)
-        assert lib.stcd_plan_add_absdiff_split(h, a24, b24) < 0
-        assert lib.stcd_plan_add_absdiff_split(h, a32, b32) >= 0
-        assert lib.stcd_plan_add_subdiff_split(h, a24, -1, b24) < 0
-        assert lib.stcd_plan_add_subdiff_split(h, a32, t(1, 8, 8, 32), b32) >= 0
-        assert lib.stcd_plan_add_sum_split(h, (C.c_int * 2)(b24, b24), 2, b24) < 0
-        assert lib.stcd_plan_add_sum_split(h, (C.c_int * 2)(b32, b32), 2, t(1, 8, 8, 32)) >= 0
+        assert lib.stcd_plan_add_maxpool_s2d(h, s4, d2, 64) < 0
+        assert lib.stcd_plan_add_maxpool_s2d(h, s8, d1, 64) < 0
+        assert lib.stcd_plan_add_maxpool_s2d(h, s8, d2, 64) >= 0
+        # differences and sums: a split plan declares no tensor that cannot hold two planes of 8-channel groups
+        assert t(2, 8, 8, 24) < 0 and t(1, 8, 8, 24) < 0
+        a32, b32 = t(2, 8, 8, 32), t(1, 8, 8, 32)
+        assert lib.stcd_plan_add_absdiff(h, a32, b32) >= 0
+        assert lib.stcd_plan_add_subdiff(h, a32, t(1, 8, 8, 32), b32) >= 0
+        assert lib.stcd_plan_add_sum(h, (C.c_int * 2)(b32, b32), 2, t(1, 8, 8, 32)) >= 0
         # SE gate: src / res / dst 2c, space-to-depth copy 8c
         w1, w2 = np.ones((4, 64), np.float32), np.ones((64, 4), np.float32)
         g1, g2, gs4, gs8 = t(2, 16, 16, 64), t(2, 16, 16, 128), t(2, 8, 8, 256), t(2, 8, 8, 512)
-        gate = lambda src, res, dst, s2d: lib.stcd_plan_add_channel_gate_split(h, src, res, dst, s2d, 64, 4, f(w1), f(w2), None, 0)  # noqa: E731
+        gate = lambda src, res, dst, s2d: lib.stcd_plan_add_channel_gate(h, src, res, dst, s2d, 64, 4, f(w1), f(w2), None, 0)  # noqa: E731
         assert gate(g1, -1, g2, -1) < 0
         assert gate(g2, g1, g2, -1) < 0
         assert gate(g2, g2, g2, gs4) < 0
@@ -128,8 +126,8 @@ def test_split_entry_points_reject_single_plane_tensors():
         keep = [np.zeros(n, np.float32) for n in (4 * 32, 8 * 32, 100000, 100000)]
         d.conv_a, d.pos, d.enc, d.dec = (f(a) for a in keep)
         m32, m64 = t(2, 16, 16, 32), t(2, 16, 16, 64)
-        assert lib.stcd_plan_add_bit_transformer_split(h, m32, m32, C.byref(d)) < 0
-        assert lib.stcd_plan_add_bit_transformer_split(h, m64, t(2, 16, 16, 64), C.byref(d)) >= 0
+        assert lib.stcd_plan_add_bit_transformer(h, m32, m32, C.byref(d)) < 0
+        assert lib.stcd_plan_add_bit_transformer(h, m64, t(2, 16, 16, 64), C.byref(d)) >= 0
     finally:
         lib.stcd_plan_destroy(h)
 
